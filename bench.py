@@ -13,7 +13,8 @@ collective; one NCCL all-reduce of the 8-double episode statistics per step).
 
     python bench.py --workload ph    # configs[3]: pH plant, 2^23 envs over the ranks, T=50, Modular-128 (not the bench line)
 
-Prints ONE JSON line (rank 0).
+Prints ONE JSON line (rank 0).  --dump-outputs DIR also writes, as .npy files, what the last timed rollout computed (a
+seeded sample of envs): the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -70,7 +71,15 @@ def parse():
     p.add_argument("--batch-size", type=int, default=1 << 17, help="train workload: PPO minibatch rows")
     p.add_argument("--repeat-times", type=int, default=2, help="train workload: PPO epochs over the buffer")
     p.add_argument("--tf32", action="store_true", help="train workload: TF32 cuBLAS GEMMs in the learner (default: fp32 like the reference)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last timed rollout returned (replay rows and final env state of a "
+                        "fixed sample of envs, episode statistics) as DIR/<name>.npy")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "train"):
+        p.error("--dump-outputs applies to the GPU rollout workloads (wt, ph, wts10)")
+    return args
 
 
 def peaks():
@@ -302,6 +311,29 @@ def ph_e2e(env, actor, T, K, bs, bo, stats, steps, world, barrier, dist):
     return e
 
 
+DUMP_BYTES = 48 << 20   # --dump-outputs writes well under 64 MB
+
+
+def dump_outputs(path, env, bs, bo, stats):
+    """What one rollout hands its caller: the replay rows [T, n, S] and [T, n, 4], the episode statistics and the float
+    env state it leaves behind.  These are GBs at the default sizes, so a fixed, seeded sample of envs is written (every
+    time step of each; the same envs for the same --envs)."""
+    import torch
+    T, n, S = bs.shape
+    names = ["h1", "h2", "r", "I", "a1", "a2", "Kp"] if hasattr(env, "h1") else ["x", "y", "r", "I", "A", "B", "C", "qww_V", "qc_V"]
+    state = {"env_" + k: getattr(env, k) for k in names + ["ep_return"]}      # [n] each
+    if getattr(env, "frames", None) is not None:
+        state["env_frames"] = env.frames                                       # [3 * num_stack, n]
+    env_bytes = 4 * T * (S + 4) + sum(t.element_size() * t.numel() // n for t in state.values())
+    m = min(n, max(1, DUMP_BYTES // env_bytes))
+    idx = torch.as_tensor(np.sort(np.random.default_rng(0).choice(n, m, replace=False)), device=bs.device)
+    out = {"buf_state": bs[:, idx], "buf_other": bo[:, idx], "stats": stats}
+    out.update({k: t[..., idx] for k, t in state.items()})
+    os.makedirs(path, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(path, k + ".npy"), v.cpu().numpy())
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -373,6 +405,8 @@ def run_b200(args):
     value = world * n * T * args.steps / (ms_total * 1e-3)
     st = stats.cpu().numpy()
     env.check_status()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, env, bs, bo, stats)   # before the e2e calls below overwrite bs, bo, stats and the env
 
     # ---- e2e: the host-buffer API call (pinned host state in, ep_return out), H2D/D2H inside the timed region; timed over
     # args.steps calls directly after the device-timed loop (same clocks / thermal state, so the two numbers compare)

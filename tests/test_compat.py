@@ -1,12 +1,10 @@
 """compat/: the reference's module names (gym_control, elegantrl.*, utils.*) on top of pime_b200, so that the reference's
 unmodified train.py / run_*_changing.sh drive the library (SURVEY.md 8b).
 
-Host tests: every import of the reference's train.py and every attribute it reads on the env / agent / argument objects
-resolves under compat/ (AST walk of /root/reference/train.py; skipped where the reference checkout is absent, e.g. on the
-GPU box), plus the SB3-style logger.  GPU test: the flow of train.py:main() written against the compat names only, in a
+Host tests: every compat module imports, the agent / env methods the reference's train.py, elegantrl/run.py and utils/
+call exist, plus the SB3-style logger.  GPU test: the flow of train.py:main() written against the compat names only, in a
 subprocess with PYTHONPATH = repo : compat : compat/_shims.
 """
-import ast
 import csv
 import importlib
 import os
@@ -18,7 +16,6 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 COMPAT = os.path.join(ROOT, "compat")
-REF_TRAIN = "/root/reference/train.py"
 PATHS = [ROOT, COMPAT, os.path.join(COMPAT, "_shims")]
 
 
@@ -55,43 +52,11 @@ def test_every_compat_module_imports(compat_path):
         u.MODELS["td3"]()
 
 
-@pytest.mark.skipif(not os.path.exists(REF_TRAIN), reason="the reference checkout is not on this machine")
-def test_reference_train_py_resolves_in_compat(compat_path):
-    tree = ast.parse(open(REF_TRAIN).read())
-    star_from = []
-    for node in ast.walk(tree):
-        if isinstance(node, ast.ImportFrom):
-            m = importlib.import_module(node.module)
-            for a in node.names:
-                if a.name == "*":
-                    star_from.append(m)
-                else:
-                    assert hasattr(m, a.name), f"from {node.module} import {a.name}"
-        elif isinstance(node, ast.Import):
-            for a in node.names:
-                importlib.import_module(a.name)
-    # free names train.py calls that can only come from the star import
-    called = {n.func.id for n in ast.walk(tree) if isinstance(n, ast.Call) and isinstance(n.func, ast.Name)}
-    star = {n for n in called if n.startswith(("test_", "robust_test"))}
-    assert star and all(any(hasattr(m, n) for m in star_from) or n == "robust_test_nonlinear_watertank" for n in star), star
-    # attributes read / called on the objects train.py handles
+def test_agent_and_env_methods_the_reference_scripts_call_exist(compat_path):
     import pime_b200.gym_api as G
     import pime_b200.rl as R
-    used = {}
-    for n in ast.walk(tree):
-        if isinstance(n, ast.Attribute) and isinstance(n.value, ast.Name) and n.value.id in ("env", "agent", "kargs"):
-            used.setdefault(n.value.id, set()).add(n.attr)
-    env_cls = (G.NonLinearWaterTankChangingParamUniformGoalIntegrator, G.NonLinearWaterTankChangingParamUniformGoalStacking,
-               G.PH1DChangingParamUniformGoalIntegrator)
-    instance_attrs = {"K", "action_space", "target_return"}   # set in __init__ / by train.py itself
-    for attr in used["env"]:
-        for cls in env_cls:
-            assert attr in instance_attrs or hasattr(cls, attr), f"env.{attr} ({cls.__name__})"
-    for attr in used["agent"]:
-        assert attr in ("act",) or hasattr(R.AgentResidualIntegratorModularPPO, attr), f"agent.{attr}"
-    ka = R.Arguments(if_on_policy=True)
-    for attr in used["kargs"]:
-        assert hasattr(ka, attr), f"kargs.{attr}"
+    # the import statements of the train.py flow (FLOW below) resolve without a GPU
+    exec("\n".join(line for line in FLOW.splitlines() if line.startswith(("import ", "from "))), {})
     # the call sites of elegantrl/run.py:train_and_evaluate on the agent and the evaluator
     for name in ("init", "init_residual", "init_actor_zero", "fix_K", "frozen_integrator", "frozen_transfer", "save_load_model",
                  "explore_env", "update_net", "select_action"):
