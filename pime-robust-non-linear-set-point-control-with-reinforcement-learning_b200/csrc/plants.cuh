@@ -105,16 +105,20 @@ __device__ __forceinline__ void wt_advance(const WtConst<T> &c, WtEnv<T> &e, T a
     reward = rew;
 }
 
+// low + (high - low) u of numpy's uniform(low, high), product and sum rounded separately: left to itself nvcc contracts
+// the expression into one DFMA, and the f64 parameters would no longer be the ones numpy's arithmetic gives
+__device__ __forceinline__ double uniform_in(double lo, double w, double u) { return __dadd_rn(lo, __dmul_rn(w, u)); }
+
 // reset_all()/reset_r() (:902-939): u[] are the six uniforms of reset_uniforms().
 template <typename T> __device__ __forceinline__ void wt_reset(const WtConst<T> &c, WtEnv<T> &e, const double u[6], bool resample) {
     if (resample) {  // sample_parameters (:890-894): low + (high-low)*u
-        e.a1 = (T)((double)c.a1_lo + (double)c.a1_w * u[0]);
-        e.a2 = (T)((double)c.a2_lo + (double)c.a2_w * u[1]);
-        e.Kp = (T)((double)c.Kp_lo + (double)c.Kp_w * u[2]);
+        e.a1 = (T)uniform_in((double)c.a1_lo, (double)c.a1_w, u[0]);
+        e.a2 = (T)uniform_in((double)c.a2_lo, (double)c.a2_w, u[1]);
+        e.Kp = (T)uniform_in((double)c.Kp_lo, (double)c.Kp_w, u[2]);
     }
-    e.h1 = (T)((double)c.h_lo + (double)c.h_w * u[3]);  // :912
-    e.h2 = (T)((double)c.h_lo + (double)c.h_w * u[4]);
-    e.r = (T)((double)c.r_lo + (double)c.r_w * u[5]);   // :913
+    e.h1 = (T)uniform_in((double)c.h_lo, (double)c.h_w, u[3]);  // :912
+    e.h2 = (T)uniform_in((double)c.h_lo, (double)c.h_w, u[4]);
+    e.r = (T)uniform_in((double)c.r_lo, (double)c.r_w, u[5]);   // :913
     e.t = 0;
     e.I = (T)0;
 }
@@ -218,14 +222,14 @@ template <typename T>
 __device__ __forceinline__ bool ph_reset(const PhConst<T> &c, const T *__restrict__ table, PhEnv<T> &e, T &qww, T &qc,
                                          const double u[6], bool resample, double last_x) {
     if (resample) {  // sample_parameters (:409-410) + update_system (:414)
-        qww = (T)(c.qww_lo + c.qww_w * u[0]);
-        qc = (T)(c.qc_lo + c.qc_w * u[1]);
+        qww = (T)uniform_in(c.qww_lo, c.qww_w, u[0]);
+        qc = (T)uniform_in(c.qc_lo, c.qc_w, u[1]);
         ph_update_system<T>(c.sample_t, qww, qc, e.A, e.B, e.C);
     }
-    e.x = last_x == last_x ? last_x : c.x_lo + c.x_w * u[2];                        // :417-420
+    e.x = last_x == last_x ? last_x : uniform_in(c.x_lo, c.x_w, u[2]);              // :417-420
     bool ok = ph_lookup(table, c.table_len, (double)e.C, e.x, e.y); // :422
     e.t = 0;
-    e.r = (T)(c.r_lo + c.r_w * u[3]);                   // :424
+    e.r = (T)uniform_in(c.r_lo, c.r_w, u[3]);           // :424
     e.I = (T)0;
     return ok;
 }

@@ -72,8 +72,30 @@ def _torch_forward(kind, sd, obs, relu=False):
     return (h @ t["net.6.weight"].T + t["net.6.bias"])[:, 0]
 
 
-@pytest.mark.parametrize("kind,H,S,D", [("modular", 256, 4, 1), ("modular", 128, 3, 1), ("plain", 256, 30, 0), ("plain", 256, 3, 0),
-                                        ("plain", 128, 12, 0), ("plain", 64, 4, 0), ("critic", 256, 4, 0), ("critic", 128, 3, 0)])
+# Bounds on (a_avg - fp32 torch) per compiled (kind, H): (RMS over n = 1 / 129 / 40000, |mean| at n = 40000), set from one
+# B200 run (NVIDIA B200, 1000 W power limit) at 1.5x the measured value; the comment gives the measured max |error|, RMS and
+# |mean|.  The fused rollout's network is pinned bit for bit to this kernel (test_gpu_08), so these bounds carry over to it.
+FWD_BOUNDS = {  # (kind)(H)-S(S): (rms, |mean|),  measured: max      rms      |mean|
+    "modular256-S4": (2.6e-04, 1.4e-04),  # 5.8e-04  1.7e-04  9.2e-05
+    "modular128-S3": (3.6e-04, 4.2e-05),  # 4.5e-04  2.4e-04  2.8e-05
+    "modular64-S3": (1.1e-04, 2.7e-05),  # 2.5e-04  7.2e-05  1.8e-05
+    "modular32-S4": (6.8e-05, 8.3e-06),  # 1.4e-04  4.5e-05  5.5e-06
+    "plain256-S30": (2.5e-04, 4.9e-05),  # 6.9e-04  1.6e-04  3.2e-05
+    "plain256-S3": (3.0e-04, 1.4e-04),  # 4.8e-04  2.0e-04  8.7e-05
+    "plain128-S12": (1.9e-04, 7.4e-05),  # 5.1e-04  1.2e-04  4.9e-05
+    "plain64-S4": (1.8e-04, 6.2e-05), # 2.1e-04  1.1e-04  4.1e-05
+    "plain32-S3": (1.6e-04, 6.1e-05), # 1.7e-04  1.0e-04  4.0e-05
+    "critic256-S4": (4.6e-04, 3.8e-05),  # 1.5e-03  3.0e-04  2.5e-05
+    "critic128-S3": (2.3e-04, 1.6e-05),  # 8.2e-04  1.5e-04  1.0e-05
+    "critic64-S4": (7.6e-04, 1.1e-04),  # 9.4e-04  5.0e-04  6.9e-05
+    "critic32-S3": (2.2e-04, 1.4e-06),  # 3.8e-04  1.4e-04  9.0e-07
+}
+
+
+@pytest.mark.parametrize("kind,H,S,D", [("modular", 256, 4, 1), ("modular", 128, 3, 1), ("modular", 64, 3, 1), ("modular", 32, 4, 1),
+                                        ("plain", 256, 30, 0), ("plain", 256, 3, 0), ("plain", 128, 12, 0), ("plain", 64, 4, 0),
+                                        ("plain", 32, 3, 0), ("critic", 256, 4, 0), ("critic", 128, 3, 0), ("critic", 64, 4, 0),
+                                        ("critic", 32, 3, 0)])
 @pytest.mark.parametrize("n", [1, 129, 40000])
 def test_forward_vs_torch_fp32(V, oracle, kind, H, S, D, n):
     torch.backends.cuda.matmul.allow_tf32 = False
@@ -85,9 +107,14 @@ def test_forward_vs_torch_fp32(V, oracle, kind, H, S, D, n):
         obs[:, -1] = rng.uniform(-25, 25, n)
     got = host(pack.forward(dev(obs)))
     want = host(_torch_forward("modular" if kind == "modular" else "plain", sd, dev(obs), relu=(kind == "critic")))
-    err = np.max(np.abs(got - want))
-    print(f"{kind} H{H} S{S} n{n}: max err {err:.3e}, rms {np.sqrt(np.mean((got - want) ** 2)):.3e}, |want| max {np.abs(want).max():.3f}")
+    e = got.astype(np.float64) - want
+    err, rms, mean = np.max(np.abs(e)), np.sqrt(np.mean(e ** 2)), np.mean(e)
+    print(f"{kind} H{H} S{S} n{n}: max err {err:.3e}, rms {rms:.3e}, mean {mean:+.3e}, |want| max {np.abs(want).max():.3f}")
     np.testing.assert_allclose(got, want, atol=ATOL, rtol=RTOL)
+    rb, mb = FWD_BOUNDS[f"{kind}{H}-S{S}"]
+    assert rms <= rb, (rms, rb)
+    if n == 40000:
+        assert abs(mean) <= mb, (mean, mb)
     if kind != "critic" and n <= 129:  # the C oracle restates the same fp32 forward
         acfg = oracle.ActorCfg(kind=1 if kind == "modular" else 0, state_dim=S, mid_dim=H, integrator_dim=D)
         o = oracle.actor_forward(acfg, oracle.pack_actor_params(sd, acfg.kind), obs)
