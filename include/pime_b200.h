@@ -246,6 +246,8 @@ int pime_actor_forward(const pime_actor_config *cfg, const void *pack, int64_t n
  *   action  = tanh(a_raw) + obs32 . priorK                   agent_residual.py:61 / net_residual.py:167-170
  *   env.step(action)                                         as pime_*_step_*
  *   row     = obs32[S], reward*reward_scale, (done?0:gamma), a_raw, eps      agent_residual.py:64-65, replay.py:278
+ *
+ * The config and state are checked as by the step entries (PIME_EINVAL, also without a device and for n = 0).
  * ------------------------------------------------------------------------------------------------------- */
 typedef struct pime_rollout_args {
     const pime_actor_config *actor; /* NULL: prior-only policy (a_avg = 0)                                   */

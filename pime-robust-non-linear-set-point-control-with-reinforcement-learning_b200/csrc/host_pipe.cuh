@@ -26,6 +26,8 @@ struct HostArr {
     bool back;       // copied back after the rollout
 };
 
+template <typename E> inline HostArr host_arr(E *hp, E *dp, bool back) { return {hp, dp, (int)sizeof(E), back}; }
+
 struct HostPipe {
     bool ready = false;
     cudaStream_t in = nullptr, out = nullptr;

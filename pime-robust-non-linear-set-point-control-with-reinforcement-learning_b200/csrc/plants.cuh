@@ -1,4 +1,5 @@
-// plants.cuh -- per-env device arithmetic of the two gym_control plants (one thread = one env, state in registers).
+// plants.cuh -- per-env device arithmetic of the two gym_control plants (one thread = one env, state in registers), the
+// typed view of each plant's SoA state arrays and the argument checks of its entry points.
 // Used by the stand-alone step/reset kernels (step.cu) and by the fused rollout kernels (rollout_impl.cuh).
 #pragma once
 
@@ -42,6 +43,74 @@ template <typename T> struct WtEnv {
     T h1, h2, r, I, a1, a2, Kp;
     int t;
 };
+
+// The per-env arrays of pime_wt_state with their element types.  The loaders and storers are small on purpose: each
+// kernel reads and writes only the arrays it needs (HBM traffic is the cost of the stand-alone kernels).
+template <typename T> struct WtPtrs {
+    T *h1, *h2, *r, *I, *a1, *a2, *Kp, *ep_return, *frames, *last_h1, *last_h2;
+    int32_t *t;
+    uint32_t *episode;
+
+    WtPtrs() = default;
+    explicit WtPtrs(const pime_wt_state &s)
+        : h1((T *)s.h1), h2((T *)s.h2), r((T *)s.r), I((T *)s.I), a1((T *)s.a1), a2((T *)s.a2), Kp((T *)s.Kp),
+          ep_return((T *)s.ep_return), frames((T *)s.frames), last_h1((T *)s.last_h1), last_h2((T *)s.last_h2), t(s.t),
+          episode(s.episode) {}
+
+    // the arrays of envs [off, ...).  frames ([3 num_stack][n], row stride n) is not shifted: a range of envs would need
+    // every row shifted and the stride kept, so the stacking observation always runs as a single slice.
+    WtPtrs shifted(int64_t off) const {
+        auto adv = [off](auto *q) { return q ? q + off : q; };
+        WtPtrs p;
+        p.h1 = adv(h1); p.h2 = adv(h2); p.r = adv(r); p.I = adv(I);
+        p.a1 = adv(a1); p.a2 = adv(a2); p.Kp = adv(Kp);
+        p.ep_return = adv(ep_return); p.frames = frames; p.last_h1 = adv(last_h1); p.last_h2 = adv(last_h2);
+        p.t = adv(t); p.episode = adv(episode);
+        return p;
+    }
+
+    // what env.step() reads; I only when the observation carries the integrator (the array may be NULL otherwise)
+    __device__ __forceinline__ void load(WtEnv<T> &e, int64_t i, bool integ) const {
+        e.h1 = h1[i]; e.h2 = h2[i]; e.r = r[i];
+        e.I = integ ? I[i] : (T)0;
+        load_params(e, i);
+        e.t = t[i];
+    }
+    __device__ __forceinline__ void load_params(WtEnv<T> &e, int64_t i) const { e.a1 = a1[i]; e.a2 = a2[i]; e.Kp = Kp[i]; }
+    // what env.step() changes (the set-point and the ensemble parameters stay)
+    __device__ __forceinline__ void store_step(const WtEnv<T> &e, int64_t i, bool integ) const {
+        h1[i] = e.h1; h2[i] = e.h2;
+        if (integ) I[i] = e.I;
+        t[i] = e.t;
+    }
+    // everything load() reads
+    __device__ __forceinline__ void store(const WtEnv<T> &e, int64_t i, bool integ) const {
+        h1[i] = e.h1; h2[i] = e.h2; r[i] = e.r;
+        if (integ) I[i] = e.I;
+        a1[i] = e.a1; a2[i] = e.a2; Kp[i] = e.Kp;
+        t[i] = e.t;
+    }
+};
+
+// width of the observation vector
+inline int wt_obs_dim(const pime_wt_config &c) {
+    return c.obs_mode == PIME_WT_OBS_GOAL ? 3 : (c.obs_mode == PIME_WT_OBS_INTEGRATOR ? 4 : 3 * c.num_stack);
+}
+
+// The argument checks of every water-tank entry point (step, reset, rollout, host-buffer rollout).  They need no device, so
+// the entries run them before require_device().
+inline int validate_wt(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st) {
+    PIME_REQUIRE(cfg && st, "null config/state");
+    PIME_REQUIRE(n >= 0, "negative n");
+    PIME_REQUIRE(st->h1 && st->h2 && st->r && st->a1 && st->a2 && st->Kp && st->t && st->episode, "null state array");
+    PIME_REQUIRE(cfg->obs_mode >= 0 && cfg->obs_mode <= 2, "obs_mode");
+    PIME_REQUIRE(cfg->obs_mode != PIME_WT_OBS_INTEGRATOR || st->I, "integrator array missing");
+    PIME_REQUIRE(cfg->obs_mode != PIME_WT_OBS_STACKING || (st->frames && cfg->num_stack >= 1 && cfg->num_stack <= 10),
+                 "stacking needs frames and 1 <= num_stack <= 10");
+    PIME_REQUIRE(cfg->n_discrete >= 1 && cfg->reward_type >= 0 && cfg->reward_type <= 2, "n_discrete/reward_type");
+    PIME_REQUIRE(!cfg->reset_from_last_state || (st->last_h1 && st->last_h2), "reset_from_last_state needs last_h1/last_h2");
+    return PIME_OK;
+}
 
 // 20 Euler sub-steps (nonlinear_watertank.py:805-809).  f64: the reference's operation order, no contraction.
 __device__ __forceinline__ void wt_integrate(const WtConst<double> &c, double a1, double a2, double Kp, double u, double &x1,
@@ -169,6 +238,72 @@ template <typename T> struct PhEnv {
     T y, r, I, C;
     int t;
 };
+
+// The per-env arrays of pime_ph_state with their element types (x, A, B, last_x fp64 in both flavours, see above).
+template <typename T> struct PhPtrs {
+    double *x, *A, *B, *last_x;
+    T *y, *r, *I, *C, *qww, *qc, *ep_return;
+    int32_t *t;
+    uint32_t *episode;
+
+    PhPtrs() = default;
+    explicit PhPtrs(const pime_ph_state &s)
+        : x((double *)s.x), A((double *)s.A), B((double *)s.B), last_x((double *)s.last_x), y((T *)s.y), r((T *)s.r),
+          I((T *)s.I), C((T *)s.C), qww((T *)s.qww_V), qc((T *)s.qc_V), ep_return((T *)s.ep_return), t(s.t),
+          episode(s.episode) {}
+
+    // the arrays of envs [off, ...)
+    PhPtrs shifted(int64_t off) const {
+        auto adv = [off](auto *q) { return q ? q + off : q; };
+        PhPtrs p;
+        p.x = adv(x); p.A = adv(A); p.B = adv(B); p.last_x = adv(last_x);
+        p.y = adv(y); p.r = adv(r); p.I = adv(I); p.C = adv(C); p.qww = adv(qww); p.qc = adv(qc); p.ep_return = adv(ep_return);
+        p.t = adv(t); p.episode = adv(episode);
+        return p;
+    }
+
+    // what env.step() reads; I only when the plant integrates (the array may be NULL otherwise).  y is an output of the step:
+    // with_y also loads it, for a caller that observes the env before stepping it.
+    __device__ __forceinline__ void load(PhEnv<T> &e, int64_t i, bool integ, bool with_y = false) const {
+        e.x = x[i];
+        if (with_y) e.y = y[i];
+        e.r = r[i];
+        e.I = integ ? I[i] : (T)0;
+        load_system(e, i);
+        e.t = t[i];
+    }
+    __device__ __forceinline__ void load_system(PhEnv<T> &e, int64_t i) const { e.A = A[i]; e.B = B[i]; e.C = C[i]; }
+    __device__ __forceinline__ void store_system(const PhEnv<T> &e, int64_t i) const { A[i] = e.A; B[i] = e.B; C[i] = e.C; }
+    // what env.step() changes
+    __device__ __forceinline__ void store_step(const PhEnv<T> &e, int64_t i, bool integ) const {
+        x[i] = e.x; y[i] = e.y;
+        if (integ) I[i] = e.I;
+        t[i] = e.t;
+    }
+    // the whole PhEnv
+    __device__ __forceinline__ void store(const PhEnv<T> &e, int64_t i, bool integ) const {
+        x[i] = e.x; y[i] = e.y; r[i] = e.r;
+        if (integ) I[i] = e.I;
+        store_system(e, i);
+        t[i] = e.t;
+    }
+};
+
+inline int ph_obs_dim(const pime_ph_config &c) { return c.integrator_mode == PIME_PH_NO_INTEGRATOR ? 2 : 3; }
+
+// The argument checks of every pH entry point (step, reset, update_system, rollout, host-buffer rollout), run before
+// require_device().  table_len > 1 also keeps ph_lookup's clamp to the last entry inside the table.
+inline int validate_ph(const pime_ph_config *cfg, int64_t n, const pime_ph_state *st) {
+    PIME_REQUIRE(cfg && st, "null config/state");
+    PIME_REQUIRE(n >= 0, "negative n");
+    PIME_REQUIRE(st->x && st->y && st->r && st->A && st->B && st->C && st->qww_V && st->qc_V && st->t && st->episode,
+                 "null state array");
+    PIME_REQUIRE(cfg->integrator_mode >= 0 && cfg->integrator_mode <= 2, "integrator_mode");
+    PIME_REQUIRE(cfg->integrator_mode == PIME_PH_NO_INTEGRATOR || st->I, "integrator array missing");
+    PIME_REQUIRE(cfg->table_len > 1 && cfg->reward_type >= 0 && cfg->reward_type <= 2, "table_len/reward_type");
+    PIME_REQUIRE(!cfg->reset_from_last_state || st->last_x, "reset_from_last_state needs last_x");
+    return PIME_OK;
+}
 
 // observe_state (ph.py:187-189): first i with MHCl[i] >= around(C*x,5)  ==  rint(C*x*1e5)  (MHCl[i] = i*1e-5;
 // equivalence checked on the reference in tests/golden/ph.npz).  The index is computed in fp64 for both table types.

@@ -42,9 +42,7 @@ template <typename T, bool STACK> struct WtGlue {
     using Real = T;
     static constexpr int kObsMax = STACK ? kMaxFrames : 4;   // widest observation of this plant (loop bounds)
     WtConst<T> c;
-    T *h1, *h2, *r, *I, *a1, *a2, *Kp, *ep_return, *frames, *last_h1, *last_h2;
-    int32_t *t;
-    uint32_t *episode;
+    WtPtrs<T> p;
 
     struct Env {
         WtEnv<T> e;
@@ -54,30 +52,24 @@ template <typename T, bool STACK> struct WtGlue {
     };
 
     __device__ __forceinline__ void load(Env &v, int64_t i, int64_t n) const {
-        v.e.h1 = h1[i]; v.e.h2 = h2[i]; v.e.r = r[i];
-        v.e.I = c.obs_mode == PIME_WT_OBS_INTEGRATOR ? I[i] : (T)0;
-        v.e.a1 = a1[i]; v.e.a2 = a2[i]; v.e.Kp = Kp[i];
-        v.e.t = t[i];
-        v.ret = ep_return ? ep_return[i] : (T)0;
-        v.episode = episode[i];
+        p.load(v.e, i, c.obs_mode == PIME_WT_OBS_INTEGRATOR);
+        v.ret = p.ep_return ? p.ep_return[i] : (T)0;
+        v.episode = p.episode[i];
         if constexpr (STACK) {
             const int m = 3 * c.num_stack;
 #pragma unroll
-            for (int j = 0; j < kMaxFrames; ++j) v.fr[j] = j < m ? frames[(int64_t)j * n + i] : (T)0;
+            for (int j = 0; j < kMaxFrames; ++j) v.fr[j] = j < m ? p.frames[(int64_t)j * n + i] : (T)0;
         }
     }
     __device__ __forceinline__ void store(const Env &v, int64_t i, int64_t n) const {
-        h1[i] = v.e.h1; h2[i] = v.e.h2; r[i] = v.e.r;
-        if (c.obs_mode == PIME_WT_OBS_INTEGRATOR) I[i] = v.e.I;
-        a1[i] = v.e.a1; a2[i] = v.e.a2; Kp[i] = v.e.Kp;
-        t[i] = v.e.t;
-        if (ep_return) ep_return[i] = v.ret;
-        episode[i] = v.episode;
+        p.store(v.e, i, c.obs_mode == PIME_WT_OBS_INTEGRATOR);
+        if (p.ep_return) p.ep_return[i] = v.ret;
+        p.episode[i] = v.episode;
         if constexpr (STACK) {
             const int m = 3 * c.num_stack;
 #pragma unroll
             for (int j = 0; j < kMaxFrames; ++j)
-                if (j < m) frames[(int64_t)j * n + i] = v.fr[j];
+                if (j < m) p.frames[(int64_t)j * n + i] = v.fr[j];
         }
     }
     // float32(obs): elegantrl/env.py:46,72.  obs[] is indexed with compile-time indices only (registers).
@@ -107,7 +99,7 @@ template <typename T, bool STACK> struct WtGlue {
     __device__ __forceinline__ T tracking_error(const Env &v) const { return Num<T>::abs(v.e.r - v.e.h2); }
     // `done` bookkeeping of reset_from_last_state (:819-821)
     __device__ __forceinline__ void record_done(const Env &v, int64_t i) const {
-        if (last_h1) { last_h1[i] = v.e.h1; last_h2[i] = v.e.h2; }
+        if (p.last_h1) { p.last_h1[i] = v.e.h1; p.last_h2[i] = v.e.h2; }
     }
     // the in-kernel reset always follows a `done`, so "the levels of the last finished episode" are the current ones
     __device__ __forceinline__ bool reset(Env &v, uint64_t seed, uint64_t index, bool resample) const {
@@ -132,10 +124,7 @@ template <typename T> struct PhGlue {
     static constexpr int kObsMax = 3;
     PhConst<T> c;
     const T *table;
-    double *x, *A, *B, *last_x;   // fp64 in both flavours (plants.cuh)
-    T *y, *r, *I, *C, *qww, *qc, *ep_return;
-    int32_t *t;
-    uint32_t *episode;
+    PhPtrs<T> p;
 
     struct Env {
         PhEnv<T> e;
@@ -143,22 +132,16 @@ template <typename T> struct PhGlue {
         uint32_t episode;
     };
     __device__ __forceinline__ void load(Env &v, int64_t i, int64_t) const {
-        v.e.x = x[i]; v.e.y = y[i]; v.e.r = r[i];
-        v.e.I = c.integrator_mode != PIME_PH_NO_INTEGRATOR ? I[i] : (T)0;
-        v.e.A = A[i]; v.e.B = B[i]; v.e.C = C[i];
-        v.e.t = t[i];
-        v.qww = qww[i]; v.qc = qc[i];
-        v.ret = ep_return ? ep_return[i] : (T)0;
-        v.episode = episode[i];
+        p.load(v.e, i, c.integrator_mode != PIME_PH_NO_INTEGRATOR, true);
+        v.qww = p.qww[i]; v.qc = p.qc[i];
+        v.ret = p.ep_return ? p.ep_return[i] : (T)0;
+        v.episode = p.episode[i];
     }
     __device__ __forceinline__ void store(const Env &v, int64_t i, int64_t) const {
-        x[i] = v.e.x; y[i] = v.e.y; r[i] = v.e.r;
-        if (c.integrator_mode != PIME_PH_NO_INTEGRATOR) I[i] = v.e.I;
-        A[i] = v.e.A; B[i] = v.e.B; C[i] = v.e.C;
-        t[i] = v.e.t;
-        qww[i] = v.qww; qc[i] = v.qc;
-        if (ep_return) ep_return[i] = v.ret;
-        episode[i] = v.episode;
+        p.store(v.e, i, c.integrator_mode != PIME_PH_NO_INTEGRATOR);
+        p.qww[i] = v.qww; p.qc[i] = v.qc;
+        if (p.ep_return) p.ep_return[i] = v.ret;
+        p.episode[i] = v.episode;
     }
     __device__ __forceinline__ void observe(const Env &v, float (&obs)[kMaxS]) const {
         obs[0] = (float)v.e.y; obs[1] = (float)v.e.r;
@@ -171,7 +154,7 @@ template <typename T> struct PhGlue {
     }
     __device__ __forceinline__ T tracking_error(const Env &v) const { return Num<T>::abs(v.e.r - v.e.y); }
     __device__ __forceinline__ void record_done(const Env &v, int64_t i) const {   // ph.py:345-346
-        if (last_x) last_x[i] = v.e.x;
+        if (p.last_x) p.last_x[i] = v.e.x;
     }
     __device__ __forceinline__ bool reset(Env &v, uint64_t seed, uint64_t index, bool resample) const {
         double u[6];

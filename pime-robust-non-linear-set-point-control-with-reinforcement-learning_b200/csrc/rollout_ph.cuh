@@ -4,28 +4,16 @@
 
 namespace pime {
 
+// The rollout of n envs whose config and state passed validate_ph; p is the state of these n envs.
 template <typename T>
-int ph_rollout_impl(const pime_ph_config *cfg, const T *table, int64_t n, const pime_ph_state *st, const pime_rollout_args *args,
-                    void *stream) {
-    PIME_REQUIRE(cfg && st && table, "null config/state/table");
-    PIME_REQUIRE(n >= 0, "negative n");
-    PIME_REQUIRE(st->x && st->y && st->r && st->A && st->B && st->C && st->qww_V && st->qc_V && st->t && st->episode,
-                 "null state array");
-    PIME_REQUIRE(cfg->integrator_mode >= 0 && cfg->integrator_mode <= 2, "integrator_mode");
-    PIME_REQUIRE(cfg->integrator_mode == PIME_PH_NO_INTEGRATOR || st->I, "integrator array missing");
-    PIME_REQUIRE(!cfg->reset_from_last_state || st->last_x, "reset_from_last_state needs last_x");
-    const int S = cfg->integrator_mode == PIME_PH_NO_INTEGRATOR ? 2 : 3;
+int ph_rollout_launch(const pime_ph_config *cfg, const T *table, int64_t n, const PhPtrs<T> &p, const pime_rollout_args *args,
+                      void *stream) {
     RolloutParams rp;
     tc::PackLayout L;
-    if (int rc = fill_rollout_params(args, n, S, rp, L)) return rc;
+    if (int rc = fill_rollout_params(args, n, ph_obs_dim(*cfg), rp, L)) return rc;
     if (int rc = require_device()) return rc;
     if (n == 0) return PIME_OK;
-    PhGlue<T> g;
-    g.c = make_ph_const<T>(*cfg);
-    g.table = table;
-    g.x = (double *)st->x; g.y = (T *)st->y; g.r = (T *)st->r; g.I = (T *)st->I;
-    g.A = (double *)st->A; g.B = (double *)st->B; g.C = (T *)st->C; g.qww = (T *)st->qww_V; g.qc = (T *)st->qc_V;
-    g.ep_return = (T *)st->ep_return; g.last_x = (double *)st->last_x; g.t = st->t; g.episode = st->episode;
+    const PhGlue<T> g{make_ph_const<T>(*cfg), table, p};
     cudaStream_t s = (cudaStream_t)stream;
     if (!rp.has_actor) return launch_rollout_prior<PhGlue<T>>(g, rp, s);
     PIME_REQUIRE(args->actor->kind != PIME_ACTOR_MODULAR || cfg->integrator_mode != PIME_PH_NO_INTEGRATOR,
@@ -35,6 +23,14 @@ int ph_rollout_impl(const pime_ph_config *cfg, const T *table, int64_t n, const 
         return launch_rollout_k<PhGlue<T>, PIME_ACTOR_MODULAR>(g, &L, args->actor_pack, rp, L.H, s);
     }
     return launch_rollout_k<PhGlue<T>, PIME_ACTOR_PLAIN>(g, &L, args->actor_pack, rp, L.H, s);
+}
+
+template <typename T>
+int ph_rollout_impl(const pime_ph_config *cfg, const T *table, int64_t n, const pime_ph_state *st, const pime_rollout_args *args,
+                    void *stream) {
+    if (int rc = validate_ph(cfg, n, st)) return rc;
+    PIME_REQUIRE(table, "null table");
+    return ph_rollout_launch<T>(cfg, table, n, PhPtrs<T>(*st), args, stream);
 }
 
 }  // namespace pime

@@ -12,25 +12,26 @@ extern "C" int pime_ph_rollout_f32(const pime_ph_config *cfg, const float *table
 extern "C" int pime_ph_rollout_host_f32(const pime_ph_config *cfg, const float *table, int64_t n, const pime_ph_state *h,
                                         const pime_ph_state *d, const pime_rollout_args *args, float *ep_return_host, void *stream) {
     PIME_REQUIRE(cfg && table && h && d && args, "null pointer");
+    if (int rc = validate_ph(cfg, n, d)) return rc;
     PIME_REQUIRE(d->ep_return, "device ep_return scratch is required");
-    PIME_REQUIRE(n >= 0, "negative n");
+    const int S = ph_obs_dim(*cfg);
+    {   // the argument block is checked before anything is enqueued; each slice fills its own RolloutParams
+        RolloutParams rp;
+        tc::PackLayout L;
+        if (int rc = fill_rollout_params(args, n, S, rp, L)) return rc;
+    }
     if (int rc = require_device()) return rc;
-    const HostArr arr[11] = {{h->x, d->x, 8, true}, {h->y, d->y, 4, true}, {h->r, d->r, 4, true}, {h->I, d->I, 4, true},
-                             {h->A, d->A, 8, false}, {h->B, d->B, 8, false}, {h->C, d->C, 4, false},
-                             {h->qww_V, d->qww_V, 4, false}, {h->qc_V, d->qc_V, 4, false},
-                             {h->t, d->t, 4, false}, {h->episode, d->episode, 4, false}};
+    const PhPtrs<float> hp(*h), dp(*d);
+    const HostArr arr[11] = {host_arr(hp.x, dp.x, true), host_arr(hp.y, dp.y, true), host_arr(hp.r, dp.r, true),
+                             host_arr(hp.I, dp.I, true), host_arr(hp.A, dp.A, false), host_arr(hp.B, dp.B, false),
+                             host_arr(hp.C, dp.C, false), host_arr(hp.qww, dp.qww, false), host_arr(hp.qc, dp.qc, false),
+                             host_arr(hp.t, dp.t, false), host_arr(hp.episode, dp.episode, false)};
     auto launch = [&](int64_t off, int64_t cnt, const pime_rollout_args &a) {
-        pime_ph_state st = *d;
-        auto sh = [&](void *p, int elem) { return p ? (void *)((char *)p + off * elem) : nullptr; };
-        st.x = sh(d->x, 8); st.y = sh(d->y, 4); st.r = sh(d->r, 4); st.I = sh(d->I, 4);
-        st.A = sh(d->A, 8); st.B = sh(d->B, 8); st.C = sh(d->C, 4); st.qww_V = sh(d->qww_V, 4); st.qc_V = sh(d->qc_V, 4);
-        st.t = (int32_t *)sh(d->t, 4); st.episode = (uint32_t *)sh(d->episode, 4);
-        st.ep_return = sh(d->ep_return, 4); st.last_x = sh(d->last_x, 8);
         pime_rollout_args b = a;
-        shift_step_buffers(b, off, cfg->integrator_mode == PIME_PH_NO_INTEGRATOR ? 2 : 3, 4);
-        return ph_rollout_impl<float>(cfg, table, cnt, &st, &b, stream);
+        shift_step_buffers(b, off, S, sizeof(float));
+        return ph_rollout_launch<float>(cfg, table, cnt, dp.shifted(off), &b, stream);
     };
-    return host_pipelined_rollout(n, arr, 11, (float *)d->ep_return, ep_return_host, args, (cudaStream_t)stream, launch, false);
+    return host_pipelined_rollout(n, arr, 11, dp.ep_return, ep_return_host, args, (cudaStream_t)stream, launch, false);
 }
 
 #ifdef PIME_PROFILE_WORKER

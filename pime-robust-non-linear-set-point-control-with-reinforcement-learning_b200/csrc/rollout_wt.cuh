@@ -4,40 +4,23 @@
 
 namespace pime {
 
+// The rollout of n envs whose config and state passed validate_wt; p is the state of these n envs.
 template <typename T>
-int wt_rollout_impl(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st, const pime_rollout_args *args, void *stream) {
-    PIME_REQUIRE(cfg && st, "null config/state");
-    PIME_REQUIRE(n >= 0, "negative n");
-    PIME_REQUIRE(st->h1 && st->h2 && st->r && st->a1 && st->a2 && st->Kp && st->t && st->episode, "null state array");
-    PIME_REQUIRE(cfg->obs_mode >= 0 && cfg->obs_mode <= 2, "obs_mode");
-    PIME_REQUIRE(cfg->obs_mode != PIME_WT_OBS_INTEGRATOR || st->I, "integrator array missing");
-    PIME_REQUIRE(cfg->obs_mode != PIME_WT_OBS_STACKING || (st->frames && cfg->num_stack >= 1 && cfg->num_stack <= 10),
-                 "stacking needs frames and 1 <= num_stack <= 10");
-    PIME_REQUIRE(!cfg->reset_from_last_state || (st->last_h1 && st->last_h2), "reset_from_last_state needs last_h1/last_h2");
-    const int S = cfg->obs_mode == PIME_WT_OBS_GOAL ? 3 : (cfg->obs_mode == PIME_WT_OBS_INTEGRATOR ? 4 : 3 * cfg->num_stack);
+int wt_rollout_launch(const pime_wt_config *cfg, int64_t n, const WtPtrs<T> &p, const pime_rollout_args *args, void *stream) {
     RolloutParams rp;
     tc::PackLayout L;
-    if (int rc = fill_rollout_params(args, n, S, rp, L)) return rc;
+    if (int rc = fill_rollout_params(args, n, wt_obs_dim(*cfg), rp, L)) return rc;
     if (int rc = require_device()) return rc;
     if (n == 0) return PIME_OK;
     cudaStream_t s = (cudaStream_t)stream;
-    auto fill = [&](auto &g) {
-        g.c = make_wt_const<T>(*cfg);
-        g.h1 = (T *)st->h1; g.h2 = (T *)st->h2; g.r = (T *)st->r; g.I = (T *)st->I;
-        g.a1 = (T *)st->a1; g.a2 = (T *)st->a2; g.Kp = (T *)st->Kp;
-        g.ep_return = (T *)st->ep_return; g.frames = (T *)st->frames; g.t = st->t; g.episode = st->episode;
-        g.last_h1 = (T *)st->last_h1; g.last_h2 = (T *)st->last_h2;
-    };
     if (cfg->obs_mode == PIME_WT_OBS_STACKING) {   // observation history: plain actor only (the modular one needs the integrator)
-        WtGlue<T, true> g;
-        fill(g);
+        const WtGlue<T, true> g{make_wt_const<T>(*cfg), p};
         if (!rp.has_actor) return launch_rollout_prior<WtGlue<T, true>>(g, rp, s);
         PIME_REQUIRE(args->actor->kind == PIME_ACTOR_PLAIN, "the stacking observation goes with the plain actor");
         if (args->actor->precision == PIME_PRECISION_FP32) return launch_rollout_fp32<WtGlue<T, true>>(g, L, args->actor_pack, rp, s);
         return launch_rollout_k<WtGlue<T, true>, PIME_ACTOR_PLAIN>(g, &L, args->actor_pack, rp, L.H, s);
     }
-    WtGlue<T, false> g;
-    fill(g);
+    const WtGlue<T, false> g{make_wt_const<T>(*cfg), p};
     if (!rp.has_actor) return launch_rollout_prior<WtGlue<T, false>>(g, rp, s);
     PIME_REQUIRE(args->actor->kind != PIME_ACTOR_MODULAR || cfg->obs_mode == PIME_WT_OBS_INTEGRATOR,
                  "the modular actor needs the integrator observation");
@@ -46,6 +29,12 @@ int wt_rollout_impl(const pime_wt_config *cfg, int64_t n, const pime_wt_state *s
         return launch_rollout_k<WtGlue<T, false>, PIME_ACTOR_MODULAR>(g, &L, args->actor_pack, rp, L.H, s);
     }
     return launch_rollout_k<WtGlue<T, false>, PIME_ACTOR_PLAIN>(g, &L, args->actor_pack, rp, L.H, s);
+}
+
+template <typename T>
+int wt_rollout_impl(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st, const pime_rollout_args *args, void *stream) {
+    if (int rc = validate_wt(cfg, n, st)) return rc;
+    return wt_rollout_launch<T>(cfg, n, WtPtrs<T>(*st), args, stream);
 }
 
 }  // namespace pime

@@ -11,25 +11,26 @@ extern "C" int pime_wt_rollout_f32(const pime_wt_config *cfg, int64_t n, const p
 extern "C" int pime_wt_rollout_host_f32(const pime_wt_config *cfg, int64_t n, const pime_wt_state *h, const pime_wt_state *d,
                                         const pime_rollout_args *args, float *ep_return_host, void *stream) {
     PIME_REQUIRE(cfg && h && d && args, "null pointer");
+    if (int rc = validate_wt(cfg, n, d)) return rc;
     PIME_REQUIRE(d->ep_return, "device ep_return scratch is required");
-    PIME_REQUIRE(n >= 0, "negative n");
+    const int S = wt_obs_dim(*cfg);
+    {   // the argument block is checked before anything is enqueued; each slice fills its own RolloutParams
+        RolloutParams rp;
+        tc::PackLayout L;
+        if (int rc = fill_rollout_params(args, n, S, rp, L)) return rc;
+    }
     if (int rc = require_device()) return rc;
-    const HostArr arr[9] = {{h->h1, d->h1, 4, true}, {h->h2, d->h2, 4, true}, {h->r, d->r, 4, true}, {h->I, d->I, 4, true},
-                            {h->a1, d->a1, 4, false}, {h->a2, d->a2, 4, false}, {h->Kp, d->Kp, 4, false},
-                            {h->t, d->t, 4, false}, {h->episode, d->episode, 4, false}};
+    const WtPtrs<float> hp(*h), dp(*d);
+    const HostArr arr[9] = {host_arr(hp.h1, dp.h1, true), host_arr(hp.h2, dp.h2, true), host_arr(hp.r, dp.r, true),
+                            host_arr(hp.I, dp.I, true), host_arr(hp.a1, dp.a1, false), host_arr(hp.a2, dp.a2, false),
+                            host_arr(hp.Kp, dp.Kp, false), host_arr(hp.t, dp.t, false), host_arr(hp.episode, dp.episode, false)};
     const bool single = cfg->obs_mode == PIME_WT_OBS_STACKING;
     auto launch = [&](int64_t off, int64_t cnt, const pime_rollout_args &a) {
-        pime_wt_state st = *d;
-        auto sh = [&](void *p, int elem) { return p ? (void *)((char *)p + off * elem) : nullptr; };
-        st.h1 = sh(d->h1, 4); st.h2 = sh(d->h2, 4); st.r = sh(d->r, 4); st.I = sh(d->I, 4);
-        st.a1 = sh(d->a1, 4); st.a2 = sh(d->a2, 4); st.Kp = sh(d->Kp, 4);
-        st.t = (int32_t *)sh(d->t, 4); st.episode = (uint32_t *)sh(d->episode, 4);
-        st.ep_return = sh(d->ep_return, 4); st.last_h1 = sh(d->last_h1, 4); st.last_h2 = sh(d->last_h2, 4);
         pime_rollout_args b = a;
-        shift_step_buffers(b, off, cfg->obs_mode == PIME_WT_OBS_INTEGRATOR ? 4 : 3, 4);   // (stacking: one slice, off = 0)
-        return wt_rollout_impl<float>(cfg, cnt, &st, &b, stream);
+        shift_step_buffers(b, off, S, sizeof(float));   // (stacking: one slice, off = 0)
+        return wt_rollout_launch<float>(cfg, cnt, dp.shifted(off), &b, stream);
     };
-    return host_pipelined_rollout(n, arr, 9, (float *)d->ep_return, ep_return_host, args, (cudaStream_t)stream, launch, single);
+    return host_pipelined_rollout(n, arr, 9, dp.ep_return, ep_return_host, args, (cudaStream_t)stream, launch, single);
 }
 
 // the slicing the host-buffer entries would use for n envs on the current device (148 SMs assumed when there is none):

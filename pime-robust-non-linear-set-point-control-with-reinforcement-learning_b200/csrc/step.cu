@@ -10,22 +10,6 @@ namespace pime {
 constexpr int kBlock = 256;
 
 // ---------------------------------------------------------------------------------------------- water tank
-template <typename T> struct WtPtrs {
-    T *h1, *h2, *r, *I, *a1, *a2, *Kp, *ep_return, *frames, *last_h1, *last_h2;
-    int32_t *t;
-    uint32_t *episode;
-};
-
-template <typename T> static WtPtrs<T> wt_ptrs(const pime_wt_state *s) {
-    WtPtrs<T> p;
-    p.h1 = (T *)s->h1; p.h2 = (T *)s->h2; p.r = (T *)s->r; p.I = (T *)s->I;
-    p.a1 = (T *)s->a1; p.a2 = (T *)s->a2; p.Kp = (T *)s->Kp;
-    p.ep_return = (T *)s->ep_return; p.frames = (T *)s->frames;
-    p.last_h1 = (T *)s->last_h1; p.last_h2 = (T *)s->last_h2;
-    p.t = s->t; p.episode = s->episode;
-    return p;
-}
-
 template <typename T>
 __device__ __forceinline__ void wt_write_obs(const WtConst<T> &c, const WtPtrs<T> &p, const WtEnv<T> &e, int64_t i, int64_t n,
                                              T *obs_out, bool fill_frames) {
@@ -62,10 +46,7 @@ __global__ void __launch_bounds__(kBlock) wt_step_kernel(WtConst<T> c, int64_t i
     const bool integ = c.obs_mode == PIME_WT_OBS_INTEGRATOR;
     for (int64_t i = i_begin + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         WtEnv<T> e;
-        e.h1 = p.h1[i]; e.h2 = p.h2[i]; e.r = p.r[i];
-        e.I = integ ? p.I[i] : (T)0;
-        e.a1 = p.a1[i]; e.a2 = p.a2[i]; e.Kp = p.Kp[i];
-        e.t = p.t[i];
+        p.load(e, i, integ);
         T nz1 = (T)0, nz2 = (T)0;
         if (noise1) {
             nz1 = noise1[i];
@@ -80,9 +61,7 @@ __global__ void __launch_bounds__(kBlock) wt_step_kernel(WtConst<T> c, int64_t i
         T rew;
         bool dn;
         wt_advance(c, e, action[i], nz1, nz2, rew, dn);
-        p.h1[i] = e.h1; p.h2[i] = e.h2;
-        if (integ) p.I[i] = e.I;
-        p.t[i] = e.t;
+        p.store_step(e, i, integ);
         if (p.ep_return) p.ep_return[i] += rew;
         reward[i] = rew;
         done[i] = dn ? 1 : 0;
@@ -220,62 +199,47 @@ __global__ void __launch_bounds__(kBlock) wt_reset_kernel(WtConst<T> c, int64_t 
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         if (mask && !mask[i]) continue;
         WtEnv<T> e;
-        e.a1 = p.a1[i]; e.a2 = p.a2[i]; e.Kp = p.Kp[i];
+        p.load_params(e, i);
         uint32_t ep = p.episode[i];
         double u[6];
         reset_uniforms(seed, env_offset + (uint64_t)i, ep, u);
         wt_reset(c, e, u, resample != 0);
         if (c.from_last) wt_reset_levels_from_last(e, u, p.last_h1[i], p.last_h2[i]);
         p.episode[i] = ep + 1;
-        p.a1[i] = e.a1; p.a2[i] = e.a2; p.Kp[i] = e.Kp;
-        p.h1[i] = e.h1; p.h2[i] = e.h2; p.r[i] = e.r;
-        if (p.I) p.I[i] = (T)0;
-        p.t[i] = 0;
+        p.store(e, i, p.I != nullptr);   // I = 0 and t = 0 after wt_reset; I is zeroed whenever the array exists
         if (p.ep_return) p.ep_return[i] = (T)0;
         wt_write_obs(c, p, e, i, n, obs_out, true);
     }
-}
-
-static int check_wt(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st) {
-    PIME_REQUIRE(cfg && st, "null config/state");
-    PIME_REQUIRE(n >= 0, "negative n");
-    PIME_REQUIRE(st->h1 && st->h2 && st->r && st->a1 && st->a2 && st->Kp && st->t && st->episode, "null state array");
-    PIME_REQUIRE(cfg->obs_mode >= 0 && cfg->obs_mode <= 2, "obs_mode");
-    PIME_REQUIRE(cfg->obs_mode != PIME_WT_OBS_INTEGRATOR || st->I, "integrator array missing");
-    PIME_REQUIRE(cfg->obs_mode != PIME_WT_OBS_STACKING || (st->frames && cfg->num_stack >= 1 && cfg->num_stack <= 10),
-                 "stacking needs frames and 1 <= num_stack <= 10");
-    PIME_REQUIRE(cfg->n_discrete >= 1 && cfg->reward_type >= 0 && cfg->reward_type <= 2, "n_discrete/reward_type");
-    PIME_REQUIRE(!cfg->reset_from_last_state || (st->last_h1 && st->last_h2), "reset_from_last_state needs last_h1/last_h2");
-    return PIME_OK;
 }
 
 template <typename T>
 static int wt_step_impl(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st, const T *action, const T *noise1,
                         const T *noise2, uint64_t seed, uint64_t env_offset, uint32_t tick, T *obs_out, T *reward, uint8_t *done,
                         void *stream) {
-    if (int rc = check_wt(cfg, n, st)) return rc;
+    if (int rc = validate_wt(cfg, n, st)) return rc;
     PIME_REQUIRE(action && reward && done, "null action/reward/done");
     PIME_REQUIRE((noise1 == nullptr) == (noise2 == nullptr), "noise1/noise2 must both be given or both be NULL");
     if (int rc = require_device()) return rc;
     if (n == 0) return PIME_OK;
+    const WtPtrs<T> p(*st);
     int64_t i_begin = 0;
     if constexpr (sizeof(T) == 4) {   // float: 4 envs per thread where layout and alignment allow, scalar kernel for the tail
         const bool vec_ok = cfg->obs_mode != PIME_WT_OBS_STACKING && n >= kVec && (obs_out == nullptr || n % kVec == 0) &&
-                            aligned16({st->h1, st->h2, st->r, st->I, st->a1, st->a2, st->Kp, st->t, st->ep_return, action, noise1,
-                                       noise2, obs_out, reward}) && ((uintptr_t)done & 3) == 0;
+                            aligned16({p.h1, p.h2, p.r, p.I, p.a1, p.a2, p.Kp, p.t, p.ep_return, action, noise1, noise2, obs_out,
+                                       reward}) && ((uintptr_t)done & 3) == 0;
         if (vec_ok) {
             const int64_t groups = n / kVec;
             wt_step_vec4_kernel<<<grid_for(groups, kVecBlock, 32), kVecBlock, 0, (cudaStream_t)stream>>>(
-                make_wt_const<float>(*cfg), groups, n, wt_ptrs<float>(st), (const float *)action, (const float *)noise1,
-                (const float *)noise2, seed, env_offset, tick, (float *)obs_out, (float *)reward, done);
+                make_wt_const<float>(*cfg), groups, n, p, (const float *)action, (const float *)noise1, (const float *)noise2, seed,
+                env_offset, tick, (float *)obs_out, (float *)reward, done);
             PIME_LAUNCH_CHECK();
             i_begin = groups * kVec;
             if (i_begin == n) return PIME_OK;
         }
     }
-    wt_step_kernel<T><<<grid_for(n - i_begin, kBlock), kBlock, 0, (cudaStream_t)stream>>>(make_wt_const<T>(*cfg), i_begin, n,
-                                                                                        wt_ptrs<T>(st), action, noise1, noise2, seed,
-                                                                                        env_offset, tick, obs_out, reward, done);
+    wt_step_kernel<T><<<grid_for(n - i_begin, kBlock), kBlock, 0, (cudaStream_t)stream>>>(make_wt_const<T>(*cfg), i_begin, n, p,
+                                                                                        action, noise1, noise2, seed, env_offset,
+                                                                                        tick, obs_out, reward, done);
     PIME_LAUNCH_CHECK();
     return PIME_OK;
 }
@@ -283,31 +247,16 @@ static int wt_step_impl(const pime_wt_config *cfg, int64_t n, const pime_wt_stat
 template <typename T>
 static int wt_reset_impl(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st, uint64_t seed, uint64_t env_offset,
                          int resample, const uint8_t *mask, T *obs_out, void *stream) {
-    if (int rc = check_wt(cfg, n, st)) return rc;
+    if (int rc = validate_wt(cfg, n, st)) return rc;
     if (int rc = require_device()) return rc;
     if (n == 0) return PIME_OK;
-    wt_reset_kernel<T><<<grid_for(n, kBlock), kBlock, 0, (cudaStream_t)stream>>>(make_wt_const<T>(*cfg), n, wt_ptrs<T>(st), seed,
+    wt_reset_kernel<T><<<grid_for(n, kBlock), kBlock, 0, (cudaStream_t)stream>>>(make_wt_const<T>(*cfg), n, WtPtrs<T>(*st), seed,
                                                                                 env_offset, resample, mask, obs_out);
     PIME_LAUNCH_CHECK();
     return PIME_OK;
 }
 
 // ---------------------------------------------------------------------------------------------- pH
-template <typename T> struct PhPtrs {
-    double *x, *A, *B, *last_x;   // fp64 in both flavours (plants.cuh)
-    T *y, *r, *I, *C, *qww, *qc, *ep_return;
-    int32_t *t;
-    uint32_t *episode;
-};
-
-template <typename T> static PhPtrs<T> ph_ptrs(const pime_ph_state *s) {
-    PhPtrs<T> p;
-    p.x = (double *)s->x; p.y = (T *)s->y; p.r = (T *)s->r; p.I = (T *)s->I;
-    p.A = (double *)s->A; p.B = (double *)s->B; p.C = (T *)s->C; p.qww = (T *)s->qww_V; p.qc = (T *)s->qc_V;
-    p.ep_return = (T *)s->ep_return; p.last_x = (double *)s->last_x; p.t = s->t; p.episode = s->episode;
-    return p;
-}
-
 template <typename T>
 __device__ __forceinline__ void ph_write_obs(const PhConst<T> &c, const PhEnv<T> &e, int64_t i, int64_t n, T *obs_out) {
     if (!obs_out) return;
@@ -323,16 +272,12 @@ __global__ void __launch_bounds__(kBlock) ph_step_kernel(PhConst<T> c, const T *
     const bool integ = c.integrator_mode != PIME_PH_NO_INTEGRATOR;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         PhEnv<T> e;
-        e.x = p.x[i]; e.r = p.r[i]; e.I = integ ? p.I[i] : (T)0;
-        e.A = p.A[i]; e.B = p.B[i]; e.C = p.C[i];
-        e.t = p.t[i];
+        p.load(e, i, integ);
         T rew;
         bool dn;
         bool ok = ph_advance(c, table, e, action[i], rew, dn);
         if (!ok && status) atomicMin(status, (int32_t)PIME_ERANGE);
-        p.x[i] = e.x; p.y[i] = e.y;
-        if (integ) p.I[i] = e.I;
-        p.t[i] = e.t;
+        p.store_step(e, i, integ);
         if (p.ep_return) p.ep_return[i] += rew;
         reward[i] = rew;
         done[i] = dn ? 1 : 0;
@@ -348,7 +293,7 @@ __global__ void __launch_bounds__(kBlock) ph_reset_kernel(PhConst<T> c, const T 
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         if (mask && !mask[i]) continue;
         PhEnv<T> e;
-        e.A = p.A[i]; e.B = p.B[i]; e.C = p.C[i];
+        p.load_system(e, i);
         T qww = p.qww[i], qc = p.qc[i];
         uint32_t ep = p.episode[i];
         double u[6];
@@ -357,10 +302,9 @@ __global__ void __launch_bounds__(kBlock) ph_reset_kernel(PhConst<T> c, const T 
         if (!ok && status) atomicMin(status, (int32_t)PIME_ERANGE);
         p.episode[i] = ep + 1;
         p.qww[i] = qww; p.qc[i] = qc;
-        p.A[i] = e.A; p.B[i] = e.B; p.C[i] = e.C;
-        p.x[i] = e.x; p.y[i] = e.y; p.r[i] = e.r;
-        if (p.I) p.I[i] = (T)0;
-        p.t[i] = 0;
+        p.store_system(e, i);                 // the new episode's system, set-point and step state
+        p.r[i] = e.r;
+        p.store_step(e, i, p.I != nullptr);   // I = 0 and t = 0 after ph_reset; I is zeroed whenever the array exists
         if (p.ep_return) p.ep_return[i] = (T)0;
         ph_write_obs(c, e, i, n, obs_out);
     }
@@ -369,10 +313,9 @@ __global__ void __launch_bounds__(kBlock) ph_reset_kernel(PhConst<T> c, const T 
 template <typename T>
 __global__ void __launch_bounds__(kBlock) ph_update_system_kernel(double sample_t, int64_t n, PhPtrs<T> p) {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        double A, B;
-        T C;
-        ph_update_system<T>(sample_t, p.qww[i], p.qc[i], A, B, C);
-        p.A[i] = A; p.B[i] = B; p.C[i] = C;
+        PhEnv<T> e;
+        ph_update_system<T>(sample_t, p.qww[i], p.qc[i], e.A, e.B, e.C);
+        p.store_system(e, i);
     }
 }
 
@@ -412,26 +355,14 @@ __global__ void __launch_bounds__(kBlock) ph_table_kernel(int table_len, double 
     if (t32) t32[i] = (float)v;
 }
 
-static int check_ph(const pime_ph_config *cfg, int64_t n, const pime_ph_state *st) {
-    PIME_REQUIRE(cfg && st, "null config/state");
-    PIME_REQUIRE(n >= 0, "negative n");
-    PIME_REQUIRE(st->x && st->y && st->r && st->A && st->B && st->C && st->qww_V && st->qc_V && st->t && st->episode,
-                 "null state array");
-    PIME_REQUIRE(cfg->integrator_mode >= 0 && cfg->integrator_mode <= 2, "integrator_mode");
-    PIME_REQUIRE(cfg->integrator_mode == PIME_PH_NO_INTEGRATOR || st->I, "integrator array missing");
-    PIME_REQUIRE(cfg->table_len > 1 && cfg->reward_type >= 0 && cfg->reward_type <= 2, "table_len/reward_type");
-    PIME_REQUIRE(!cfg->reset_from_last_state || st->last_x, "reset_from_last_state needs last_x");
-    return PIME_OK;
-}
-
 template <typename T>
 static int ph_step_impl(const pime_ph_config *cfg, const T *table, int64_t n, const pime_ph_state *st, const T *action,
                         T *obs_out, T *reward, uint8_t *done, int32_t *status, void *stream) {
-    if (int rc = check_ph(cfg, n, st)) return rc;
+    if (int rc = validate_ph(cfg, n, st)) return rc;
     PIME_REQUIRE(table && action && reward && done, "null table/action/reward/done");
     if (int rc = require_device()) return rc;
     if (n == 0) return PIME_OK;
-    ph_step_kernel<T><<<grid_for(n, kBlock), kBlock, 0, (cudaStream_t)stream>>>(make_ph_const<T>(*cfg), table, n, ph_ptrs<T>(st),
+    ph_step_kernel<T><<<grid_for(n, kBlock), kBlock, 0, (cudaStream_t)stream>>>(make_ph_const<T>(*cfg), table, n, PhPtrs<T>(*st),
                                                                                action, obs_out, reward, done, status);
     PIME_LAUNCH_CHECK();
     return PIME_OK;
@@ -440,21 +371,21 @@ static int ph_step_impl(const pime_ph_config *cfg, const T *table, int64_t n, co
 template <typename T>
 static int ph_reset_impl(const pime_ph_config *cfg, const T *table, int64_t n, const pime_ph_state *st, uint64_t seed,
                          uint64_t env_offset, int resample, const uint8_t *mask, T *obs_out, int32_t *status, void *stream) {
-    if (int rc = check_ph(cfg, n, st)) return rc;
+    if (int rc = validate_ph(cfg, n, st)) return rc;
     PIME_REQUIRE(table, "null table");
     if (int rc = require_device()) return rc;
     if (n == 0) return PIME_OK;
-    ph_reset_kernel<T><<<grid_for(n, kBlock), kBlock, 0, (cudaStream_t)stream>>>(make_ph_const<T>(*cfg), table, n, ph_ptrs<T>(st),
+    ph_reset_kernel<T><<<grid_for(n, kBlock), kBlock, 0, (cudaStream_t)stream>>>(make_ph_const<T>(*cfg), table, n, PhPtrs<T>(*st),
                                                                                 seed, env_offset, resample, mask, obs_out, status);
     PIME_LAUNCH_CHECK();
     return PIME_OK;
 }
 
 template <typename T> static int ph_update_impl(const pime_ph_config *cfg, int64_t n, const pime_ph_state *st, void *stream) {
-    if (int rc = check_ph(cfg, n, st)) return rc;
+    if (int rc = validate_ph(cfg, n, st)) return rc;
     if (int rc = require_device()) return rc;
     if (n == 0) return PIME_OK;
-    ph_update_system_kernel<T><<<grid_for(n, kBlock), kBlock, 0, (cudaStream_t)stream>>>(cfg->sample_t, n, ph_ptrs<T>(st));
+    ph_update_system_kernel<T><<<grid_for(n, kBlock), kBlock, 0, (cudaStream_t)stream>>>(cfg->sample_t, n, PhPtrs<T>(*st));
     PIME_LAUNCH_CHECK();
     return PIME_OK;
 }

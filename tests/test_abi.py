@@ -109,6 +109,32 @@ def test_compute_entry_points_fail_loudly_without_gpu(L):
         L.check(rc)
 
 
+def test_rollout_entries_reject_out_of_range_configs(L):
+    """The device and host-buffer rollout entries check the config as the step entries do: n_discrete < 1, reward_type
+    outside 0..2 and table_len <= 1 (with which the fused pH kernel would read before the start of its table) are
+    PIME_EINVAL, with or without a GPU.  n = 0 and a prior-only argument block: nothing would be launched if the check
+    were missing, and every pointer is non-null, so only the config can be what the call rejects."""
+    lib = L.lib()
+    buf = (C.c_double * 8)()
+    p = C.cast(buf, C.c_void_p)
+    ep_host = (C.c_float * 8)()
+    args = L.RolloutArgs(actor=None, priorK_host=(C.c_double * 4)(), T=1)
+    wst = L.WtState(**{f: p for f, _ in L.WtState._fields_})
+    pst = L.PhState(**{f: p for f, _ in L.PhState._fields_})
+    n0 = C.c_int64(0)
+    for bad in ({"n_discrete": 0}, {"reward_type": 3}):
+        cfg = L.wt_config(**bad)
+        for fn in (lib.pime_wt_rollout_f32, lib.pime_wt_rollout_f64):
+            assert fn(C.byref(cfg), n0, C.byref(wst), C.byref(args), None) == L.EINVAL, bad
+        rc = lib.pime_wt_rollout_host_f32(C.byref(cfg), n0, C.byref(wst), C.byref(wst), C.byref(args), ep_host, None)
+        assert rc == L.EINVAL, bad
+    cfg = L.ph_config(table_len=0)
+    for fn in (lib.pime_ph_rollout_f32, lib.pime_ph_rollout_f64):
+        assert fn(C.byref(cfg), p, n0, C.byref(pst), C.byref(args), None) == L.EINVAL
+    rc = lib.pime_ph_rollout_host_f32(C.byref(cfg), p, n0, C.byref(pst), C.byref(pst), C.byref(args), ep_host, None)
+    assert rc == L.EINVAL
+
+
 def test_product_never_touches_the_oracle():
     """The oracle is test infrastructure: nothing under the package or include/ may import, link or mention it."""
     pkg = os.path.join(ROOT, "pime-robust-non-linear-set-point-control-with-reinforcement-learning_b200")
