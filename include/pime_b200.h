@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define PIME_B200_ABI_VERSION 4
+#define PIME_B200_ABI_VERSION 5
 
 enum {
     PIME_OK = 0,
@@ -372,11 +372,6 @@ int pime_ppo_apply_grad(const pime_ppo_args *args, const float *grad, float scal
 int64_t pime_ppo_tc_work_bytes(const pime_actor_config *actor, int32_t batch);
 int pime_ppo_tc_layout(const pime_actor_config *actor, int32_t batch, int64_t *out34);
 int pime_ppo_grad_tc(const pime_ppo_args *args, void *work_tc, float *grad, void *stream);
-/* The same step in two calls, for overlapping the gradient all-reduce with compute in a data-parallel job: parts = 1 runs
- * everything but the actor's weight gradients -- afterwards grad[critic offset ...] (critic, a_std_log) is final and can be
- * all-reduced on another stream --, parts = 2 adds the actor's weight gradients (same stream, after parts = 1 of the same
- * step); parts = 3 is pime_ppo_grad_tc. */
-int pime_ppo_grad_tc_parts(const pime_ppo_args *args, void *work_tc, float *grad, int32_t parts, void *stream);
 int pime_ppo_close_step(const pime_ppo_args *args, void *stream);
 
 /* misc */

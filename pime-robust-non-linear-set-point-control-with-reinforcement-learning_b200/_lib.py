@@ -84,7 +84,7 @@ SYMBOLS = [
     "pime_wt_rollout_f32", "pime_wt_rollout_f64", "pime_ph_rollout_f32", "pime_ph_rollout_f64",
     "pime_gae_scan", "pime_reduce_episode_stats_f32", "pime_reduce_episode_stats_f64",
     "pime_ppo_theta_count", "pime_ppo_theta_layout", "pime_ppo_work_floats", "pime_ppo_transpose", "pime_ppo_step", "pime_ppo_apply_grad",
-    "pime_ppo_tc_work_bytes", "pime_ppo_tc_layout", "pime_ppo_grad_tc", "pime_ppo_grad_tc_parts", "pime_ppo_close_step",
+    "pime_ppo_tc_work_bytes", "pime_ppo_tc_layout", "pime_ppo_grad_tc", "pime_ppo_close_step",
     "pime_wt_rollout_host_f32", "pime_ph_rollout_host_f32", "pime_set_host_slices", "pime_host_slice_plan", "pime_abi_version", "pime_last_error", "pime_device_info", "pime_philox_probe",
 ]
 

@@ -13,8 +13,7 @@
 //                     copy and the moments.  Every gradient element is produced by exactly one thread: no atomics.
 //
 // fp32 throughout (the reference trains in fp32); sums run in a different order than cuBLAS, nothing else differs.
-#include "pime_common.cuh"
-#include "tc_mlp.cuh"
+#include "ppo_common.cuh"
 
 namespace pime {
 namespace ppo {
@@ -27,6 +26,7 @@ constexpr int kMaxStages = 8;          // slabs in flight (cp.async.bulk ring): 
 constexpr int kMaxPasses = 12;
 constexpr int kMaxLayers = 10;
 constexpr int kOutAcc = 272;           // floats per output-layer accumulator (H + 1 <= 257)
+static_assert(State::kGOut + 2 * kOutAcc <= 1024, "the two output-layer accumulators must fit in the state block");
 constexpr int kXInt = 4;               // modular: aligned copy of the integrator observation inside the gathered row
 constexpr int kXStride = 32;      // gathered state row (S <= 32)
 constexpr int kRowVals = 8;       // per-row scalars in shared memory
@@ -46,12 +46,6 @@ struct LayerDesc {
     int tile0, tn, tk;    // first tile, tiles along N and K
 };
 
-struct NetDims {
-    int kind, S, H, So, LA;   // LA: activation columns per row
-    int theta_off;            // first parameter of this net in theta
-    int src[12];              // offsets of the state_dict tensors inside the net's parameters
-};
-
 struct StreamPass {       // one hidden-layer weight matrix streamed through the shared-memory ring, 16 rows per slab
     int off;              // offset in theta (backward: torch layout [N][K]) or theta_t (forward: [K][N])
     int transposed;       // 1: theta_t
@@ -60,7 +54,8 @@ struct StreamPass {       // one hidden-layer weight matrix streamed through the
 };
 
 struct StepParams {
-    NetDims act, cri;
+    Net act, cri;
+    int LA[2];                // activation columns per row of the actor and the critic (act_cols)
     int n_layers, n_tiles;
     int n_passes;
     StreamPass pass[kMaxPasses];
@@ -71,11 +66,7 @@ struct StepParams {
     const int64_t *idx;
     int B;
     float ratio_clip, lambda_entropy, lr, beta1, beta2, eps;
-    int *step_dev;            // Adam step count so far (the step being taken is *step_dev + 1)
-    unsigned *ticket;
-    float *g_astd;            // accumulated gradient of a_std_log
-    float *adam_c;            // [2]: lr / bias_correction1 and 1 / sqrt(bias_correction2) of the step being taken (written by the rows kernel)
-    float *g_out;             // [2][kOutAcc]: accumulated gradients of the two output layers Linear(H -> 1): weight[H], bias
+    State st;                 // adam_c is written by the rows kernel; g_out holds [2][kOutAcc]: weight[H], bias
     float *X, *ACT_A, *DZ_A, *ACT_C, *DZ_C, *DOUT;
     float *loss_ring;
     int ring_len;
@@ -329,7 +320,7 @@ __device__ __forceinline__ float block_sum(float v, float *scratch) {
 // forward (and its mirror, the data-gradient chain) of one net on R rows held in shared memory.  Compute warps only; the
 // hidden layers take their weights from the ring in the order fill_passes() lists them.
 template <int R>
-__device__ __forceinline__ void net_forward(Ring &ring, const NetDims &d, const float *__restrict__ th, const float *__restrict__ tt,
+__device__ __forceinline__ void net_forward(Ring &ring, const Net &d, const float *__restrict__ th, const float *__restrict__ tt,
                                             const float *sX, float *A, int as, float *out, int out_stride, float *part) {
     const int H = d.H;
     if (d.kind == PIME_ACTOR_MODULAR) {   // net_residual.py:150-170
@@ -357,7 +348,7 @@ __device__ __forceinline__ void net_forward(Ring &ring, const NetDims &d, const 
 }
 
 template <int R>
-__device__ __forceinline__ void net_backward(Ring &ring, const NetDims &d, const float *__restrict__ th, const float *A, float *Z, int as,
+__device__ __forceinline__ void net_backward(Ring &ring, const Net &d, const float *__restrict__ th, const float *A, float *Z, int as,
                                              const float *d_out, int d_stride, float *part) {
     const int H = d.H;
     if (d.kind == PIME_ACTOR_MODULAR) {
@@ -379,8 +370,6 @@ __device__ __forceinline__ void net_backward(Ring &ring, const NetDims &d, const
     sync_compute();
 }
 
-__device__ __forceinline__ void adam_prepare(const StepParams &p);
-
 // grid = (row tiles, 2): blockIdx.y = 0 runs the actor (forward, policy objectives, backward), 1 the critic.  The two
 // nets share nothing but the gathered rows (obj_united = obj_actor + obj_critic / (std + 1e-5) is a sum), so splitting
 // them halves the chain of dependent layers a CTA walks through.
@@ -388,8 +377,8 @@ template <int R>
 __global__ void __launch_bounds__(kRowsThreads, 1) ppo_rows_kernel(const StepParams p) {
     extern __shared__ __align__(128) float sm[];
     const int net = blockIdx.y;
-    const NetDims &d = net == 0 ? p.act : p.cri;
-    const int LA = d.LA;
+    const Net &d = net == 0 ? p.act : p.cri;
+    const int LA = p.LA[net];
     Ring ring;
     constexpr int kStages = R <= 4 ? kMaxStages : 4;
     ring.buf = sm;                          // [kStages][kSlabFloats]
@@ -429,7 +418,7 @@ __global__ void __launch_bounds__(kRowsThreads, 1) ppo_rows_kernel(const StepPar
     const int B = p.B;
     const int b0 = blockIdx.x * R;
 
-    if (blockIdx.x == 0 && net == 0 && tid == 0) adam_prepare(p);
+    if (blockIdx.x == 0 && net == 0 && tid == 0) adam_prepare(p.st.step, p.lr, p.beta1, p.beta2, p.st.adam_c);
     float inv_cs = 0.0f;
     if (net == 1) {   // r_sum.std() of the minibatch (agent.py:652; unbiased), two passes
         float s = 0.0f;
@@ -471,32 +460,10 @@ __global__ void __launch_bounds__(kRowsThreads, 1) ppo_rows_kernel(const StepPar
     if (tid < R) {
         float *rv = sV + tid * kRowVals;
         const bool live = b0 + tid < B;
-        const float invB = 1.0f / (float)B;
-        float o_act = 0.0f, o_cri = 0.0f, o_ent = 0.0f, g_asl = 0.0f;
-        if (net == 0) {
-            const float asl = __ldg(p.theta + p.n_theta - 1);
-            const float std = expf(asl);
-            const float dd = (rv[4] - rv[0]) / std;
-            const float lp = -(asl + 0.9189385332046727f + dd * dd * 0.5f);      // compute_logprob (net_residual.py:62-66)
-            const float ratio = expf(lp - rv[2]);
-            const float adv = rv[3];
-            const float s1 = adv * ratio;
-            const float s2 = adv * fminf(fmaxf(ratio, 1.0f - p.ratio_clip), 1.0f + p.ratio_clip);
-            const float sur = fminf(s1, s2);
-            const float elp = expf(lp);
-            const float ent = elp * lp;
-            const float g_lp = (-(s1 <= s2 ? s1 : 0.0f) + p.lambda_entropy * (ent + elp)) * invB;   // d united / d new_logprob
-            rv[6] = live ? g_lp * (-dd / std) : 0.0f;                            // d united / d a_avg
-            o_act = live ? (-sur + p.lambda_entropy * ent) * invB : 0.0f;
-            o_ent = live ? ent * invB : 0.0f;
-            g_asl = live ? g_lp * (dd * dd - 1.0f) : 0.0f;
-        } else {
-            const float e = rv[4] - rv[1];
-            const float ae = fabsf(e);
-            const float l1 = ae < 1.0f ? 0.5f * e * e : ae - 0.5f;               // SmoothL1Loss, beta = 1
-            rv[6] = live ? fminf(fmaxf(e, -1.0f), 1.0f) * invB * inv_cs : 0.0f;  // d united / d value
-            o_cri = live ? l1 * invB : 0.0f;
-        }
+        const RowObj ob = row_objectives(net, rv[4], rv[0], rv[1], rv[2], rv[3], __ldg(p.theta + p.n_theta - 1), inv_cs,
+                                         p.ratio_clip, p.lambda_entropy, 1.0f / (float)B, live);
+        rv[6] = ob.d_out;
+        float o_act = ob.o_act, o_cri = ob.o_cri, o_ent = ob.o_ent, g_asl = ob.g_asl;
 #pragma unroll
         for (int o = 1; o < R; o <<= 1) {   // R is a power of two <= 32, the rows sit in one warp
             o_act += __shfl_xor_sync((1u << R) - 1u, o_act, o);
@@ -505,9 +472,9 @@ __global__ void __launch_bounds__(kRowsThreads, 1) ppo_rows_kernel(const StepPar
             g_asl += __shfl_xor_sync((1u << R) - 1u, g_asl, o);
         }
         if (tid == 0) {
-            float *row = p.loss_ring + (size_t)(*p.step_dev % p.ring_len) * 4;
+            float *row = p.loss_ring + (size_t)(*p.st.step % p.ring_len) * 4;
             atomicAdd(row + 0, o_act + o_cri * inv_cs);
-            if (net == 0) { atomicAdd(row + 1, o_act); atomicAdd(row + 3, o_ent); atomicAdd(p.g_astd, g_asl); }
+            if (net == 0) { atomicAdd(row + 1, o_act); atomicAdd(row + 3, o_ent); atomicAdd(p.st.g_astd, g_asl); }
             else atomicAdd(row + 2, o_cri);
         }
     }
@@ -521,7 +488,7 @@ __global__ void __launch_bounds__(kRowsThreads, 1) ppo_rows_kernel(const StepPar
         float g = 0.0f;
 #pragma unroll
         for (int r = 0; r < R; ++r) g = fmaf(sV[r * kRowVals + 6], k < d.H ? Alast[r * LA + k] : 1.0f, g);
-        atomicAdd(p.g_out + net * kOutAcc + k, g);
+        atomicAdd(p.st.g_out + net * kOutAcc + k, g);
     }
 
     // rows -> scratch (inputs of the weight-gradient kernel)
@@ -536,34 +503,6 @@ __global__ void __launch_bounds__(kRowsThreads, 1) ppo_rows_kernel(const StepPar
         if (net == 0 && tid < kXStride) p.X[(size_t)b * kXStride + tid] = sX[r * kXStride + tid];
         if (tid == 0) p.DOUT[(size_t)b * 2 + net] = sV[r * kRowVals + 6];
     }
-}
-
-// torch.optim.Adam (fused implementation's arithmetic): exp_avg = lerp(exp_avg, g, 1-b1); exp_avg_sq = b2 v + (1-b2) g^2;
-// p -= (lr / bc1) * exp_avg / (sqrt(exp_avg_sq) / sqrt(bc2) + eps)
-struct AdamCoef {
-    float lr_bc1, inv_sqrt_bc2, one_m_b1, b2, one_m_b2, eps;
-};
-// the two step-dependent coefficients (double-precision pow) are computed once per step, by one thread of the rows kernel
-__device__ __forceinline__ void adam_prepare(const StepParams &p) {
-    const int t = *p.step_dev + 1;
-    const double bc1 = 1.0 - pow((double)p.beta1, (double)t), bc2 = 1.0 - pow((double)p.beta2, (double)t);
-    p.adam_c[0] = (float)((double)p.lr / bc1);
-    p.adam_c[1] = (float)(1.0 / sqrt(bc2));
-}
-__device__ __forceinline__ AdamCoef adam_coef(const StepParams &p) {
-    AdamCoef c;
-    c.lr_bc1 = p.adam_c[0];
-    c.inv_sqrt_bc2 = p.adam_c[1];
-    c.one_m_b1 = 1.0f - p.beta1; c.b2 = p.beta2; c.one_m_b2 = 1.0f - p.beta2; c.eps = p.eps;
-    return c;
-}
-// every operation is spelled out (no compiler-chosen FMA contraction): the fused weight-gradient epilogue and the
-// stand-alone Adam kernel of the data-parallel path must produce bit-identical parameters and moments
-__device__ __forceinline__ float adam_update(const AdamCoef &c, float g, float theta, float &m, float &v) {
-    m = __fmaf_rn(c.one_m_b1, __fsub_rn(g, m), m);                              // lerp(exp_avg, grad, 1 - beta1)
-    v = __fmaf_rn(__fmul_rn(c.one_m_b2, g), g, __fmul_rn(c.b2, v));             // beta2 v + (1 - beta2) g g
-    const float den = __fmaf_rn(sqrtf(v), c.inv_sqrt_bc2, c.eps);
-    return __fsub_rn(theta, __fdiv_rn(__fmul_rn(c.lr_bc1, m), den));
 }
 
 __device__ __forceinline__ void cp_async16(void *dst_smem, const void *src, bool valid) {
@@ -592,12 +531,12 @@ __global__ void __launch_bounds__(kThreads) ppo_wgrad_kernel(const StepParams p)
     const int B = p.B;
     const float *dz; int dz_stride;
     if (L.dz_col < 0) { dz = p.DOUT + L.net; dz_stride = 2; }
-    else if (L.net == 0) { dz = p.DZ_A + L.dz_col; dz_stride = p.act.LA; }
-    else { dz = p.DZ_C + L.dz_col; dz_stride = p.cri.LA; }
+    else if (L.net == 0) { dz = p.DZ_A + L.dz_col; dz_stride = p.LA[0]; }
+    else { dz = p.DZ_C + L.dz_col; dz_stride = p.LA[1]; }
     const float *in; int in_stride, in_avail;   // in_avail: readable columns of an input row (the products beyond K are dropped)
     if (L.in_col < 0) { in = p.X + L.x_col; in_stride = kXStride; in_avail = kXStride - L.x_col; }
-    else if (L.net == 0) { in = p.ACT_A + L.in_col; in_stride = p.act.LA; in_avail = L.K; }
-    else { in = p.ACT_C + L.in_col; in_stride = p.cri.LA; in_avail = L.K; }
+    else if (L.net == 0) { in = p.ACT_A + L.in_col; in_stride = p.LA[0]; in_avail = L.K; }
+    else { in = p.ACT_C + L.in_col; in_stride = p.LA[1]; in_avail = L.K; }
     // 16-byte cp.async needs aligned rows: true for every hidden layer; the output layers (dZ = DOUT, stride 2) and the
     // integrator branch's first layer (input column So of X) take the scalar path -- they are a handful of tiny tiles
     const bool fast = L.dz_col >= 0 && (L.in_col >= 0 || (L.x_col & 3) == 0);
@@ -661,8 +600,7 @@ __global__ void __launch_bounds__(kThreads) ppo_wgrad_kernel(const StepParams p)
         __syncthreads();
     }
 
-    const int t = *p.step_dev + 1;
-    const AdamCoef c = adam_coef(p);
+    const AdamCoef c = adam_coef(p.st.adam_c, p.beta1, p.beta2, p.eps);
     auto apply = [&](int idx, int idx_t, float g) {
         if (p.grad_out) { p.grad_out[idx] = g; return; }
         float m = p.m[idx], v = p.v[idx];
@@ -684,27 +622,25 @@ __global__ void __launch_bounds__(kThreads) ppo_wgrad_kernel(const StepParams p)
     // the last CTA to finish closes the step: a_std_log, step counter, the next ring row, the accumulators
     __threadfence();
     __syncthreads();
-    if (tid == 0) is_last = atomicAdd(p.ticket, 1u) == (unsigned)p.n_tiles - 1u;
+    if (tid == 0) is_last = atomicAdd(p.st.ticket, 1u) == (unsigned)p.n_tiles - 1u;
     __syncthreads();
     if (is_last) {
         __threadfence();
         for (int j = tid; j < 2 * (p.act.H + 1); j += kThreads) {   // the output layers, accumulated by the rows kernel
             const int net = j / (p.act.H + 1), k = j % (p.act.H + 1);
-            const NetDims &d = net == 0 ? p.act : p.cri;
+            const Net &d = net == 0 ? p.act : p.cri;
             const int wi = d.kind == PIME_ACTOR_MODULAR ? 10 : 6;
             const int idx = d.theta_off + (k < d.H ? d.src[wi] + k : d.src[wi + 1]);
-            float *acc_p = p.g_out + net * kOutAcc + k;
+            float *acc_p = p.st.g_out + net * kOutAcc + k;
             apply(idx, idx, *reinterpret_cast<volatile float *>(acc_p));
             *acc_p = 0.0f;
         }
         if (tid == 0) {
-            const float g = *reinterpret_cast<volatile float *>(p.g_astd);
+            const float g = *reinterpret_cast<volatile float *>(p.st.g_astd);
             apply(p.n_theta - 1, p.n_theta - 1, g);
-            *p.g_astd = 0.0f;
-            *p.ticket = 0u;
-            float *nxt = p.loss_ring + (size_t)((*p.step_dev + 1) % p.ring_len) * 4;
-            nxt[0] = nxt[1] = nxt[2] = nxt[3] = 0.0f;
-            *p.step_dev = t;
+            *p.st.g_astd = 0.0f;
+            *p.st.ticket = 0u;
+            close_step(p.st.step, p.loss_ring, p.ring_len);
         }
     }
 }
@@ -715,7 +651,7 @@ __global__ void __launch_bounds__(kThreads) ppo_wgrad_kernel(const StepParams p)
 // rows kernel of the same step (adam_prepare), so the bias corrections belong to the step whose gradient this is.
 __global__ void __launch_bounds__(kThreads) ppo_adam_kernel(const StepParams p, const float *__restrict__ grad, float scale) {
     const LayerDesc L = p.layer[blockIdx.y];
-    const AdamCoef c = adam_coef(p);
+    const AdamCoef c = adam_coef(p.st.adam_c, p.beta1, p.beta2, p.eps);
     const int nw = L.N * L.K, total = nw + L.N;
     for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < total; j += gridDim.x * blockDim.x) {
         int idx, idx_t;
@@ -746,18 +682,7 @@ __global__ void ppo_transpose_kernel(StepParams p) {
 }
 
 // ------------------------------------------------------------------------------------------------ host side
-static bool fill_net(const pime_actor_config &c, int theta_off, NetDims &d) {
-    tc::PackLayout L;
-    if (!tc::make_pack_layout(c, L)) return false;
-    d.kind = c.kind; d.S = c.state_dim; d.H = c.mid_dim;
-    d.So = c.kind == PIME_ACTOR_MODULAR ? c.state_dim - c.integrator_dim : c.state_dim;
-    d.LA = c.kind == PIME_ACTOR_MODULAR ? 4 * c.mid_dim : 3 * c.mid_dim;
-    d.theta_off = theta_off;
-    for (int j = 0; j < 12; ++j) d.src[j] = L.src[j];
-    return true;
-}
-
-static void add_layer(StepParams &p, int net, const NetDims &d, int N, int K, int w, int b, int dz_col, int in_col, int x_col) {
+static void add_layer(StepParams &p, int net, const Net &d, int N, int K, int w, int b, int dz_col, int in_col, int x_col) {
     LayerDesc &L = p.layer[p.n_layers++];
     L.net = net; L.N = N; L.K = K; L.w_off = d.theta_off + d.src[w]; L.b_off = d.theta_off + d.src[b];
     L.dz_col = dz_col; L.in_col = in_col; L.x_col = x_col;
@@ -766,7 +691,7 @@ static void add_layer(StepParams &p, int net, const NetDims &d, int N, int K, in
     p.n_tiles += L.tn * L.tk;
 }
 
-static void add_net_layers(StepParams &p, int net, const NetDims &d) {
+static void add_net_layers(StepParams &p, int net, const Net &d) {
     const int H = d.H;
     if (d.kind == PIME_ACTOR_MODULAR) {
         add_layer(p, net, d, H, d.So, 0, 1, 0, -1, 0);                      // other_net.0
@@ -783,7 +708,7 @@ static void add_net_layers(StepParams &p, int net, const NetDims &d) {
     }
 }
 
-static void add_pass(StepParams &p, const NetDims &d, int src, bool transposed, int rows, int cols) {
+static void add_pass(StepParams &p, const Net &d, int src, bool transposed, int rows, int cols) {
     StreamPass &q = p.pass[p.n_passes++];
     q.net = &d == &p.cri ? 1 : 0;
     q.off = d.theta_off + d.src[src]; q.transposed = transposed ? 1 : 0; q.rows = rows; q.cols = cols;
@@ -791,7 +716,7 @@ static void add_pass(StepParams &p, const NetDims &d, int src, bool transposed, 
 // the order in which net_forward / net_backward consume the ring
 static void fill_passes(StepParams &p) {
     for (int dir = 0; dir < 2; ++dir)
-        for (const NetDims *d : {&p.act, &p.cri}) {
+        for (const Net *d : {&p.act, &p.cri}) {
             const int H = d->H, Hh = H / 2;
             if (d->kind == PIME_ACTOR_MODULAR) {
                 if (dir == 0) { add_pass(p, *d, 2, true, H, Hh); add_pass(p, *d, 6, true, H, Hh); add_pass(p, *d, 8, true, H, H); }
@@ -803,17 +728,15 @@ static void fill_passes(StepParams &p) {
         }
 }
 
-static int64_t critic_offset(int64_t actor_params) { return (actor_params + 3) & ~(int64_t)3; }   // 16-byte aligned for the bulk copies
+// activation columns per row of a net in shared memory and in the scratch rows
+static int act_cols(const Net &d) { return d.kind == PIME_ACTOR_MODULAR ? 4 * d.H : 3 * d.H; }
 
 static int fill_params(const pime_ppo_args *a, StepParams &p) {
     PIME_REQUIRE(a && a->actor, "null ppo args / actor config");
     PIME_REQUIRE(a->actor->kind == PIME_ACTOR_PLAIN || a->actor->kind == PIME_ACTOR_MODULAR, "actor kind");
     p = StepParams{};
-    pime_actor_config cc{PIME_CRITIC_ADV, a->actor->state_dim, a->actor->mid_dim, 0};
-    PIME_REQUIRE(fill_net(*a->actor, 0, p.act), "unsupported actor dimensions");
-    const int64_t pa = pime_actor_param_count(a->actor), pc = pime_actor_param_count(&cc);
-    PIME_REQUIRE(fill_net(cc, (int)critic_offset(pa), p.cri), "unsupported critic dimensions");
-    p.n_theta = (int)(critic_offset(pa) + pc + 1);
+    PIME_REQUIRE(theta_layout(*a->actor, p.act, p.cri, p.n_theta), "unsupported network dimensions");
+    p.LA[0] = act_cols(p.act); p.LA[1] = act_cols(p.cri);
     add_net_layers(p, 0, p.act);
     add_net_layers(p, 1, p.cri);
     fill_passes(p);
@@ -821,11 +744,11 @@ static int fill_params(const pime_ppo_args *a, StepParams &p) {
     return PIME_OK;
 }
 
-static int64_t work_floats_per_row(const StepParams &p) { return kXStride + 2 * (int64_t)(p.act.LA + p.cri.LA) + 2; }
+static int64_t work_floats_per_row(const StepParams &p) { return kXStride + 2 * (int64_t)(p.LA[0] + p.LA[1]) + 2; }
 
 template <int R> static int launch_rows(const StepParams &p, cudaStream_t s) {
     constexpr int kStages = R <= 4 ? kMaxStages : 4;
-    const int LAmax = p.act.LA > p.cri.LA ? p.act.LA : p.cri.LA;
+    const int LAmax = p.LA[0] > p.LA[1] ? p.LA[0] : p.LA[1];
     const size_t smem = sizeof(float) * (size_t)(kStages * kSlabFloats + R * (kXStride + 2 * LAmax + kRowVals) + 8 + 1024 * R) +
                         2 * kStages * sizeof(uint64_t);
     auto kern = ppo_rows_kernel<R>;
@@ -849,12 +772,12 @@ int64_t pime_ppo_theta_count(const pime_actor_config *actor) {
 
 int pime_ppo_theta_layout(const pime_actor_config *actor, int64_t *out) {
     PIME_REQUIRE(actor && out, "null pointer");
-    pime_actor_config cc{PIME_CRITIC_ADV, actor->state_dim, actor->mid_dim, 0};
-    const int64_t pa = pime_actor_param_count(actor), pc = pime_actor_param_count(&cc);
-    PIME_REQUIRE(pa > 0 && pc > 0, "unsupported network dimensions");
-    out[0] = ppo::critic_offset(pa);
-    out[1] = out[0] + pc;
-    out[2] = out[1] + 1;
+    ppo::Net act, cri;
+    int n_theta;
+    PIME_REQUIRE(ppo::theta_layout(*actor, act, cri, n_theta), "unsupported network dimensions");
+    out[0] = cri.theta_off;
+    out[1] = n_theta - 1;
+    out[2] = n_theta;
     return PIME_OK;
 }
 
@@ -884,37 +807,32 @@ int pime_ppo_apply_grad(const pime_ppo_args *a, const float *grad, float scale, 
     PIME_REQUIRE(a->theta && a->theta_t && a->adam_m && a->adam_v && a->state && grad, "null theta / theta_t / moments / state / grad");
     if (int rc = require_device()) return rc;
     p.lr = a->lr; p.beta1 = a->beta1; p.beta2 = a->beta2; p.eps = a->eps;
-    p.step_dev = (int *)a->state;
-    p.adam_c = (float *)a->state + 8;
+    p.st = ppo::State(a->state);
     ppo::ppo_adam_kernel<<<dim3(32, p.n_layers), ppo::kThreads, 0, (cudaStream_t)stream>>>(p, grad, scale);
     PIME_LAUNCH_CHECK();
     return PIME_OK;
 }
 
 int pime_ppo_step(const pime_ppo_args *a, void *stream) {
+    if (int rc = ppo::validate_ppo_args(a)) return rc;
     ppo::StepParams p;
     if (int rc = ppo::fill_params(a, p)) return rc;
-    PIME_REQUIRE(a->theta && a->theta_t && a->state && a->work, "null theta / theta_t / state / work");
+    PIME_REQUIRE(a->theta_t && a->work, "null theta_t / work");
     PIME_REQUIRE(a->grad_out || (a->adam_m && a->adam_v), "Adam moments are required unless grad_out is given");
-    PIME_REQUIRE(a->buf_state && a->buf_action && a->buf_r_sum && a->buf_logprob && a->buf_advantage && a->idx, "null replay tensor");
-    PIME_REQUIRE(a->batch >= 2 && a->batch <= (1 << 20), "batch must be in [2, 2^20]");
-    PIME_REQUIRE(a->loss_ring && a->ring_len >= 2, "loss ring");
     if (int rc = require_device()) return rc;
     p.buf_state = a->buf_state; p.buf_action = a->buf_action; p.buf_r_sum = a->buf_r_sum; p.buf_logprob = a->buf_logprob;
     p.buf_adv = a->buf_advantage; p.idx = a->idx; p.B = a->batch;
     p.ratio_clip = a->ratio_clip; p.lambda_entropy = a->lambda_entropy;
     p.lr = a->lr; p.beta1 = a->beta1; p.beta2 = a->beta2; p.eps = a->eps;
-    p.step_dev = (int *)a->state; p.ticket = (unsigned *)a->state + 1; p.g_astd = (float *)a->state + 2;
-    p.g_out = (float *)a->state + 16;
-    p.adam_c = (float *)a->state + 8;
+    p.st = ppo::State(a->state);
     p.loss_ring = a->loss_ring; p.ring_len = a->ring_len;
     const int64_t B = a->batch;
     float *w = a->work;
     p.X = w; w += B * ppo::kXStride;
-    p.ACT_A = w; w += B * p.act.LA;
-    p.DZ_A = w; w += B * p.act.LA;
-    p.ACT_C = w; w += B * p.cri.LA;
-    p.DZ_C = w; w += B * p.cri.LA;
+    p.ACT_A = w; w += B * p.LA[0];
+    p.DZ_A = w; w += B * p.LA[0];
+    p.ACT_C = w; w += B * p.LA[1];
+    p.DZ_C = w; w += B * p.LA[1];
     p.DOUT = w;
     cudaStream_t s = (cudaStream_t)stream;
     const int R = B <= 128 ? 2 : (B <= 256 ? 4 : 8);   // at most 128 CTAs (64 per net) up to 512 rows: one wave

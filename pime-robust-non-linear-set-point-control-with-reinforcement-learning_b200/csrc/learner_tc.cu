@@ -23,8 +23,7 @@
 // GEMMs, the objectives kernel (clipped surrogate / entropy / SmoothL1, output layers, their gradients), data-gradient
 // GEMMs, weight-gradient GEMMs into a flat fp32 gradient in theta's layout; the caller all-reduces that buffer when the job
 // is data parallel and applies Adam with pime_ppo_apply_grad (learner.cu).
-#include "pime_common.cuh"
-#include "tc_mlp.cuh"
+#include "ppo_common.cuh"
 
 namespace pime {
 namespace tcl {
@@ -32,6 +31,7 @@ namespace tcl {
 using tc::bulk_g2s; using tc::elect_one; using tc::fence_barrier_init; using tc::make_desc; using tc::mbar_arrive_expect_tx;
 using tc::mbar_init; using tc::mbar_wait; using tc::mma_commit; using tc::mma_f16; using tc::smem_u32; using tc::tc_fence_after;
 using tc::tc_fence_before; using tc::tmem_alloc; using tc::tmem_dealloc; using tc::tmem_ld32;
+using ppo::Net;
 
 constexpr int kBlk = 16384;        // bytes of one T-format block: [8 unit groups][128 rows][8 fp16]
 constexpr int kUg = 2048;          // bytes of one unit group: 128 rows x 16 B
@@ -195,10 +195,9 @@ __device__ __forceinline__ float epi_piece(const GemmProb &P, int rt, int nt, in
     return colsum<32>(v, lane, col);          // col == lane
 }
 
-#ifndef PIME_TC_GEMM_STAGES
-#define PIME_TC_GEMM_STAGES 1
-#endif
-constexpr int kGemmStages = PIME_TC_GEMM_STAGES;   // 1: 65 KB per CTA, three CTAs per SM overlap one another's load / MMA / epilogue phases
+// 1: 65 KB per CTA, three CTAs per SM overlap one another's load / MMA / epilogue phases (3 stages, one CTA per SM: 2.21 ms
+// against 1.46 ms for this single stage)
+constexpr int kGemmStages = 1;
 constexpr int kGemmStage = 4 * kBlk;                      // A_hi, A_lo, W_hi, W_lo
 constexpr int kGemmSmem = kGemmStages * kGemmStage + 1024;
 constexpr int kGemmThreads = 320;                         // warp 0: TMA, warp 1: MMA, warps 2-9: epilogue (two threads per row: column halves)
@@ -472,12 +471,7 @@ __global__ void __launch_bounds__(128) gather_kernel(const StepCommon c, uint8_t
     const int rt = blockIdx.x, row = threadIdx.x, b = rt * 128 + row;
     const bool live = b < c.B;
     const int64_t i = live ? __ldg(c.idx + b) : 0;
-    if (rt == 0 && row == 0) {   // bias corrections of the step being taken (torch.optim.Adam), as learner.cu:adam_prepare
-        const int t = *c.step_dev + 1;
-        const double bc1 = 1.0 - pow((double)c.beta1, (double)t), bc2 = 1.0 - pow((double)c.beta2, (double)t);
-        c.adam_c[0] = (float)((double)c.lr / bc1);
-        c.adam_c[1] = (float)(1.0 / sqrt(bc2));
-    }
+    if (rt == 0 && row == 0) ppo::adam_prepare(c.step_dev, c.lr, c.beta1, c.beta2, c.adam_c);
 #pragma unroll
     for (int ug = 0; ug < 8; ++ug) {
         float x[8];
@@ -558,28 +552,10 @@ __global__ void __launch_bounds__(256) out_obj_kernel(const StepCommon c, const 
         float out = __ldg(c.theta + N.b_off);
         for (int ug = 0; ug < UG; ++ug) out += part[ug][row];
         const float4 rv = reinterpret_cast<const float4 *>(c.rowv)[b];   // action, r_sum, old logprob, advantage
-        const float invB = 1.0f / (float)c.B;
-        float o_act = 0.0f, o_cri = 0.0f, o_ent = 0.0f, g_asl = 0.0f, d = 0.0f;
-        if (net == 0) {
-            const float asl = __ldg(c.theta + c.n_theta - 1);
-            const float std = expf(asl);
-            const float dd = (out - rv.x) / std;
-            const float lp = -(asl + 0.9189385332046727f + dd * dd * 0.5f);      // compute_logprob (net_residual.py:62-66)
-            const float ratio = expf(lp - rv.z);
-            const float s1 = rv.w * ratio;
-            const float s2 = rv.w * fminf(fmaxf(ratio, 1.0f - c.ratio_clip), 1.0f + c.ratio_clip);
-            const float sur = fminf(s1, s2);
-            const float elp = expf(lp);
-            const float ent = elp * lp;
-            const float g_lp = (-(s1 <= s2 ? s1 : 0.0f) + c.lambda_entropy * (ent + elp)) * invB;   // d united / d new_logprob
-            if (live) { d = g_lp * (-dd / std); o_act = (-sur + c.lambda_entropy * ent) * invB; o_ent = ent * invB; g_asl = g_lp * (dd * dd - 1.0f); }
-        } else {
-            const float inv_cs = *c.inv_cs;
-            const float e = out - rv.y;
-            const float ae = fabsf(e);
-            const float l1 = ae < 1.0f ? 0.5f * e * e : ae - 0.5f;               // SmoothL1Loss, beta = 1
-            if (live) { d = fminf(fmaxf(e, -1.0f), 1.0f) * invB * inv_cs; o_cri = l1 * invB; }
-        }
+        const ppo::RowObj ob = ppo::row_objectives(net, out, rv.x, rv.y, rv.z, rv.w, __ldg(c.theta + c.n_theta - 1), *c.inv_cs,
+                                                   c.ratio_clip, c.lambda_entropy, 1.0f / (float)c.B, live);
+        const float d = ob.d_out;
+        float o_act = ob.o_act, o_cri = ob.o_cri, o_ent = ob.o_ent, g_asl = ob.g_asl;
         dout[row] = d;
         float db = d;
 #pragma unroll
@@ -625,27 +601,9 @@ __global__ void __launch_bounds__(256) out_obj_kernel(const StepCommon c, const 
     if (tid == 0) atomicAdd(c.grad + N.b_off, gw[H]);
 }
 
-__global__ void close_step_kernel(int *step_dev, float *loss_ring, int ring_len) {
-    const int t = *step_dev + 1;
-    float *nxt = loss_ring + (size_t)(t % ring_len) * 4;
-    nxt[0] = nxt[1] = nxt[2] = nxt[3] = 0.0f;
-    *step_dev = t;
-}
+__global__ void close_step_kernel(int *step_dev, float *loss_ring, int ring_len) { ppo::close_step(step_dev, loss_ring, ring_len); }
 
 // ------------------------------------------------------------------------------------------------ host side: the step's program
-struct Net {
-    int kind, S, H, So, theta_off;
-    int src[12];
-};
-static bool fill_net(const pime_actor_config &cfg, int theta_off, Net &d) {
-    tc::PackLayout L;
-    if (!tc::make_pack_layout(cfg, L)) return false;
-    d.kind = cfg.kind; d.S = cfg.state_dim; d.H = cfg.mid_dim; d.theta_off = theta_off;
-    d.So = cfg.kind == PIME_ACTOR_MODULAR ? cfg.state_dim - cfg.integrator_dim : cfg.state_dim;
-    for (int j = 0; j < 12; ++j) d.src[j] = L.src[j];
-    return true;
-}
-
 // work buffer layout (bytes).  Activation / gradient matrices are [row_tiles * 128][units] in T-format (hi + lo: 4 B per element).
 struct Plan {
     Net act, cri;
@@ -667,15 +625,8 @@ static bool build_plan(const pime_actor_config &actor, int B, Plan &pl) {
     const int H = actor.mid_dim, S = actor.state_dim;
     if (!(H == 128 || H == 256) || S > 56) return false;
     if (!(actor.kind == PIME_ACTOR_MODULAR || actor.kind == PIME_ACTOR_PLAIN)) return false;
-    pime_actor_config cc{PIME_CRITIC_ADV, S, H, 0, 0};
-    if (!fill_net(actor, 0, pl.act)) return false;
-    tc::PackLayout La, Lc;
-    tc::make_pack_layout(actor, La);
-    tc::make_pack_layout(cc, Lc);
-    const int cri_off = (La.param_count + 3) & ~3;
-    if (!fill_net(cc, cri_off, pl.cri)) return false;
+    if (!ppo::theta_layout(actor, pl.act, pl.cri, pl.n_theta)) return false;
     pl.B = B; pl.H = H; pl.row_tiles = (B + 127) / 128;
-    pl.n_theta = cri_off + Lc.param_count + 1;
     size_t o = 0;
     auto take = [&](size_t bytes) { size_t r = o; o += (bytes + 1023) & ~(size_t)1023; return r; };
     pl.X = take(mat_bytes(pl.row_tiles, 64));
@@ -796,21 +747,15 @@ int pime_ppo_tc_layout(const pime_actor_config *actor, int32_t batch, int64_t *o
 int pime_ppo_close_step(const pime_ppo_args *a, void *stream) {
     PIME_REQUIRE(a && a->state && a->loss_ring && a->ring_len >= 2, "null ppo args / state / loss ring");
     if (int rc = require_device()) return rc;
-    tcl::close_step_kernel<<<1, 1, 0, (cudaStream_t)stream>>>((int *)a->state, a->loss_ring, a->ring_len);
+    tcl::close_step_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(ppo::State(a->state).step, a->loss_ring, a->ring_len);
     PIME_LAUNCH_CHECK();
     return PIME_OK;
 }
 
-}  // extern "C"
-
-// parts: bit 0 = everything but the actor's weight gradients (after it the critic's part of grad, the bias gradients of both
-// nets and d a_std_log are complete), bit 1 = the actor's weight gradients (needs bit 0 of the same step to have run).
-static int ppo_grad_tc_impl(const pime_ppo_args *a, void *work_tc, float *grad, void *stream, int parts) {
+int pime_ppo_grad_tc(const pime_ppo_args *a, void *work_tc, float *grad, void *stream) {
     using namespace tcl;
-    PIME_REQUIRE(a && a->actor && work_tc && grad, "null ppo args / work / grad");
-    PIME_REQUIRE(a->theta && a->state && a->loss_ring && a->ring_len >= 2, "null theta / state / loss ring");
-    PIME_REQUIRE(a->buf_state && a->buf_action && a->buf_r_sum && a->buf_logprob && a->buf_advantage && a->idx, "null replay tensor");
-    PIME_REQUIRE(a->batch >= 2 && a->batch <= (1 << 20), "batch must be in [2, 2^20]");
+    if (int rc = ppo::validate_ppo_args(a)) return rc;
+    PIME_REQUIRE(work_tc && grad, "null work_tc / grad");
     Plan pl;
     PIME_REQUIRE(build_plan(*a->actor, a->batch, pl), "the tensor-core learner needs mid_dim 128 or 256 and a plain / modular actor");
     PIME_REQUIRE(((uintptr_t)work_tc & 255) == 0, "work_tc must be 256-byte aligned");
@@ -825,7 +770,8 @@ static int ppo_grad_tc_impl(const pime_ppo_args *a, void *work_tc, float *grad, 
     c.buf_state = a->buf_state; c.buf_action = a->buf_action; c.buf_r_sum = a->buf_r_sum; c.buf_logprob = a->buf_logprob; c.buf_adv = a->buf_advantage;
     c.idx = a->idx; c.B = a->batch; c.S = a->actor->state_dim; c.row_tiles = RT;
     c.ratio_clip = a->ratio_clip; c.lambda_entropy = a->lambda_entropy; c.lr = a->lr; c.beta1 = a->beta1; c.beta2 = a->beta2;
-    c.step_dev = (int *)a->state; c.adam_c = (float *)a->state + 8; c.loss_ring = a->loss_ring; c.ring_len = a->ring_len;
+    const ppo::State st(a->state);
+    c.step_dev = st.step; c.adam_c = st.adam_c; c.loss_ring = a->loss_ring; c.ring_len = a->ring_len;
     c.grad = grad; c.n_theta = pl.n_theta; c.rowv = (float *)(w + pl.rowv); c.inv_cs = (float *)(w + pl.inv_cs); c.theta = th;
 
     float pow2B = 1.0f;
@@ -836,7 +782,6 @@ static int ppo_grad_tc_impl(const pime_ppo_args *a, void *work_tc, float *grad, 
 
     const Net &A = pl.act, &C = pl.cri;
     const int actA = ACT_TANH, actC = ACT_RELU;
-    if (parts & 1) {
     PIME_CUDA(cudaMemsetAsync(grad, 0, (size_t)pl.n_theta * sizeof(float), s));
     split_weights_kernel<<<dim3(64, pl.ws.n), 256, 0, s>>>(pl.ws, th, w);
     PIME_LAUNCH_CHECK();
@@ -914,19 +859,13 @@ static int ppo_grad_tc_impl(const pime_ppo_args *a, void *work_tc, float *grad, 
         g.p[g.n++] = bwd(w, pl, un_c, pl.Z[6], 0, HC, pl.WT[6], HC, H, actC, pl.A[5], pl.Z[5], nullptr);
         if (int rc = run_gemm(g)) return rc;
     }
-    }   // parts & 1 (the critic's weight gradients below belong to it too)
-    // ---- weight gradients: all matrices in one launch, or the critic's (bit 0) and the actor's (bit 1) in separate launches
-    // so that a data-parallel caller can all-reduce the critic's part while the actor's is still being computed
-    for (int part = 1; part <= 2; part <<= 1) {
-        if (!(parts & part)) continue;
-        if (parts == 3 && part == 2) break;                 // one launch did both
-        const bool do_act = parts == 3 || part == 2, do_cri = parts == 3 || part == 1;
+    // ---- weight gradients: all matrices in one launch
+    {
         WgBatch g{};
         g.grad = grad; g.row_tiles = RT;
         auto W_ = [&](const Net &d, int j) { return d.theta_off + d.src[j]; };
         const int S = c.S;
-        if (!do_act) {
-        } else if (mod) {
+        if (mod) {
             g.p[g.n++] = wg(w, pl, un_a, pl.Z[0], 0, H, pl.X, 1, 64, W_(A, 0), A.So, 0, A.So, kBiasCol, W_(A, 1));                 // other_net.0
             g.p[g.n++] = wg(w, pl, un_a, pl.Z[1], 0, H, pl.X, 1, 64, W_(A, 4), S - A.So, A.So, S, kBiasCol, W_(A, 5));            // integrator_net.0
             g.p[g.n++] = wg(w, pl, un_a, pl.Z[2], 0, Hh, pl.A[0], HC, H, W_(A, 2), H, 0, H, -1, 0);                               // other_net.2
@@ -937,28 +876,15 @@ static int ppo_grad_tc_impl(const pime_ppo_args *a, void *work_tc, float *grad, 
             g.p[g.n++] = wg(w, pl, un_a, pl.Z[2], 0, H, pl.A[0], HC, H, W_(A, 2), H, 0, H, -1, 0);
             g.p[g.n++] = wg(w, pl, un_a, pl.Z[4], 0, H, pl.A[2], HC, H, W_(A, 4), H, 0, H, -1, 0);
         }
-        if (do_cri) {
-            g.p[g.n++] = wg(w, pl, un_c, pl.Z[5], 0, H, pl.X, 1, 64, W_(C, 0), S, 0, S, kBiasCol, W_(C, 1));
-            g.p[g.n++] = wg(w, pl, un_c, pl.Z[6], 0, H, pl.A[5], HC, H, W_(C, 2), H, 0, H, -1, 0);
-            g.p[g.n++] = wg(w, pl, un_c, pl.Z[7], 0, H, pl.A[6], HC, H, W_(C, 4), H, 0, H, -1, 0);
-        }
+        g.p[g.n++] = wg(w, pl, un_c, pl.Z[5], 0, H, pl.X, 1, 64, W_(C, 0), S, 0, S, kBiasCol, W_(C, 1));
+        g.p[g.n++] = wg(w, pl, un_c, pl.Z[6], 0, H, pl.A[5], HC, H, W_(C, 2), H, 0, H, -1, 0);
+        g.p[g.n++] = wg(w, pl, un_c, pl.Z[7], 0, H, pl.A[6], HC, H, W_(C, 4), H, 0, H, -1, 0);
         int mx = 1;
         for (int i = 0; i < g.n; ++i) mx = g.p[i].m_tiles * g.p[i].n_tiles > mx ? g.p[i].m_tiles * g.p[i].n_tiles : mx;
         int split = RT < 32 ? RT : 32;
         if (int rc = launch_batch(wgrad_mn_kernel, g, dim3(mx, split, g.n), kWgThreads, kWgSmem, s)) return rc;
     }
     return PIME_OK;
-}
-
-extern "C" {
-
-int pime_ppo_grad_tc(const pime_ppo_args *a, void *work_tc, float *grad, void *stream) {
-    return ppo_grad_tc_impl(a, work_tc, grad, stream, 3);
-}
-
-int pime_ppo_grad_tc_parts(const pime_ppo_args *a, void *work_tc, float *grad, int32_t parts, void *stream) {
-    PIME_REQUIRE(parts == 1 || parts == 2 || parts == 3, "parts must be 1, 2 or 3");
-    return ppo_grad_tc_impl(a, work_tc, grad, stream, parts);
 }
 
 }  // extern "C"

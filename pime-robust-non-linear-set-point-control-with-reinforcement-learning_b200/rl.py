@@ -224,7 +224,6 @@ class FusedLearner:
         self.grad = None        # distributed: flat gradient of this rank's minibatch, all-reduced before the Adam kernel
         self.work_tc = None     # scratch of the tensor-core step (activations / gradients of one minibatch in T-format)
         self.steps = 0          # host mirror of the device step count
-        self._comm = self._ev = None   # data parallel: side stream / event of the overlapped all-reduce
         self._args = None
         self._step_fn = V.L.lib().pime_ppo_step
         self._keys = (V.ActorPack.KEYS[act.kind], V.ActorPack.KEYS["critic"])
@@ -276,42 +275,49 @@ class FusedLearner:
             for t, o in self._slices(act, cri):
                 t.copy_(self.theta[o:o + t.numel()].view_as(t))
 
-    def step(self, data, idx, agent, grad_out=None):
-        """One minibatch step on rows ``idx`` of data = (state, action, r_sum, logprob, advantage)."""
+    def _bind(self, data, idx, agent, tc, grad_out=None):
+        """The argument block (by reference) for rows ``idx`` of data = (state, action, r_sum, logprob, advantage) on the
+        SIMT step or, with ``tc``, the tensor-core step.  It is rebuilt, and its scratch grown, only when a data pointer, the
+        batch size, the path or grad_out changes; the scalars follow the agent / optimizer on every call (a learning-rate
+        change between two update_net calls must reach the kernels)."""
         C, L = self.C, self.L
         B = int(idx.numel())
-        key = (tuple(t.data_ptr() for t in data), B, None if grad_out is None else grad_out.data_ptr())
-        if self._args is None or self._args[0] != key:      # the argument block is rebuilt only when a pointer changes
+        key = (tuple(t.data_ptr() for t in data), B, tc, None if grad_out is None else grad_out.data_ptr())
+        if self._args is None or self._args[0] != key:
             state, action, r_sum, logprob, advantage = data
-            need = int(L.lib().pime_ppo_work_floats(C.byref(self.cfg), C.c_int32(B)))
-            if self.work is None or self.work.numel() < need:
-                self.work = torch.empty(need, dtype=torch.float32, device=self.device)
-            grp = agent.optimizer.param_groups[0]
+            if tc:
+                need = int(L.lib().pime_ppo_tc_work_bytes(C.byref(self.cfg), C.c_int32(B)))
+                if need < 0:
+                    raise ValueError("the tensor-core learner needs net_dim 128 or 256")
+                if self.work_tc is None or self.work_tc.numel() < need:
+                    self.work_tc = torch.empty(need, dtype=torch.uint8, device=self.device)
+            else:
+                need = int(L.lib().pime_ppo_work_floats(C.byref(self.cfg), C.c_int32(B)))
+                if self.work is None or self.work.numel() < need:
+                    self.work = torch.empty(need, dtype=torch.float32, device=self.device)
             a = L.PpoArgs(actor=C.pointer(self.cfg), theta=L.ptr(self.theta), theta_t=L.ptr(self.theta_t), adam_m=L.ptr(self.m),
                           adam_v=L.ptr(self.v), grad_out=L.ptr(grad_out), buf_state=L.ptr(state), buf_action=L.ptr(action),
                           buf_r_sum=L.ptr(r_sum), buf_logprob=L.ptr(logprob), buf_advantage=L.ptr(advantage), batch=B,
-                          ratio_clip=agent.ratio_clip, lambda_entropy=agent.lambda_entropy, lr=grp["lr"],
-                          beta1=grp["betas"][0], beta2=grp["betas"][1], eps=grp["eps"], state=L.ptr(self.state),
-                          work=L.ptr(self.work), loss_ring=L.ptr(self.loss_ring), ring_len=self.RING)
+                          state=L.ptr(self.state), work=None if tc else L.ptr(self.work), loss_ring=L.ptr(self.loss_ring),
+                          ring_len=self.RING)
             self._args = (key, a, C.byref(a), data)
         a = self._args[1]
         a.idx = idx.data_ptr()
-        self._hyper(a, agent)
-        stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-        L.check(self._step_fn(self._args[2], stream))
-        if grad_out is not None and grad_out is self.grad:   # data parallel: mean gradient over the job, then Adam
-            torch.distributed.all_reduce(grad_out)
-            L.check(L.lib().pime_ppo_apply_grad(self._args[2], L.ptr(grad_out), C.c_float(1.0 / torch.distributed.get_world_size()),
-                                                stream))
-        self.steps += 1
-
-    @staticmethod
-    def _hyper(a, agent):
-        """The scalars of the cached argument block follow the agent / optimizer (a learning-rate change between two
-        update_net calls must reach the kernels)."""
         grp = agent.optimizer.param_groups[0]
         a.ratio_clip, a.lambda_entropy = agent.ratio_clip, agent.lambda_entropy
         a.lr, a.beta1, a.beta2, a.eps = grp["lr"], grp["betas"][0], grp["betas"][1], grp["eps"]
+        return self._args[2]
+
+    def step(self, data, idx, agent, grad_out=None):
+        """One minibatch step on rows ``idx`` of data = (state, action, r_sum, logprob, advantage)."""
+        C, L = self.C, self.L
+        args = self._bind(data, idx, agent, False, grad_out)
+        stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+        L.check(self._step_fn(args, stream))
+        if grad_out is not None and grad_out is self.grad:   # data parallel: mean gradient over the job, then Adam
+            torch.distributed.all_reduce(grad_out)
+            L.check(L.lib().pime_ppo_apply_grad(args, L.ptr(grad_out), C.c_float(1.0 / torch.distributed.get_world_size()), stream))
+        self.steps += 1
 
     def dist_grad(self):
         if self.grad is None:
@@ -321,55 +327,17 @@ class FusedLearner:
     def step_tc(self, data, idx, agent, distributed=False):
         """One minibatch step on the tensor cores: pime_ppo_grad_tc -> (all-reduce) -> pime_ppo_apply_grad -> close."""
         C, L = self.C, self.L
-        B = int(idx.numel())
+        args = self._bind(data, idx, agent, True)
         grad = self.dist_grad()
-        key = ("tc", tuple(t.data_ptr() for t in data), B)
-        if self._args is None or self._args[0] != key:
-            state, action, r_sum, logprob, advantage = data
-            need = int(L.lib().pime_ppo_tc_work_bytes(C.byref(self.cfg), C.c_int32(B)))
-            if need < 0:
-                raise ValueError("the tensor-core learner needs net_dim 128 or 256")
-            if self.work_tc is None or self.work_tc.numel() < need:
-                self.work_tc = torch.empty(need, dtype=torch.uint8, device=self.device)
-            grp = agent.optimizer.param_groups[0]
-            a = L.PpoArgs(actor=C.pointer(self.cfg), theta=L.ptr(self.theta), theta_t=L.ptr(self.theta_t), adam_m=L.ptr(self.m),
-                          adam_v=L.ptr(self.v), grad_out=None, buf_state=L.ptr(state), buf_action=L.ptr(action),
-                          buf_r_sum=L.ptr(r_sum), buf_logprob=L.ptr(logprob), buf_advantage=L.ptr(advantage), batch=B,
-                          ratio_clip=agent.ratio_clip, lambda_entropy=agent.lambda_entropy, lr=grp["lr"],
-                          beta1=grp["betas"][0], beta2=grp["betas"][1], eps=grp["eps"], state=L.ptr(self.state),
-                          work=None, loss_ring=L.ptr(self.loss_ring), ring_len=self.RING)
-            self._args = (key, a, C.byref(a), data)
-        a = self._args[1]
-        a.idx = idx.data_ptr()
-        self._hyper(a, agent)
         stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
         lib = L.lib()
+        L.check(lib.pime_ppo_grad_tc(args, L.ptr(self.work_tc), L.ptr(grad), stream))
         scale = 1.0
-        if distributed and not getattr(agent, "tc_allreduce_overlap", False):
-            L.check(lib.pime_ppo_grad_tc(self._args[2], L.ptr(self.work_tc), L.ptr(grad), stream))
+        if distributed:
             torch.distributed.all_reduce(grad)               # one flat 1.07-MB all-reduce between two of this library's kernels
             scale = 1.0 / torch.distributed.get_world_size()
-        elif distributed:
-            # agent.tc_allreduce_overlap: the critic's half of the flat gradient (+ d a_std_log) is final before the actor's
-            # weight-gradient launch: its NCCL all-reduce runs on a side stream under that launch, the actor's half follows on
-            # the main stream.  Measured on 8 B200s (131 072-row minibatches): 340.6 ms per 200 minibatches against 337.0 ms
-            # for the single all-reduce -- two launches + two collectives cost more than the ~25 us they hide; off by default.
-            dist, main = torch.distributed, torch.cuda.current_stream()
-            if self._comm is None:
-                self._comm, self._ev = torch.cuda.Stream(), torch.cuda.Event()
-            L.check(lib.pime_ppo_grad_tc_parts(self._args[2], L.ptr(self.work_tc), L.ptr(grad), C.c_int32(1), stream))
-            self._ev.record(main)
-            with torch.cuda.stream(self._comm):
-                self._comm.wait_event(self._ev)
-                dist.all_reduce(grad[self.cri_off:])
-            L.check(lib.pime_ppo_grad_tc_parts(self._args[2], L.ptr(self.work_tc), L.ptr(grad), C.c_int32(2), stream))
-            dist.all_reduce(grad[:self.cri_off])
-            main.wait_stream(self._comm)
-            scale = 1.0 / dist.get_world_size()
-        else:
-            L.check(lib.pime_ppo_grad_tc(self._args[2], L.ptr(self.work_tc), L.ptr(grad), stream))
-        L.check(lib.pime_ppo_apply_grad(self._args[2], L.ptr(grad), C.c_float(scale), stream))
-        L.check(lib.pime_ppo_close_step(self._args[2], stream))
+        L.check(lib.pime_ppo_apply_grad(args, L.ptr(grad), C.c_float(scale), stream))
+        L.check(lib.pime_ppo_close_step(args, stream))
         self.steps += 1
 
     def losses(self, first, count):
@@ -511,7 +479,6 @@ class AgentPPO:
         self.use_fused_learner = True   # pime_ppo_step (two launches per minibatch) when FusedLearner.eligible
         self.fused_max_batch = 4096     # the fp32 SIMT kernels (pime_ppo_step) up to here
         self.tc_learner_min_batch = 2048  # from here on the tcgen05 step (pime_ppo_grad_tc) when net_dim is 128 or 256
-        self.tc_allreduce_overlap = False  # data parallel: all-reduce the critic's half under the actor's weight-gradient launch
         self._fused = None
         self.learner_path = None        # which minibatch step the last update_net ran (reported by bench.py)
         self.value_fp32_max_rows = 1 << 20

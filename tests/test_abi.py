@@ -37,7 +37,7 @@ def test_every_declared_symbol_is_exported(L):
     assert not missing, f"declared in the header but not exported: {missing}"
     assert sorted(L.SYMBOLS) == declared, "pime_b200._lib.SYMBOLS must list exactly the header's functions"
     lib = L.lib()
-    assert lib.pime_abi_version() == 4
+    assert lib.pime_abi_version() == 5
 
 
 def test_struct_layouts_match_header(L, tmp_path):

@@ -474,11 +474,9 @@ for it in range(2):
     steps = agent.explore_env(env, buf, n * 200, 1.0, 0.99)
     agent.update_net(buf, steps, 256, 2)
 assert "all-reduce" in agent.learner_path, agent.learner_path
-# large minibatches: the tensor-core step, its critic-half all-reduce overlapped with the actor's weight-gradient launch
+# large minibatches: the tensor-core step, one flat all-reduce of its gradient before the Adam kernel
 agent.update_net(buf, steps, 2048, 2)
 assert "pime_ppo_grad_tc" in agent.learner_path and "all-reduce" in agent.learner_path, agent.learner_path
-agent.tc_allreduce_overlap = True                  # the two-part gradient call with the critic's half reduced on a side stream
-agent.update_net(buf, steps, 2048, 2)
 flat = torch.cat([p.detach().reshape(-1) for p in list(agent.act.parameters()) + list(agent.cri.parameters())])
 ref = flat.clone(); dist.broadcast(ref, 0)
 assert torch.equal(flat, ref), "replicas diverged"

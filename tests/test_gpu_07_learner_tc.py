@@ -54,20 +54,10 @@ def _decode(work, off, row_tiles, units):
 def _grad_tc(f, data, idx, agent):
     """pime_ppo_grad_tc only (no Adam): the flat gradient and the scratch buffer."""
     import pime_b200._lib as L
-    f._args = None
-    B = int(idx.numel())
-    need = int(L.lib().pime_ppo_tc_work_bytes(C.byref(f.cfg), C.c_int32(B)))
-    assert need > 0
-    f.work_tc = torch.zeros(need, dtype=torch.uint8, device="cuda")
+    args = f._bind(data, idx, agent, True)
+    f.work_tc.zero_()
     grad = torch.zeros_like(f.theta)
-    grp = agent.optimizer.param_groups[0]
-    state, action, r_sum, logprob, advantage = data
-    a = L.PpoArgs(actor=C.pointer(f.cfg), theta=L.ptr(f.theta), theta_t=L.ptr(f.theta_t), adam_m=L.ptr(f.m), adam_v=L.ptr(f.v),
-                  grad_out=None, buf_state=L.ptr(state), buf_action=L.ptr(action), buf_r_sum=L.ptr(r_sum), buf_logprob=L.ptr(logprob),
-                  buf_advantage=L.ptr(advantage), idx=L.ptr(idx), batch=B, ratio_clip=agent.ratio_clip, lambda_entropy=agent.lambda_entropy,
-                  lr=grp["lr"], beta1=grp["betas"][0], beta2=grp["betas"][1], eps=grp["eps"], state=L.ptr(f.state), work=None,
-                  loss_ring=L.ptr(f.loss_ring), ring_len=f.RING)
-    L.check(L.lib().pime_ppo_grad_tc(C.byref(a), L.ptr(f.work_tc), L.ptr(grad), L.stream_ptr()))
+    L.check(L.lib().pime_ppo_grad_tc(args, L.ptr(f.work_tc), L.ptr(grad), L.stream_ptr()))
     torch.cuda.synchronize()
     return grad, f.work_tc
 
@@ -158,35 +148,6 @@ def test_tc_steps_track_the_autograd_path(kind, S, H, B):
             continue
         d = (p1 - p2).detach().abs()
         assert float(d.max()) <= 0.6 * lr and float(d.mean()) <= 0.02 * lr, n1
-
-
-def test_tc_gradient_in_two_parts_equals_the_single_call():
-    """pime_ppo_grad_tc_parts: parts = 1 leaves the critic's half of the flat gradient (+ d a_std_log) final -- the all-reduce
-    of that half overlaps the actor's weight-gradient launch in a data-parallel job --, parts = 2 completes the actor's half."""
-    import pime_b200._lib as L
-    import pime_b200.rl as R
-    (agent,) = _agents("modular", 4, 256, 1)
-    data = _data(agent, 4)
-    idx = torch.randint(data[0].shape[0], size=(5000,), device="cuda")
-    f = R.FusedLearner(agent.act, agent.cri, 4, 256, agent.device)
-    f.load(agent.act, agent.cri)
-    whole, _ = _grad_tc(f, data, idx, agent)
-    whole = whole.clone()
-    f.step_tc(data, idx, agent)                              # builds the cached argument block; its Adam step is irrelevant here
-    f.load(agent.act, agent.cri)
-    args, stream = f._args[2], L.stream_ptr()
-    grad = torch.full_like(f.theta, 7.0)
-    L.check(L.lib().pime_ppo_grad_tc_parts(args, L.ptr(f.work_tc), L.ptr(grad), C.c_int32(1), stream))
-    torch.cuda.synchronize()
-    half = grad.clone()
-    scale = float(whole.abs().max())
-    assert float((half[f.cri_off:] - whole[f.cri_off:]).abs().max()) <= 1e-6 * scale      # critic + a_std_log: final (atomics reorder only)
-    ws = [o for t, o in f._slices(agent.act, agent.cri) if t.dim() == 2 and t.shape[0] > 1 and o < f.cri_off]   # (net.2 [1, H] comes from out_obj)
-    assert all(float(half[o:o + 8].abs().max()) == 0.0 for o in ws)                       # the actor's weight matrices are still zero
-    L.check(L.lib().pime_ppo_grad_tc_parts(args, L.ptr(f.work_tc), L.ptr(grad), C.c_int32(2), stream))
-    torch.cuda.synchronize()
-    assert float((grad - whole).abs().max()) <= 1e-6 * scale
-    assert torch.equal(grad[f.cri_off:], half[f.cri_off:])                                # part 2 does not touch the critic's half
 
 
 def test_update_net_takes_the_tensor_core_path_for_large_batches():
