@@ -280,6 +280,41 @@ int pime_wt_rollout_f64(const pime_wt_config *cfg, int64_t n, const pime_wt_stat
 int pime_ph_rollout_f32(const pime_ph_config *cfg, const float *table, int64_t n, const pime_ph_state *st, const pime_rollout_args *args, void *stream);
 int pime_ph_rollout_f64(const pime_ph_config *cfg, const double *table, int64_t n, const pime_ph_state *st, const pime_rollout_args *args, void *stream);
 
+/* ---------------------------------------------------------------------------------------------------------
+ * Scheduled rollout: the set-point staircase (utils/test.py:70-347, :1369-1407) as one fused launch.  args->T = K L
+ * steps run as K segments of L steps; segment k tracks setpoints_host[k].  Each segment begins (right after an env is
+ * loaded, and after step k L - 1) with
+ *
+ *   keep the plant state (h1, h2 / x); reset() keyed as pime_*_reset (episode counter, reset_all when resample_params
+ *   is 1, reset_r when 0; reset_from_last_state; t = 0, I = 0, ep_return = 0; stacking frames from the reset's state);
+ *   restore the kept state (pH: y = table lookup under the new C, PIME_ERANGE past the table); r = setpoints_host[k].
+ *
+ * Per env and segment, in fp64, with y the controlled output after a step (h2 / y) and e = r - y:
+ *   metrics[0][k][i] = sum of rewards (unscaled)     metrics[1][k][i] = sum of |e| over the segment's steps
+ *   metrics[2][k][i] = |e| after the last step       metrics[3][k][i] = max(0, max of d (y - r)),  d = +1 if r >= y at
+ *                                                                         the segment begin, else -1
+ * The replay rows, env_action, stats and status keep their meaning; args->auto_reset must be 0.  The schedule is checked
+ * with the config, state and argument block (PIME_EINVAL, also without a device and for n = 0).
+ * ------------------------------------------------------------------------------------------------------- */
+#define PIME_MAX_SEGMENTS 16
+typedef struct pime_schedule {
+    int32_t num_segments;           /* K, 1 .. PIME_MAX_SEGMENTS                                             */
+    int32_t segment_steps;          /* L >= 1; args->T must equal K * L                                      */
+    int32_t resample_params;        /* segment begin = reset_all (1) / reset_r (0)                           */
+    int32_t reserved0;
+    const double *setpoints_host;   /* [K] HOST doubles                                                      */
+    double *metrics;                /* device double[4][K][n] (ret, iae, final_err, overshoot); may be NULL  */
+} pime_schedule;
+
+int pime_wt_rollout_schedule_f32(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st, const pime_rollout_args *args,
+                                 const pime_schedule *sched, void *stream);
+int pime_wt_rollout_schedule_f64(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st, const pime_rollout_args *args,
+                                 const pime_schedule *sched, void *stream);
+int pime_ph_rollout_schedule_f32(const pime_ph_config *cfg, const float *table, int64_t n, const pime_ph_state *st,
+                                 const pime_rollout_args *args, const pime_schedule *sched, void *stream);
+int pime_ph_rollout_schedule_f64(const pime_ph_config *cfg, const double *table, int64_t n, const pime_ph_state *st,
+                                 const pime_rollout_args *args, const pime_schedule *sched, void *stream);
+
 /* Per-env GAE / reward-to-go reverse scan over a time-major replay (AgentPPO.compute_reward_gae
  * agent.py:685-708 without the final normalisation): reward, mask, value are [T][n] with element stride
  * `stride` floats (4 for buf_other columns, 1 for dense); r_sum, adv are dense [T][n]. */

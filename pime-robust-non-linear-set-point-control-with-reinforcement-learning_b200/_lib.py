@@ -66,6 +66,14 @@ class RolloutArgs(C.Structure):
                 ("buf_state", vp), ("buf_other", vp), ("env_action", vp), ("stats", vp), ("status", vp), ("ld", C.c_int64)]
 
 
+MAX_SEGMENTS = 16
+
+
+class Schedule(C.Structure):
+    _fields_ = [("num_segments", C.c_int32), ("segment_steps", C.c_int32), ("resample_params", C.c_int32),
+                ("reserved0", C.c_int32), ("setpoints_host", C.POINTER(C.c_double)), ("metrics", vp)]
+
+
 class PpoArgs(C.Structure):
     _fields_ = [("actor", C.POINTER(ActorConfig)), ("theta", vp), ("theta_t", vp), ("adam_m", vp), ("adam_v", vp),
                 ("grad_out", vp), ("buf_state", vp), ("buf_action", vp), ("buf_r_sum", vp), ("buf_logprob", vp),
@@ -82,6 +90,7 @@ SYMBOLS = [
     "pime_prior_action_f32", "pime_prior_action_f64",
     "pime_actor_param_count", "pime_actor_pack_bytes", "pime_actor_block_list", "pime_actor_pack", "pime_actor_forward",
     "pime_wt_rollout_f32", "pime_wt_rollout_f64", "pime_ph_rollout_f32", "pime_ph_rollout_f64",
+    "pime_wt_rollout_schedule_f32", "pime_wt_rollout_schedule_f64", "pime_ph_rollout_schedule_f32", "pime_ph_rollout_schedule_f64",
     "pime_gae_scan", "pime_reduce_episode_stats_f32", "pime_reduce_episode_stats_f64",
     "pime_ppo_theta_count", "pime_ppo_theta_layout", "pime_ppo_work_floats", "pime_ppo_transpose", "pime_ppo_step", "pime_ppo_apply_grad",
     "pime_ppo_tc_work_bytes", "pime_ppo_tc_layout", "pime_ppo_grad_tc", "pime_ppo_close_step",

@@ -41,6 +41,7 @@ constexpr int kMaxFrames = 30;
 template <typename T, bool STACK> struct WtGlue {
     using Real = T;
     static constexpr int kObsMax = STACK ? kMaxFrames : 4;   // widest observation of this plant (loop bounds)
+    static constexpr bool kSegmented = false;
     WtConst<T> c;
     WtPtrs<T> p;
 
@@ -109,19 +110,45 @@ template <typename T, bool STACK> struct WtGlue {
         wt_reset(c, v.e, u, resample);
         if (c.from_last) { v.e.h1 = k1; v.e.h2 = k2; }
         v.episode += 1;
+        fill_frames(v);
+        return true;
+    }
+    // every frame = the current state (nonlinear_watertank.py:1183-1184)
+    __device__ __forceinline__ void fill_frames(Env &v) const {
         if constexpr (STACK) {
             const int m = 3 * c.num_stack;
 #pragma unroll
             for (int j = 0; j < kMaxFrames; j += 3)
                 if (j < m) { v.fr[j] = v.e.h1; v.fr[j + 1] = v.e.h2; v.fr[j + 2] = v.e.r; }
         }
+    }
+
+    // Segment begin of a scheduled launch: reset() exactly as wt_reset_kernel (step.cu) computes it, then set_state() of
+    // the levels before it and set_r(r) (utils/test.py:102-106).  set_state / set_r leave the frame history alone, so
+    // the segment's first observations still show the frames of the reset.
+    __device__ __forceinline__ bool restart(Env &v, T r, uint64_t seed, uint64_t index, int64_t i, bool resample) const {
+        const T h1 = v.e.h1, h2 = v.e.h2;
+        double u[6];
+        reset_uniforms(seed, index, v.episode, u);
+        wt_reset(c, v.e, u, resample);
+        if (c.from_last) wt_reset_levels_from_last(v.e, u, p.last_h1[i], p.last_h2[i]);
+        v.episode += 1;
+        fill_frames(v);
+        v.e.h1 = h1; v.e.h2 = h2; v.e.r = r;
         return true;
+    }
+    // the controlled output (the level tracking_error compares with r)
+    __device__ __forceinline__ T output(const Env &v) const { return v.e.h2; }
+    // what the reset writes and store() does not: I = 0 when the observation does not carry the integrator
+    __device__ __forceinline__ void store_reset_extra(int64_t i) const {
+        if (c.obs_mode != PIME_WT_OBS_INTEGRATOR && p.I) p.I[i] = (T)0;
     }
 };
 
 template <typename T> struct PhGlue {
     using Real = T;
     static constexpr int kObsMax = 3;
+    static constexpr bool kSegmented = false;
     PhConst<T> c;
     const T *table;
     PhPtrs<T> p;
@@ -162,6 +189,46 @@ template <typename T> struct PhGlue {
         bool ok = ph_reset(c, table, v.e, v.qww, v.qc, u, resample, c.from_last ? v.e.x : nan_of<double>());
         v.episode += 1;
         return ok;
+    }
+    // Segment begin of a scheduled launch: reset() exactly as ph_reset_kernel (step.cu) computes it, then the state x
+    // before it restored with its observation y under the new C, and r set (utils/test.py:1386-1388).
+    __device__ __forceinline__ bool restart(Env &v, T r, uint64_t seed, uint64_t index, int64_t i, bool resample) const {
+        const double x = v.e.x;
+        double u[6];
+        reset_uniforms(seed, index, v.episode, u);
+        bool ok = ph_reset(c, table, v.e, v.qww, v.qc, u, resample, c.from_last ? p.last_x[i] : nan_of<double>());
+        v.episode += 1;
+        v.e.x = x;
+        ok = ph_lookup(table, c.table_len, (double)v.e.C, x, v.e.y) && ok;   // observe_state (ph.py:187-189)
+        v.e.r = r;
+        return ok;
+    }
+    __device__ __forceinline__ T output(const Env &v) const { return v.e.y; }
+    __device__ __forceinline__ void store_reset_extra(int64_t i) const {
+        if (c.integrator_mode == PIME_PH_NO_INTEGRATOR && p.I) p.I[i] = (T)0;
+    }
+};
+
+// ------------------------------------------------------------------------------------------------ scheduled launch
+// T = K L steps in K segments of L steps (pime_schedule); segment k tracks set-point r[k].  Segmented<Glue> is the plant
+// glue of such a launch: Stepper restarts each env at every segment begin and keeps its tracking metrics in registers.
+// Every plain glue has kSegmented = false, for which none of this generates code.
+struct SegParams {
+    int K, L, resample;
+    double r[PIME_MAX_SEGMENTS];
+    double *metrics;   // [4][K][n] (ret, iae, final_err, overshoot), or NULL
+};
+
+template <typename Glue> struct Segmented : Glue {
+    static constexpr bool kSegmented = true;
+    SegParams sg;
+    struct Env : Glue::Env {
+        double m_ret, m_iae, m_err, m_ovs;   // this segment's sum of rewards, sum of |e|, last |e|, overshoot
+        bool up;                             // r >= y at the segment begin: the overshoot is y - r, else r - y
+    };
+    __device__ __forceinline__ void store(const Env &v, int64_t i, int64_t n) const {
+        Glue::store(v, i, n);
+        Glue::store_reset_extra(i);
     }
 };
 
@@ -277,6 +344,38 @@ template <typename Plant> struct Stepper {
             if (!plant.reset(env, rp.seed, rp.env_offset + (uint64_t)ii, rp.keep_params == 0)) fault = true;
             env.ret = (T)0;
         }
+        if constexpr (Plant::kSegmented) track(plant, rp, env, rew, s, ii, live);
+    }
+
+    // Segment k begins for the env: reset + restore + set-point (the glue's restart), metrics cleared.  The kernels call
+    // it for k = 0 right after an env is loaded; track() calls it for the later segments.  No code for a plain launch.
+    __device__ __forceinline__ void begin_segment(const Plant &plant, const RolloutParams &rp, typename Plant::Env &env, int k,
+                                                  int64_t ii) {
+        if constexpr (Plant::kSegmented) {
+            const T r = (T)plant.sg.r[k];
+            if (!plant.restart(env, r, rp.seed, rp.env_offset + (uint64_t)ii, ii, plant.sg.resample != 0)) fault = true;
+            env.ret = (T)0;
+            env.m_ret = env.m_iae = env.m_err = env.m_ovs = 0.0;
+            env.up = r >= plant.output(env);
+        }
+    }
+
+    // after step s: the metrics of the step; at a segment end, their store (live envs only) and the next segment's begin
+    __device__ __forceinline__ void track(const Plant &plant, const RolloutParams &rp, typename Plant::Env &env, T rew, int s,
+                                          int64_t ii, bool live) {
+        const double y = (double)plant.output(env), r = (double)env.e.r;
+        env.m_ret += (double)rew;
+        env.m_err = fabs(r - y);
+        env.m_iae += env.m_err;
+        env.m_ovs = fmax(env.m_ovs, env.up ? y - r : r - y);
+        const int k = (s + 1) / plant.sg.L;
+        if (k * plant.sg.L != s + 1) return;
+        if (live && plant.sg.metrics) {   // metrics[m][k - 1][ii]
+            const int64_t stride = (int64_t)plant.sg.K * rp.n;
+            double *m = plant.sg.metrics + (int64_t)(k - 1) * rp.n + ii;
+            m[0] = env.m_ret; m[stride] = env.m_iae; m[2 * stride] = env.m_err; m[3 * stride] = env.m_ovs;
+        }
+        if (s + 1 < rp.T) begin_segment(plant, rp, env, k, ii);
     }
 
     // warp-shuffle reduction of the episode / set-point statistics; lane 0 of each calling warp adds to red[][slot]
@@ -328,6 +427,8 @@ __global__ void __launch_bounds__(tc::kThreads, 1) rollout_kernel(Plant plant, t
         int64_t ii0 = live0 ? i0 : n - 1, ii1 = live1 ? i1 : n - 1;  // tail rows shadow the last env and write nothing
         plant.load(env0, ii0, n);
         plant.load(env1, ii1, n);
+        sp.begin_segment(plant, rp, env0, 0, ii0);
+        sp.begin_segment(plant, rp, env1, 0, ii1);
         plant.observe(env0, obs);
         eng.write_obs(row, 0, obs);
         plant.observe(env1, obs);
@@ -355,6 +456,7 @@ __global__ void __launch_bounds__(tc::kThreads, 1) rollout_kernel(Plant plant, t
                         if (live0) plant.store(env0, i0, n);
                         i0 = j0; live0 = i0 < n; ii0 = live0 ? i0 : n - 1;
                         plant.load(env0, ii0, n);
+                        sp.begin_segment(plant, rp, env0, 0, ii0);
                     }
                     if (more || next_tile) { plant.observe(env0, obs); eng.write_obs(row, 0, obs); }
                     PIME_TICK(c_work)
@@ -370,6 +472,7 @@ __global__ void __launch_bounds__(tc::kThreads, 1) rollout_kernel(Plant plant, t
                         if (live1) plant.store(env1, i1, n);
                         i1 = j1; live1 = i1 < n; ii1 = live1 ? i1 : n - 1;
                         plant.load(env1, ii1, n);
+                        sp.begin_segment(plant, rp, env1, 0, ii1);
                     }
                     if (more || next_tile) { plant.observe(env1, obs); eng.write_obs(row, 1, obs); }
                     PIME_TICK(c_work)
@@ -411,6 +514,7 @@ __global__ void __launch_bounds__(f32::kFThreads) rollout_fp32_kernel(Plant plan
     typename Plant::Env env;
     if (owner) plant.load(env, ii, n);
     Stepper<Plant> sp;
+    if (owner) sp.begin_segment(plant, rp, env, 0, ii);
     float obs[kMaxS];
     if (tid < 24) red[tid / 4][tid % 4] = 0.0;
     for (int s = 0; s < rp.T; ++s) {
@@ -454,6 +558,7 @@ __global__ void __launch_bounds__(128) rollout_prior_kernel(Plant plant, Rollout
     typename Plant::Env env;
     plant.load(env, ii, n);
     Stepper<Plant> sp;
+    sp.begin_segment(plant, rp, env, 0, ii);
     float obs[kMaxS];
     for (int s = 0; s < rp.T; ++s) {
         plant.observe(env, obs);
@@ -502,6 +607,43 @@ int launch_rollout_k(const Plant &plant, const tc::PackLayout *L, const void *pa
     }
     set_error("mid_dim must be 32, 64, 128 or 256");
     return PIME_EINVAL;
+}
+
+// The kernel for the actor of `a`: the prior kernel without one, the fidelity kernel in fp32 precision, else the tcgen05
+// kernel of its kind.  MODULAR = false for a plant without a modular instantiation (the caller has rejected that actor).
+template <typename Plant, bool MODULAR>
+int launch_rollout_actor(const Plant &plant, const RolloutParams &rp, const tc::PackLayout &L, const pime_rollout_args *a,
+                         cudaStream_t stream) {
+    if (!rp.has_actor) return launch_rollout_prior<Plant>(plant, rp, stream);
+    if (a->actor->precision == PIME_PRECISION_FP32) return launch_rollout_fp32<Plant>(plant, L, a->actor_pack, rp, stream);
+    if constexpr (MODULAR) {
+        if (a->actor->kind == PIME_ACTOR_MODULAR)
+            return launch_rollout_k<Plant, PIME_ACTOR_MODULAR>(plant, &L, a->actor_pack, rp, L.H, stream);
+    }
+    return launch_rollout_k<Plant, PIME_ACTOR_PLAIN>(plant, &L, a->actor_pack, rp, L.H, stream);
+}
+
+// the plain launch of glue g, or the scheduled one (Segmented<Glue>) when sg is given
+template <bool MODULAR, typename Glue>
+int launch_rollout_glue(const Glue &g, const SegParams *sg, const RolloutParams &rp, const tc::PackLayout &L,
+                        const pime_rollout_args *a, cudaStream_t stream) {
+    if (sg) return launch_rollout_actor<Segmented<Glue>, MODULAR>(Segmented<Glue>{g, *sg}, rp, L, a, stream);
+    return launch_rollout_actor<Glue, MODULAR>(g, rp, L, a, stream);
+}
+
+// Checks a schedule against the argument block and fills SegParams (host arithmetic only).
+inline int fill_seg_params(const pime_schedule *sc, const pime_rollout_args *a, SegParams &sg) {
+    PIME_REQUIRE(sc && a, "null schedule / rollout args");
+    PIME_REQUIRE(sc->num_segments >= 1 && sc->num_segments <= PIME_MAX_SEGMENTS, "num_segments must be in 1..16");
+    PIME_REQUIRE(sc->segment_steps >= 1, "segment_steps must be >= 1");
+    PIME_REQUIRE((int64_t)sc->num_segments * sc->segment_steps == (int64_t)a->T, "args->T must equal num_segments * segment_steps");
+    PIME_REQUIRE(sc->setpoints_host, "setpoints_host is NULL");
+    PIME_REQUIRE(a->auto_reset == 0, "a scheduled rollout resets at segment begins only: auto_reset must be 0");
+    sg = SegParams{};
+    sg.K = sc->num_segments; sg.L = sc->segment_steps; sg.resample = sc->resample_params != 0;
+    for (int k = 0; k < sg.K; ++k) sg.r[k] = sc->setpoints_host[k];
+    sg.metrics = sc->metrics;
+    return PIME_OK;
 }
 
 // Fills RolloutParams from the public argument block; returns the pack layout in L when an actor is given.

@@ -5,6 +5,10 @@ extern "C" int pime_ph_rollout_f32(const pime_ph_config *cfg, const float *table
                                    const pime_rollout_args *args, void *stream) {
     return ph_rollout_impl<float>(cfg, table, n, st, args, stream);
 }
+extern "C" int pime_ph_rollout_schedule_f32(const pime_ph_config *cfg, const float *table, int64_t n, const pime_ph_state *st,
+                                            const pime_rollout_args *args, const pime_schedule *sched, void *stream) {
+    return ph_rollout_schedule_impl<float>(cfg, table, n, st, args, sched, stream);
+}
 
 // Host-buffer entry (configs[3] end to end): H2D of the per-env state, fused rollout, D2H of ep_return + the final state,
 // pipelined over env slices (host_pipe.cuh).  x, A, B are double arrays in the float flavour (include/pime_b200.h),

@@ -5,6 +5,10 @@ extern "C" int pime_wt_rollout_f32(const pime_wt_config *cfg, int64_t n, const p
                                    void *stream) {
     return wt_rollout_impl<float>(cfg, n, st, args, stream);
 }
+extern "C" int pime_wt_rollout_schedule_f32(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st,
+                                            const pime_rollout_args *args, const pime_schedule *sched, void *stream) {
+    return wt_rollout_schedule_impl<float>(cfg, n, st, args, sched, stream);
+}
 
 // Host-buffer entry: H2D of the per-env state, fused rollout, D2H of ep_return (+ final state), pipelined over env slices
 // (host_pipe.cuh).  The stacking observation keeps its frames [3 num_stack][n] with stride n: one slice.

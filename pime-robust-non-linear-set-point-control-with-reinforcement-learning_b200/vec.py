@@ -146,6 +146,21 @@ def _rollout_args(env, T, actor, priorK, deterministic, auto_reset, reward_scale
     return a, out
 
 
+def _schedule(env, setpoints, segment_steps, resample_params, metrics, keep):
+    """pime_schedule of K = len(setpoints) segments of segment_steps steps; metrics: True (allocated [4, K, n] float64),
+    a tensor of that shape (or wider in n), or None."""
+    sp = np.ascontiguousarray(np.asarray(setpoints, dtype=np.float64).reshape(-1))
+    keep.append(sp)
+    K = sp.shape[0]
+    if metrics is True:
+        metrics = torch.empty((4, K, env.n), dtype=torch.float64, device=env.device)
+    if metrics is not None:
+        assert metrics.shape == (4, K, env.n) and metrics.dtype == torch.float64 and metrics.is_cuda
+    sc = L.Schedule(num_segments=K, segment_steps=int(segment_steps), resample_params=int(bool(resample_params)),
+                    setpoints_host=sp.ctypes.data_as(C.POINTER(C.c_double)), metrics=L.ptr(metrics))
+    return sc, metrics
+
+
 class _VecBase:
     def _alloc(self, names, n, f64=()):
         for k in names:
@@ -254,6 +269,23 @@ class WaterTankVec(_VecBase):
         L.check(_fn("pime_wt_rollout", self.dtype)(C.byref(self.cfg), C.c_int64(self.n), C.byref(self._st), C.byref(a),
                                                    L.stream_ptr()))
         self.tick += T
+        return out
+
+    def rollout_schedule(self, setpoints, segment_steps: int, priorK, actor: Optional[ActorPack] = None, deterministic=False,
+                         reward_scale=1.0, gamma=0.99, eps=None, pnoise=None, replay=None, want_actions=False, stats=None,
+                         a_std_log=None, resample_params=False, metrics=True):
+        """The set-point staircase in one launch (pime_wt_rollout_schedule_*): T = K * segment_steps fused steps, segment k
+        tracking setpoints[k] and beginning with reset(resample_params) -> set_state(levels before it) -> set_r(setpoints[k]).
+        Returns rollout()'s dict plus metrics [4, K, n] float64 (ret, iae, final_err, overshoot per segment and env)."""
+        keep = []
+        sc, metrics = _schedule(self, setpoints, segment_steps, resample_params, metrics, keep)
+        T = sc.num_segments * sc.segment_steps
+        a, out = _rollout_args(self, T, actor, priorK, deterministic, False, reward_scale, gamma, eps, pnoise, replay,
+                               want_actions, stats, keep, a_std_log)
+        L.check(_fn("pime_wt_rollout_schedule", self.dtype)(C.byref(self.cfg), C.c_int64(self.n), C.byref(self._st), C.byref(a),
+                                                            C.byref(sc), L.stream_ptr()))
+        self.tick += T
+        out["metrics"] = metrics
         return out
 
     def rollout_host(self, host_state: dict, T: int, priorK, actor: Optional[ActorPack] = None, deterministic=False,
@@ -385,6 +417,22 @@ class PHVec(_VecBase):
         L.check(_fn("pime_ph_rollout", self.dtype)(C.byref(self.cfg), L.ptr(self.table), C.c_int64(self.n), C.byref(self._st),
                                                    C.byref(a), L.stream_ptr()))
         self.tick += T
+        return out
+
+    def rollout_schedule(self, setpoints, segment_steps: int, priorK, actor: Optional[ActorPack] = None, deterministic=False,
+                         reward_scale=1.0, gamma=0.99, eps=None, replay=None, want_actions=False, stats=None, a_std_log=None,
+                         resample_params=False, metrics=True):
+        """The set-point staircase in one launch (pime_ph_rollout_schedule_*): segment k begins with reset(resample_params),
+        the state x before it restored (y looked up under the new C) and r = setpoints[k].  See WaterTankVec.rollout_schedule."""
+        keep = []
+        sc, metrics = _schedule(self, setpoints, segment_steps, resample_params, metrics, keep)
+        T = sc.num_segments * sc.segment_steps
+        a, out = _rollout_args(self, T, actor, priorK, deterministic, False, reward_scale, gamma, eps, None, replay,
+                               want_actions, stats, keep, a_std_log)
+        L.check(_fn("pime_ph_rollout_schedule", self.dtype)(C.byref(self.cfg), L.ptr(self.table), C.c_int64(self.n),
+                                                            C.byref(self._st), C.byref(a), C.byref(sc), L.stream_ptr()))
+        self.tick += T
+        out["metrics"] = metrics
         return out
 
     HOST_FIELDS = ("x", "y", "r", "I", "A", "B", "C", "qww_V", "qc_V", "t", "episode")
