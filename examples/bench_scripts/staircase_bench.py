@@ -5,9 +5,15 @@
 Cases (env-steps/s = envs x K x L / time, CUDA events, after a warm-up launch of every shape):
   wt  2^20 envs, Modular-256 actor, staircase 3, 6, 9, 4, 2 x 500 steps
   ph  2^23 envs, Modular-128 actor, staircase 10, 6, 3, 8, 5 x 50 steps
-For each case: scenarios.staircase_metrics on a ready env (the scheduled launch; metrics only), the deterministic
-vec.rollout of the same K L steps without replay rows (the ceiling: same kernel without the segment logic), alternated
-rep by rep, and scenarios.robust_map end to end (env construction, reset, parameters, launch).
+For each case: scenarios.staircase_metrics on a ready env (the scheduled launch; metrics only), the same launch with a
+[K, n] per-env set-point matrix (every column the shared staircase, so the two launches do the same work and differ by
+the set-point load alone), and the deterministic vec.rollout of the same K L steps without replay rows (the ceiling: same
+kernel without the segment logic), alternated rep by rep, and scenarios.robust_map end to end (env construction, reset,
+parameters, launch).
+Then the clipped linear baseline (policy='linear'), metrics only: the fused map of the water tank in f32 at 2^23 envs and
+in f64 at 2^20 envs (5 x 500 steps), against the per-step loop of scenarios.staircase(policy='linear') (prior kernel +
+step kernel per step, trajectories kept) at 2^18 envs.  The f32 rate is set against the MUFU ceiling of the plant: 40
+sqrt per env-step (20 Euler sub-steps x 2 tanks) at 16 MUFU ops / clk / SM, 148 SMs and 1.8 GHz = 1.07e11 env-steps/s.
 Prints the GPU name and power limit of the run first.
 """
 import argparse
@@ -50,29 +56,66 @@ def case(name, plant, n, H, steps, setpoints, K, params, reps):
     T = len(setpoints) * steps
     priorK = -np.asarray(K, np.float64)[:env.state_dim]
     sched = lambda: SC.staircase_metrics(env, K, actor=pack, setpoints=setpoints, steps=steps)   # noqa: E731
+    matrix = torch.tensor(setpoints, dtype=torch.float64, device="cuda")[:, None].expand(len(setpoints), n).contiguous()
+    per_env = lambda: SC.staircase_metrics(env, K, actor=pack, setpoints=matrix, steps=steps)   # noqa: E731
     plain = lambda: env.rollout(T, priorK, actor=pack, deterministic=True)                      # noqa: E731
     rmap = lambda: SC.robust_map(K, params, actor=pack, plant=plant, steps=steps, setpoints=setpoints)  # noqa: E731
-    for f in (sched, plain, rmap):   # warm-up
+    for f in (sched, per_env, plain, rmap):   # warm-up
         f()
     torch.cuda.synchronize()
-    ts, tp, tm = [], [], []
+    ts, te, tp, tm = [], [], [], []
     for _ in range(reps):
         ts.append(timed(sched))
+        te.append(timed(per_env))
         tp.append(timed(plain))
     for _ in range(max(1, reps // 2)):
         tm.append(timed(rmap))
     env.check_status()
     steps_total = n * T
-    s, p, m = np.median(ts), np.median(tp), np.median(tm)
+    s, e, p, m = np.median(ts), np.median(te), np.median(tp), np.median(tm)
     print(f"{name}: n={n} H={H} K={len(setpoints)} L={steps}")
     print(f"  scheduled launch (staircase_metrics) {s * 1e3:9.2f} ms  {steps_total / s:.3e} env-steps/s  "
           f"(min {min(ts) * 1e3:.2f}, max {max(ts) * 1e3:.2f} ms)")
+    print(f"  per-env set-points [K, n]            {e * 1e3:9.2f} ms  {steps_total / e:.3e} env-steps/s  "
+          f"(min {min(te) * 1e3:.2f}, max {max(te) * 1e3:.2f} ms)")
+    print(f"  per-env / shared time                {e / s:9.4f}")
     print(f"  plain deterministic rollout          {p * 1e3:9.2f} ms  {steps_total / p:.3e} env-steps/s  "
           f"(min {min(tp) * 1e3:.2f}, max {max(tp) * 1e3:.2f} ms)")
     print(f"  scheduled / plain time               {s / p:9.4f}")
     print(f"  robust_map end to end                {m * 1e3:9.2f} ms  {steps_total / m:.3e} env-steps/s", flush=True)
     del env
     torch.cuda.empty_cache()
+
+
+MUFU_CEILING = 16 * 148 * 1.8e9 / 40   # env-steps/s of the f32 water tank: 40 sqrt per env-step
+
+
+def linear_case(reps):
+    K = [0.0, 0.4, -0.4, 0.0]
+    setpoints, steps = SC.WT_INTEGRATOR_SETPOINTS, 500
+    T = len(setpoints) * steps
+    for dtype, n in ((torch.float32, 1 << 23), (torch.float64, 1 << 20)):
+        env = V.WaterTankVec(n, dtype=dtype)
+        env.reset()
+        fused = lambda: SC.staircase_metrics(env, K, setpoints=setpoints, steps=steps, policy="linear")   # noqa: E731
+        fused()
+        t = [timed(fused) for _ in range(reps)]
+        env.check_status()
+        f = np.median(t)
+        line = f"  fused linear map {str(dtype)[6:]:8s} n=2^{n.bit_length() - 1}  {f * 1e3:9.2f} ms  {n * T / f:.3e} env-steps/s"
+        if dtype == torch.float32:
+            line += f"  ({n * T / f / MUFU_CEILING:.1%} of the 1.07e11 MUFU ceiling)"
+        print(line + f"  (min {min(t) * 1e3:.2f}, max {max(t) * 1e3:.2f} ms)", flush=True)
+        del env
+        torch.cuda.empty_cache()
+    n = 1 << 18
+    env = V.WaterTankVec(n)
+    env.reset()
+    loop = lambda: SC.staircase(env, "linear", K, setpoints=setpoints, steps=steps)   # noqa: E731
+    loop()
+    t = [timed(loop) for _ in range(max(1, reps // 2))]
+    lp = np.median(t)
+    print(f"  per-step linear loop float32 n=2^18  {lp * 1e3:9.2f} ms  {n * T / lp:.3e} env-steps/s", flush=True)
 
 
 def main():
@@ -90,6 +133,9 @@ def main():
     n = 1 << 23
     ph_params = np.stack([rng.uniform(0.005, 0.015, n), rng.uniform(0.0015, 0.0025, n)], 1)
     case("ph robust map", "ph", n, 128, 50, SC.PH_SETPOINTS, [-0.02, 0.02, 0.035], ph_params, args.reps)
+    del wt_params, ph_params
+    print("wt linear baseline: K=5 L=500, metrics only", flush=True)
+    linear_case(args.reps)
 
 
 if __name__ == "__main__":

@@ -315,6 +315,41 @@ int pime_ph_rollout_schedule_f32(const pime_ph_config *cfg, const float *table, 
 int pime_ph_rollout_schedule_f64(const pime_ph_config *cfg, const double *table, int64_t n, const pime_ph_state *st,
                                  const pime_rollout_args *args, const pime_schedule *sched, void *stream);
 
+/* Scheduled rollout with an extension block: per-env set-points and the choice of policy, in the same launch.
+ *
+ *   setpoints_dev   segment k of env i tracks setpoints_dev[k * n + i] (DEVICE doubles, [K][n]; i is the env's index in
+ *                   this call, not env_offset + i); sched->setpoints_host must then be NULL.  NULL: setpoints_host as above.
+ *   policy          PIME_POLICY_ACTOR: the policy of the entries above (args->actor's residual policy, or the prior term
+ *                   alone when it is NULL).  PIME_POLICY_LINEAR: get_linear_action (utils/test.py:1056-1067), the action
+ *                   -(state . K) with K = -priorK_host, computed in the state dtype from the observation before float32
+ *                   (h1, h2, r, I / the frame history / y, r, I), summed in k order as pime_prior_action_* sums it,
+ *                   clipped to [-1, 1] for the water tank (get_P_action, nonlinear_watertank.py:755-759) and not for pH
+ *                   (ph.py:227-231).  Needs args->actor == NULL and args->deterministic != 0.  Replay rows keep their
+ *                   layout: float32(obs), (reward*scale, mask, a_raw = 0, eps = 0); env_action holds the clipped action.
+ *
+ * Besides everything the entries above reject, these reject (PIME_EINVAL, also without a device and for n = 0) a NULL
+ * ext, a policy outside PIME_POLICY_*, reserved0 != 0, set-points given as neither or both of setpoints_host /
+ * setpoints_dev, and PIME_POLICY_LINEAR with an actor or with deterministic == 0.
+ */
+#define PIME_POLICY_ACTOR 0
+#define PIME_POLICY_LINEAR 1
+typedef struct pime_schedule_ext {
+    const double *setpoints_dev;    /* DEVICE double[K][n], or NULL: sched->setpoints_host                    */
+    int32_t policy;                 /* PIME_POLICY_*                                                         */
+    int32_t reserved0;              /* must be 0                                                             */
+} pime_schedule_ext;
+
+int pime_wt_rollout_schedule_ext_f32(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st, const pime_rollout_args *args,
+                                     const pime_schedule *sched, const pime_schedule_ext *ext, void *stream);
+int pime_wt_rollout_schedule_ext_f64(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st, const pime_rollout_args *args,
+                                     const pime_schedule *sched, const pime_schedule_ext *ext, void *stream);
+int pime_ph_rollout_schedule_ext_f32(const pime_ph_config *cfg, const float *table, int64_t n, const pime_ph_state *st,
+                                     const pime_rollout_args *args, const pime_schedule *sched, const pime_schedule_ext *ext,
+                                     void *stream);
+int pime_ph_rollout_schedule_ext_f64(const pime_ph_config *cfg, const double *table, int64_t n, const pime_ph_state *st,
+                                     const pime_rollout_args *args, const pime_schedule *sched, const pime_schedule_ext *ext,
+                                     void *stream);
+
 /* Per-env GAE / reward-to-go reverse scan over a time-major replay (AgentPPO.compute_reward_gae
  * agent.py:685-708 without the final normalisation): reward, mask, value are [T][n] with element stride
  * `stride` floats (4 for buf_other columns, 1 for dense); r_sum, adv are dense [T][n]. */

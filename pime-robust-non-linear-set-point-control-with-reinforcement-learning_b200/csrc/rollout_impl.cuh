@@ -83,6 +83,17 @@ template <typename T, bool STACK> struct WtGlue {
             obs[3] = c.obs_mode == PIME_WT_OBS_INTEGRATOR ? (float)v.e.I : 0.0f;
         }
     }
+    // the observation in the plant dtype (what get_linear_action multiplies, nonlinear_watertank.py:755-759)
+    __device__ __forceinline__ void observe_state(const Env &v, T (&st)[kObsMax]) const {
+        if constexpr (STACK) {
+#pragma unroll
+            for (int j = 0; j < kMaxFrames; ++j) st[j] = v.fr[j];
+        } else {
+            st[0] = v.e.h1; st[1] = v.e.h2; st[2] = v.e.r;
+            st[3] = c.obs_mode == PIME_WT_OBS_INTEGRATOR ? v.e.I : (T)0;
+        }
+    }
+    static constexpr bool kLinearClip = true;   // get_P_action clips to the action space (:759)
     __device__ __forceinline__ bool uses_process_noise() const { return c.noise_scale > (T)0; }
     __device__ __forceinline__ T noise_sigma() const { return c.noise_scale; }
     __device__ __forceinline__ bool advance(Env &v, T action, T nz1, T nz2, T &rew, bool &done) const {
@@ -174,6 +185,11 @@ template <typename T> struct PhGlue {
         obs[0] = (float)v.e.y; obs[1] = (float)v.e.r;
         obs[2] = c.integrator_mode != PIME_PH_NO_INTEGRATOR ? (float)v.e.I : 0.0f;
     }
+    __device__ __forceinline__ void observe_state(const Env &v, T (&st)[kObsMax]) const {
+        st[0] = v.e.y; st[1] = v.e.r;
+        st[2] = c.integrator_mode != PIME_PH_NO_INTEGRATOR ? v.e.I : (T)0;
+    }
+    static constexpr bool kLinearClip = false;  // the pH linear action is not clipped (ph.py:227-231)
     __device__ __forceinline__ bool uses_process_noise() const { return false; }
     __device__ __forceinline__ T noise_sigma() const { return (T)0; }
     __device__ __forceinline__ bool advance(Env &v, T action, T, T, T &rew, bool &done) const {
@@ -215,7 +231,9 @@ template <typename T> struct PhGlue {
 // Every plain glue has kSegmented = false, for which none of this generates code.
 struct SegParams {
     int K, L, resample;
+    int linear;                 // PIME_POLICY_LINEAR: the prior kernel runs get_linear_action (Stepper::linear_action)
     double r[PIME_MAX_SEGMENTS];
+    const double *setpoints;    // [K][n] per-env set-points (device), or NULL: every env tracks r[k]
     double *metrics;   // [4][K][n] (ret, iae, final_err, overshoot), or NULL
 };
 
@@ -284,13 +302,38 @@ template <typename Plant> struct Stepper {
         }
     }
 
+    // The linear policy of a scheduled launch (get_linear_action: get_P_action, nonlinear_watertank.py:755-759, or the
+    // unclipped ph.py:227-231): -(state . K) with K = -priorK and state the observation in the plant dtype, summed term by
+    // term in k order as prior_kernel (step.cu) does: in fp64 a rounded product and a rounded sum per term, in fp32 one
+    // fused multiply-add per term (prior_kernel<float>'s acc + obs * K compiles to that FFMA chain; fmaf pins it here).
+    // Negating priorK and the sum is exact, so the action is the one pime_prior_action computes from the same state.
+    T p_linear = (T)0;
+    __device__ __forceinline__ void linear_action(const Plant &plant, const RolloutParams &rp, const typename Plant::Env &env) {
+        T st[Plant::kObsMax];
+        plant.observe_state(env, st);
+        T acc = (T)0;
+#pragma unroll
+        for (int k = 0; k < Plant::kObsMax; ++k) {
+            if (k >= rp.S) continue;
+            const T K = (T)(-rp.priorK[k]);
+            if constexpr (sizeof(T) == 4) acc = fmaf(st[k], K, acc);
+            else acc = N::add(acc, N::mul(st[k], K));
+        }
+        acc = -acc;
+        p_linear = Plant::kLinearClip ? clampT(acc, (T)-1, (T)1) : acc;
+    }
+
+    // LINEAR: the action is linear_action's (the caller guarantees deterministic = 1, so a_raw = eps = 0)
+    template <bool LINEAR = false>
     __device__ __forceinline__ void step(const Plant &plant, const RolloutParams &rp, typename Plant::Env &env,
                                          const float (&obs)[kMaxS], float a_avg, int s, int64_t ii, bool live) {
         prepare(plant, rp, obs, s, ii);
-        finish(plant, rp, env, obs, a_avg, s, ii, live);
+        if constexpr (LINEAR) linear_action(plant, rp, env);
+        finish<LINEAR>(plant, rp, env, obs, a_avg, s, ii, live);
     }
 
     // the rest of the step, after prepare(): action, plant step, replay row, statistics, auto-reset
+    template <bool LINEAR = false>
     __device__ __forceinline__ void finish(const Plant &plant, const RolloutParams &rp, typename Plant::Env &env,
                                            const float (&obs)[kMaxS], float a_avg, int s, int64_t ii, bool live) {
         const int S = rp.S;
@@ -299,7 +342,10 @@ template <typename Plant> struct Stepper {
         const T nz1 = p_nz1, nz2 = p_nz2;
         float a_raw;
         T action;
-        if (rp.deterministic) {
+        if constexpr (LINEAR) {
+            a_raw = 0.0f;
+            action = p_linear;
+        } else if (rp.deterministic) {
             a_raw = a_avg;
             action = (T)(tanhf(a_avg) + p_prior_f);
         } else {
@@ -352,7 +398,8 @@ template <typename Plant> struct Stepper {
     __device__ __forceinline__ void begin_segment(const Plant &plant, const RolloutParams &rp, typename Plant::Env &env, int k,
                                                   int64_t ii) {
         if constexpr (Plant::kSegmented) {
-            const T r = (T)plant.sg.r[k];
+            // a tail row shadows env n - 1 (ii < n), so the per-env read stays inside the matrix
+            const T r = (T)(plant.sg.setpoints ? plant.sg.setpoints[(int64_t)k * rp.n + ii] : plant.sg.r[k]);
             if (!plant.restart(env, r, rp.seed, rp.env_offset + (uint64_t)ii, ii, plant.sg.resample != 0)) fault = true;
             env.ret = (T)0;
             env.m_ret = env.m_iae = env.m_err = env.m_ovs = 0.0;
@@ -560,9 +607,18 @@ __global__ void __launch_bounds__(128) rollout_prior_kernel(Plant plant, Rollout
     Stepper<Plant> sp;
     sp.begin_segment(plant, rp, env, 0, ii);
     float obs[kMaxS];
-    for (int s = 0; s < rp.T; ++s) {
-        plant.observe(env, obs);
-        sp.step(plant, rp, env, obs, 0.0f, s, ii, live);
+    bool linear = false;   // the linear policy exists for scheduled launches only: a plain glue compiles the loop below alone
+    if constexpr (Plant::kSegmented) linear = plant.sg.linear != 0;
+    if (linear) {
+        for (int s = 0; s < rp.T; ++s) {
+            plant.observe(env, obs);
+            sp.template step<true>(plant, rp, env, obs, 0.0f, s, ii, live);
+        }
+    } else {
+        for (int s = 0; s < rp.T; ++s) {
+            plant.observe(env, obs);
+            sp.step(plant, rp, env, obs, 0.0f, s, ii, live);
+        }
     }
     if (live) plant.store(env, i, n);
     if (rp.stats) sp.reduce_warp(red, warp);
@@ -631,17 +687,34 @@ int launch_rollout_glue(const Glue &g, const SegParams *sg, const RolloutParams 
     return launch_rollout_actor<Glue, MODULAR>(g, rp, L, a, stream);
 }
 
-// Checks a schedule against the argument block and fills SegParams (host arithmetic only).
-inline int fill_seg_params(const pime_schedule *sc, const pime_rollout_args *a, SegParams &sg) {
+// Checks a schedule (and its extension, NULL for the entries without one) against the argument block and fills SegParams
+// (host arithmetic only).
+inline int fill_seg_params(const pime_schedule *sc, const pime_schedule_ext *ext, const pime_rollout_args *a, SegParams &sg) {
     PIME_REQUIRE(sc && a, "null schedule / rollout args");
     PIME_REQUIRE(sc->num_segments >= 1 && sc->num_segments <= PIME_MAX_SEGMENTS, "num_segments must be in 1..16");
     PIME_REQUIRE(sc->segment_steps >= 1, "segment_steps must be >= 1");
     PIME_REQUIRE((int64_t)sc->num_segments * sc->segment_steps == (int64_t)a->T, "args->T must equal num_segments * segment_steps");
-    PIME_REQUIRE(sc->setpoints_host, "setpoints_host is NULL");
     PIME_REQUIRE(a->auto_reset == 0, "a scheduled rollout resets at segment begins only: auto_reset must be 0");
+    const double *dev = nullptr;
+    int policy = PIME_POLICY_ACTOR;
+    if (ext) {
+        PIME_REQUIRE(ext->policy == PIME_POLICY_ACTOR || ext->policy == PIME_POLICY_LINEAR, "policy must be PIME_POLICY_*");
+        PIME_REQUIRE(ext->reserved0 == 0, "reserved0 must be 0");
+        PIME_REQUIRE((sc->setpoints_host == nullptr) != (ext->setpoints_dev == nullptr),
+                     "give exactly one of setpoints_host / setpoints_dev");
+        PIME_REQUIRE(ext->policy != PIME_POLICY_LINEAR || (a->actor == nullptr && a->deterministic != 0),
+                     "the linear policy takes no actor and is deterministic");
+        dev = ext->setpoints_dev;
+        policy = ext->policy;
+    } else {
+        PIME_REQUIRE(sc->setpoints_host, "setpoints_host is NULL");
+    }
     sg = SegParams{};
     sg.K = sc->num_segments; sg.L = sc->segment_steps; sg.resample = sc->resample_params != 0;
-    for (int k = 0; k < sg.K; ++k) sg.r[k] = sc->setpoints_host[k];
+    sg.linear = policy == PIME_POLICY_LINEAR;
+    if (sc->setpoints_host)
+        for (int k = 0; k < sg.K; ++k) sg.r[k] = sc->setpoints_host[k];
+    sg.setpoints = dev;
     sg.metrics = sc->metrics;
     return PIME_OK;
 }

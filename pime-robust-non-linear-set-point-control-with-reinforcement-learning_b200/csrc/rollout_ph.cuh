@@ -29,11 +29,11 @@ int ph_rollout_impl(const pime_ph_config *cfg, const T *table, int64_t n, const 
 
 template <typename T>
 int ph_rollout_schedule_impl(const pime_ph_config *cfg, const T *table, int64_t n, const pime_ph_state *st,
-                             const pime_rollout_args *args, const pime_schedule *sched, void *stream) {
+                             const pime_rollout_args *args, const pime_schedule *sched, const pime_schedule_ext *ext, void *stream) {
     if (int rc = validate_ph(cfg, n, st)) return rc;
     PIME_REQUIRE(table, "null table");
     SegParams sg;
-    if (int rc = fill_seg_params(sched, args, sg)) return rc;
+    if (int rc = fill_seg_params(sched, ext, args, sg)) return rc;
     return ph_rollout_launch<T>(cfg, table, n, PhPtrs<T>(*st), args, stream, &sg);
 }
 

@@ -7,7 +7,13 @@ extern "C" int pime_ph_rollout_f32(const pime_ph_config *cfg, const float *table
 }
 extern "C" int pime_ph_rollout_schedule_f32(const pime_ph_config *cfg, const float *table, int64_t n, const pime_ph_state *st,
                                             const pime_rollout_args *args, const pime_schedule *sched, void *stream) {
-    return ph_rollout_schedule_impl<float>(cfg, table, n, st, args, sched, stream);
+    return ph_rollout_schedule_impl<float>(cfg, table, n, st, args, sched, nullptr, stream);
+}
+extern "C" int pime_ph_rollout_schedule_ext_f32(const pime_ph_config *cfg, const float *table, int64_t n,
+                                                const pime_ph_state *st, const pime_rollout_args *args,
+                                                const pime_schedule *sched, const pime_schedule_ext *ext, void *stream) {
+    PIME_REQUIRE(ext, "null schedule extension");
+    return ph_rollout_schedule_impl<float>(cfg, table, n, st, args, sched, ext, stream);
 }
 
 // Host-buffer entry (configs[3] end to end): H2D of the per-env state, fused rollout, D2H of ep_return + the final state,

@@ -32,10 +32,10 @@ int wt_rollout_impl(const pime_wt_config *cfg, int64_t n, const pime_wt_state *s
 
 template <typename T>
 int wt_rollout_schedule_impl(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st, const pime_rollout_args *args,
-                             const pime_schedule *sched, void *stream) {
+                             const pime_schedule *sched, const pime_schedule_ext *ext, void *stream) {
     if (int rc = validate_wt(cfg, n, st)) return rc;
     SegParams sg;
-    if (int rc = fill_seg_params(sched, args, sg)) return rc;
+    if (int rc = fill_seg_params(sched, ext, args, sg)) return rc;
     return wt_rollout_launch<T>(cfg, n, WtPtrs<T>(*st), args, stream, &sg);
 }
 

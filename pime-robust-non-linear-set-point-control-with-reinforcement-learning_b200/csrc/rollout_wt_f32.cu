@@ -7,7 +7,13 @@ extern "C" int pime_wt_rollout_f32(const pime_wt_config *cfg, int64_t n, const p
 }
 extern "C" int pime_wt_rollout_schedule_f32(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st,
                                             const pime_rollout_args *args, const pime_schedule *sched, void *stream) {
-    return wt_rollout_schedule_impl<float>(cfg, n, st, args, sched, stream);
+    return wt_rollout_schedule_impl<float>(cfg, n, st, args, sched, nullptr, stream);
+}
+extern "C" int pime_wt_rollout_schedule_ext_f32(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st,
+                                                const pime_rollout_args *args, const pime_schedule *sched,
+                                                const pime_schedule_ext *ext, void *stream) {
+    PIME_REQUIRE(ext, "null schedule extension");
+    return wt_rollout_schedule_impl<float>(cfg, n, st, args, sched, ext, stream);
 }
 
 // Host-buffer entry: H2D of the per-env state, fused rollout, D2H of ep_return (+ final state), pipelined over env slices

@@ -14,8 +14,11 @@ what the reference does -- reset() (new ensemble member unless if_reset_all is F
 state, set the next set-point -- and it keeps per env and segment the return, the integral of |r - y|, the final |r - y|
 and the overshoot.  ``staircase`` returns the trajectories of that launch; ``staircase_metrics`` and ``robust_map``
 return the metrics alone ([K, n] per metric, no trajectory buffers), which is what a robustness map over millions of
-ensemble members needs.  The linear policy is the prior kernel + the step kernel per step (its action is clipped, which
-the fused kernel's prior term is not).
+ensemble members needs.  ``staircase_metrics`` and ``robust_map`` run either policy in that one launch -- the clipped
+linear baseline (get_linear_action, computed in the plant dtype) as well as the agent -- and take either one staircase for
+every env or a [K, n] matrix of per-env set-points (e.g. random staircases in [r_lo, r_hi], or a map over set-point
+sequence x ensemble parameters).  ``staircase(policy='linear')`` keeps the per-step loop of the prior kernel + the step
+kernel, which returns the same trajectories in fp64 and is what the fused linear policy is tested against.
 """
 from __future__ import annotations
 
@@ -53,9 +56,13 @@ def _staircase_setup(vec, setpoints, steps):
         setattr(vec.cfg, limit_field, saved_limit)
 
 
-def _scheduled(vec, K, actor, setpoints, steps, resample_params, start, trajectories):
-    """The deterministic agent policy over the whole staircase in one scheduled launch; the first segment restores
-    ``start`` after its reset (utils/test.py:102-104)."""
+def _scheduled(vec, K, actor, setpoints, steps, resample_params, start, trajectories, policy="agent"):
+    """The deterministic agent (or linear) policy over the whole staircase in one scheduled launch; the first segment
+    restores ``start`` after its reset (utils/test.py:102-104)."""
+    if policy not in ("agent", "linear"):
+        raise ValueError("policy must be 'agent' or 'linear'")
+    if policy == "linear" and actor is not None:
+        raise ValueError("the linear policy takes no actor")
     K = np.asarray(K, dtype=np.float64).reshape(-1)
     with _staircase_setup(vec, setpoints, steps) as (setpoints, steps):
         if _is_wt(vec):
@@ -63,7 +70,8 @@ def _scheduled(vec, K, actor, setpoints, steps, resample_params, start, trajecto
         else:
             vec.x.fill_(float(start[0]))
         return vec.rollout_schedule(setpoints, steps, -K[:vec.state_dim], actor=actor, deterministic=True,
-                                    replay=trajectories, want_actions=trajectories, resample_params=resample_params)
+                                    replay=trajectories, want_actions=trajectories, resample_params=resample_params,
+                                    policy="actor" if policy == "agent" else "linear")
 
 
 def _begin_segment(vec, r, resample, first, start):
@@ -134,19 +142,22 @@ def staircase(vec, policy: str, K, actor: Optional[V.ActorPack] = None, setpoint
 METRICS = ("ret", "iae", "final_err", "overshoot")
 
 
-def staircase_metrics(vec, K, actor: Optional[V.ActorPack] = None, setpoints: Optional[Sequence[float]] = None,
-                      steps: Optional[int] = None, resample_params: bool = False, start=(0.0, 0.0)):
-    """The agent-policy staircase of ``staircase`` as one launch without trajectories: {"ret", "iae", "final_err",
-    "overshoot"}, each [K, n] float64 (segment k, env i).  With y the controlled output (h2 / pH) and e = r - y:
-    ret = sum of rewards, iae = sum of |e| over the segment's steps, final_err = |e| after its last step, overshoot =
-    max(0, max of d (y - r)) with d = +1 when the segment starts below its set-point, -1 when above."""
-    m = _scheduled(vec, K, actor, setpoints, steps, resample_params, start, False)["metrics"]
+def staircase_metrics(vec, K, actor: Optional[V.ActorPack] = None, setpoints=None, steps: Optional[int] = None,
+                      resample_params: bool = False, start=(0.0, 0.0), policy: str = "agent"):
+    """The staircase of ``staircase`` as one launch without trajectories: {"ret", "iae", "final_err", "overshoot"}, each
+    [K, n] float64 (segment k, env i).  With y the controlled output (h2 / pH) and e = r - y: ret = sum of rewards, iae =
+    sum of |e| over the segment's steps, final_err = |e| after its last step, overshoot = max(0, max of d (y - r)) with
+    d = +1 when the segment starts below its set-point, -1 when above.
+    policy: 'agent' or 'linear' as in ``staircase`` (K is the reference's K; 'linear' takes no actor).  setpoints: K
+    floats for every env, or a [K, n] array / tensor (column i: env i's staircase)."""
+    m = _scheduled(vec, K, actor, setpoints, steps, resample_params, start, False, policy)["metrics"]
     return dict(zip(METRICS, m.unbind(0)))
 
 
 def robust_map(K, params, actor: Optional[V.ActorPack] = None, plant: str = "wt", setpoints=None, steps=None,
-               dtype=torch.float32, device="cuda", obs_mode="integrator", integrator="integrator", **cfg):
-    """Tracking metrics of the agent policy over any number of off-nominal parameter sets, one env per set, in one launch.
+               dtype=torch.float32, device="cuda", obs_mode="integrator", integrator="integrator", policy="agent", **cfg):
+    """Tracking metrics of the agent (or, policy='linear', the clipped linear baseline) policy over any number of off-nominal
+    parameter sets, one env per set, in one launch.  setpoints: K floats, or [K, n] with column i for parameter row i.
     plant = 'wt': rows (a1, a2, Kp) as in robust_sweep (utils/robust_test.py), steps default 500; plant = 'ph': rows
     (qww_V, qc_V) with the discretised system refreshed (set_params(update_system=True)), steps default
     max_episode_steps.  The ensemble parameters are kept between segments (if_reset_all = False).  A grid over the axes
@@ -164,7 +175,7 @@ def robust_map(K, params, actor: Optional[V.ActorPack] = None, plant: str = "wt"
         env.set_params(torch.as_tensor(p[:, 0]), torch.as_tensor(p[:, 1]), update_system=True)
     else:
         raise ValueError("plant must be 'wt' or 'ph'")
-    return staircase_metrics(env, K, actor=actor, setpoints=setpoints, steps=steps, resample_params=False), p
+    return staircase_metrics(env, K, actor=actor, setpoints=setpoints, steps=steps, resample_params=False, policy=policy), p
 
 
 ROBUST_TESTS = ((0.0024, 0.0019, 0.12), (0.0024, 0.0015, 0.12), (0.0024, 0.0015, 0.07))   # utils/robust_test.py:12-37

@@ -146,19 +146,39 @@ def _rollout_args(env, T, actor, priorK, deterministic, auto_reset, reward_scale
     return a, out
 
 
-def _schedule(env, setpoints, segment_steps, resample_params, metrics, keep):
-    """pime_schedule of K = len(setpoints) segments of segment_steps steps; metrics: True (allocated [4, K, n] float64),
-    a tensor of that shape (or wider in n), or None."""
-    sp = np.ascontiguousarray(np.asarray(setpoints, dtype=np.float64).reshape(-1))
-    keep.append(sp)
-    K = sp.shape[0]
+_POLICY = {"actor": L.POLICY_ACTOR, "linear": L.POLICY_LINEAR}
+
+
+def _schedule(env, setpoints, segment_steps, resample_params, metrics, policy, keep):
+    """pime_schedule of K segments of segment_steps steps, and its pime_schedule_ext (None when neither per-env set-points
+    nor the linear policy is asked for, so that the entries without one are called).  setpoints: K floats shared by every
+    env, or a [K, n] array / tensor (column i for env i).  metrics: True (allocated [4, K, n] float64), a tensor of that
+    shape (or wider in n), or None."""
+    if policy not in _POLICY:
+        raise ValueError(f"policy must be one of {list(_POLICY)}")
+    ext = None
+    if np.ndim(setpoints) == 2:
+        sp = torch.as_tensor(setpoints).to(device=env.device, dtype=torch.float64).contiguous()
+        K = sp.shape[0]
+        assert sp.shape == (K, env.n) and 1 <= K <= L.MAX_SEGMENTS, f"per-env set-points must be [K, {env.n}], 1 <= K <= 16"
+        keep.append(sp)
+        host = None
+        ext = L.ScheduleExt(setpoints_dev=L.ptr(sp))
+    else:
+        sp = np.ascontiguousarray(np.asarray(setpoints, dtype=np.float64).reshape(-1))
+        keep.append(sp)
+        K = sp.shape[0]
+        host = sp.ctypes.data_as(C.POINTER(C.c_double))
+    if policy != "actor":
+        ext = ext or L.ScheduleExt()
+        ext.policy = _POLICY[policy]
     if metrics is True:
         metrics = torch.empty((4, K, env.n), dtype=torch.float64, device=env.device)
     if metrics is not None:
         assert metrics.shape == (4, K, env.n) and metrics.dtype == torch.float64 and metrics.is_cuda
     sc = L.Schedule(num_segments=K, segment_steps=int(segment_steps), resample_params=int(bool(resample_params)),
-                    setpoints_host=sp.ctypes.data_as(C.POINTER(C.c_double)), metrics=L.ptr(metrics))
-    return sc, metrics
+                    setpoints_host=host, metrics=L.ptr(metrics))
+    return sc, ext, metrics
 
 
 class _VecBase:
@@ -273,17 +293,23 @@ class WaterTankVec(_VecBase):
 
     def rollout_schedule(self, setpoints, segment_steps: int, priorK, actor: Optional[ActorPack] = None, deterministic=False,
                          reward_scale=1.0, gamma=0.99, eps=None, pnoise=None, replay=None, want_actions=False, stats=None,
-                         a_std_log=None, resample_params=False, metrics=True):
+                         a_std_log=None, resample_params=False, metrics=True, policy="actor"):
         """The set-point staircase in one launch (pime_wt_rollout_schedule_*): T = K * segment_steps fused steps, segment k
         tracking setpoints[k] and beginning with reset(resample_params) -> set_state(levels before it) -> set_r(setpoints[k]).
+        setpoints: K floats for every env, or a [K, n] array / tensor whose column i is env i's staircase.
+        policy = 'actor': the residual policy of ``actor`` (None: the prior term alone); 'linear': get_linear_action,
+        clip(state . priorK, -1, 1) in the plant dtype (no actor, deterministic=True).
         Returns rollout()'s dict plus metrics [4, K, n] float64 (ret, iae, final_err, overshoot per segment and env)."""
         keep = []
-        sc, metrics = _schedule(self, setpoints, segment_steps, resample_params, metrics, keep)
+        sc, ext, metrics = _schedule(self, setpoints, segment_steps, resample_params, metrics, policy, keep)
         T = sc.num_segments * sc.segment_steps
         a, out = _rollout_args(self, T, actor, priorK, deterministic, False, reward_scale, gamma, eps, pnoise, replay,
                                want_actions, stats, keep, a_std_log)
-        L.check(_fn("pime_wt_rollout_schedule", self.dtype)(C.byref(self.cfg), C.c_int64(self.n), C.byref(self._st), C.byref(a),
-                                                            C.byref(sc), L.stream_ptr()))
+        args = (C.byref(self.cfg), C.c_int64(self.n), C.byref(self._st), C.byref(a), C.byref(sc))
+        if ext is None:
+            L.check(_fn("pime_wt_rollout_schedule", self.dtype)(*args, L.stream_ptr()))
+        else:
+            L.check(_fn("pime_wt_rollout_schedule_ext", self.dtype)(*args, C.byref(ext), L.stream_ptr()))
         self.tick += T
         out["metrics"] = metrics
         return out
@@ -421,16 +447,20 @@ class PHVec(_VecBase):
 
     def rollout_schedule(self, setpoints, segment_steps: int, priorK, actor: Optional[ActorPack] = None, deterministic=False,
                          reward_scale=1.0, gamma=0.99, eps=None, replay=None, want_actions=False, stats=None, a_std_log=None,
-                         resample_params=False, metrics=True):
+                         resample_params=False, metrics=True, policy="actor"):
         """The set-point staircase in one launch (pime_ph_rollout_schedule_*): segment k begins with reset(resample_params),
-        the state x before it restored (y looked up under the new C) and r = setpoints[k].  See WaterTankVec.rollout_schedule."""
+        the state x before it restored (y looked up under the new C) and r = setpoints[k].  policy = 'linear': state . priorK
+        in the plant dtype, not clipped (ph.py:227-231).  See WaterTankVec.rollout_schedule."""
         keep = []
-        sc, metrics = _schedule(self, setpoints, segment_steps, resample_params, metrics, keep)
+        sc, ext, metrics = _schedule(self, setpoints, segment_steps, resample_params, metrics, policy, keep)
         T = sc.num_segments * sc.segment_steps
         a, out = _rollout_args(self, T, actor, priorK, deterministic, False, reward_scale, gamma, eps, None, replay,
                                want_actions, stats, keep, a_std_log)
-        L.check(_fn("pime_ph_rollout_schedule", self.dtype)(C.byref(self.cfg), L.ptr(self.table), C.c_int64(self.n),
-                                                            C.byref(self._st), C.byref(a), C.byref(sc), L.stream_ptr()))
+        args = (C.byref(self.cfg), L.ptr(self.table), C.c_int64(self.n), C.byref(self._st), C.byref(a), C.byref(sc))
+        if ext is None:
+            L.check(_fn("pime_ph_rollout_schedule", self.dtype)(*args, L.stream_ptr()))
+        else:
+            L.check(_fn("pime_ph_rollout_schedule_ext", self.dtype)(*args, C.byref(ext), L.stream_ptr()))
         self.tick += T
         out["metrics"] = metrics
         return out
