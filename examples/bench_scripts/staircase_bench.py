@@ -1,6 +1,6 @@
 """Scheduled staircase (robustness map) throughput against the plain fused rollout of the same number of steps.
 
-    python examples/bench_scripts/staircase_bench.py [--reps 5]
+    python examples/bench_scripts/staircase_bench.py [--reps 5] [--arm all|response]
 
 Cases (env-steps/s = envs x K x L / time, CUDA events, after a warm-up launch of every shape):
   wt  2^20 envs, Modular-256 actor, staircase 3, 6, 9, 4, 2 x 500 steps
@@ -14,6 +14,10 @@ Then the clipped linear baseline (policy='linear'), metrics only: the fused map 
 in f64 at 2^20 envs (5 x 500 steps), against the per-step loop of scenarios.staircase(policy='linear') (prior kernel +
 step kernel per step, trajectories kept) at 2^18 envs.  The f32 rate is set against the MUFU ceiling of the plant: 40
 sqrt per env-step (20 Euler sub-steps x 2 tanks) at 16 MUFU ops / clk / SM, 148 SMs and 1.8 GHz = 1.07e11 env-steps/s.
+Then the step response (--arm response runs this arm alone): the metrics-only launch with and without response=True
+(settle, rise, effort, peak action per env and segment, the Tracked kernels), alternated rep by rep, for the agent on the
+water tank (2^20 envs, Modular-256, 5 x 500 steps) and pH (2^23 envs, Modular-128, 5 x 50 steps) and for the linear
+baseline in f32 on the water tank (2^23 envs, 5 x 500 steps).
 Prints the GPU name and power limit of the run first.
 """
 import argparse
@@ -118,14 +122,49 @@ def linear_case(reps):
     print(f"  per-step linear loop float32 n=2^18  {lp * 1e3:9.2f} ms  {n * T / lp:.3e} env-steps/s", flush=True)
 
 
+def response_arm(reps):
+    """metrics only, with and without the step response, alternated rep by rep in the same env"""
+    runs = (("wt agent  Modular-256 f32", "wt", 1 << 20, 256, 500, SC.WT_INTEGRATOR_SETPOINTS, [0.0, 0.4, -0.4, 0.0], "agent"),
+            ("ph agent  Modular-128 f32", "ph", 1 << 23, 128, 50, SC.PH_SETPOINTS, [-0.02, 0.02, 0.035], "agent"),
+            ("wt linear f32            ", "wt", 1 << 23, 0, 500, SC.WT_INTEGRATOR_SETPOINTS, [0.0, 0.4, -0.4, 0.0], "linear"))
+    for name, plant, n, H, steps, setpoints, K, policy in runs:
+        pack = modular_pack(4 if plant == "wt" else 3, H) if policy == "agent" else None
+        env = V.WaterTankVec(n) if plant == "wt" else V.PHVec(n)
+        env.reset()
+        kw = dict(actor=pack, setpoints=setpoints, steps=steps, policy=policy)
+        without = lambda: SC.staircase_metrics(env, K, **kw)                  # noqa: E731
+        with_r = lambda: SC.staircase_metrics(env, K, response=True, **kw)    # noqa: E731
+        without()
+        with_r()
+        torch.cuda.synchronize()
+        t0, t1 = [], []
+        for _ in range(reps):
+            t0.append(timed(without))
+            t1.append(timed(with_r))
+        env.check_status()
+        a, b = np.median(t0), np.median(t1)
+        steps_total = n * len(setpoints) * steps
+        print(f"  {name} n=2^{n.bit_length() - 1} K={len(setpoints)} L={steps}: metrics {a * 1e3:9.2f} ms "
+              f"({steps_total / a:.3e} env-steps/s, min {min(t0) * 1e3:.2f}, max {max(t0) * 1e3:.2f}), with response "
+              f"{b * 1e3:9.2f} ms ({steps_total / b:.3e}, min {min(t1) * 1e3:.2f}, max {max(t1) * 1e3:.2f}); "
+              f"with / without {b / a:.4f}", flush=True)
+        del env
+        torch.cuda.empty_cache()
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=5)
+    ap.add_argument("--arm", choices=("all", "response"), default="all")
     args = ap.parse_args()
     assert torch.cuda.is_available(), "needs a CUDA device"
     q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
                        capture_output=True, text=True)
     print("GPU:", q.stdout.strip().splitlines()[0] if q.returncode == 0 else torch.cuda.get_device_name(0), flush=True)
+    if args.arm == "response":
+        print("step response: metrics-only launch without / with response=True", flush=True)
+        response_arm(args.reps)
+        return
     rng = np.random.default_rng(1)
     n = 1 << 20
     wt_params = np.stack([rng.uniform(0.0015, 0.0024, n), rng.uniform(0.0015, 0.0024, n), rng.uniform(0.07, 0.17, n)], 1)
@@ -136,6 +175,8 @@ def main():
     del wt_params, ph_params
     print("wt linear baseline: K=5 L=500, metrics only", flush=True)
     linear_case(args.reps)
+    print("step response: metrics-only launch without / with response=True", flush=True)
+    response_arm(args.reps)
 
 
 if __name__ == "__main__":

@@ -350,6 +350,38 @@ int pime_ph_rollout_schedule_ext_f64(const pime_ph_config *cfg, const double *ta
                                      const pime_rollout_args *args, const pime_schedule *sched, const pime_schedule_ext *ext,
                                      void *stream);
 
+/* Scheduled rollout with the step response: the launch of the _ext entries (ext may be NULL: shared set-points and
+ * PIME_POLICY_ACTOR), which also stores per env and segment, in fp64, with j = 0 .. L-1 the step inside the segment, y_j
+ * the output after step j, e_j = r - y_j, u_j the action fed to the plant at step j (what env_action records), y_b the
+ * output at the segment begin (after the restore), D = |r - y_b| and d = +1 if r >= y_b, else -1:
+ *
+ *   response[0][k][i]  settle       0 if |e_j| <= settle_band * D for every j, else 1 + the largest j with |e_j| > that
+ *                                   band (L: not settled at the segment end)
+ *   response[1][k][i]  rise         1 + the smallest j with d (y_j - y_b) >= 0.9 D; -1 if no step reaches it; 0 if D = 0
+ *   response[2][k][i]  effort       sum over j = 1 .. L-1 of |u_j - u_{j-1}|, in j order
+ *   response[3][k][i]  peak_action  max over j of |u_j|
+ *
+ * Dead tail rows store nothing.  Besides everything the _ext entries reject, these reject (PIME_EINVAL, also without a
+ * device and for n = 0) a NULL resp or response, settle_band outside (0, 1) or NaN, and segment_steps > 65535.
+ */
+typedef struct pime_step_response {
+    double *response;               /* device double[4][K][n] (settle, rise, effort, peak_action)             */
+    double settle_band;             /* settling band relative to D, in (0, 1); 0.02 is the usual choice       */
+} pime_step_response;
+
+int pime_wt_rollout_schedule_response_f32(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st,
+                                          const pime_rollout_args *args, const pime_schedule *sched,
+                                          const pime_schedule_ext *ext, const pime_step_response *resp, void *stream);
+int pime_wt_rollout_schedule_response_f64(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st,
+                                          const pime_rollout_args *args, const pime_schedule *sched,
+                                          const pime_schedule_ext *ext, const pime_step_response *resp, void *stream);
+int pime_ph_rollout_schedule_response_f32(const pime_ph_config *cfg, const float *table, int64_t n, const pime_ph_state *st,
+                                          const pime_rollout_args *args, const pime_schedule *sched,
+                                          const pime_schedule_ext *ext, const pime_step_response *resp, void *stream);
+int pime_ph_rollout_schedule_response_f64(const pime_ph_config *cfg, const double *table, int64_t n, const pime_ph_state *st,
+                                          const pime_rollout_args *args, const pime_schedule *sched,
+                                          const pime_schedule_ext *ext, const pime_step_response *resp, void *stream);
+
 /* Per-env GAE / reward-to-go reverse scan over a time-major replay (AgentPPO.compute_reward_gae
  * agent.py:685-708 without the final normalisation): reward, mask, value are [T][n] with element stride
  * `stride` floats (4 for buf_other columns, 1 for dense); r_sum, adv are dense [T][n]. */

@@ -81,6 +81,10 @@ class ScheduleExt(C.Structure):
     _fields_ = [("setpoints_dev", vp), ("policy", C.c_int32), ("reserved0", C.c_int32)]
 
 
+class StepResponse(C.Structure):
+    _fields_ = [("response", vp), ("settle_band", C.c_double)]
+
+
 class PpoArgs(C.Structure):
     _fields_ = [("actor", C.POINTER(ActorConfig)), ("theta", vp), ("theta_t", vp), ("adam_m", vp), ("adam_v", vp),
                 ("grad_out", vp), ("buf_state", vp), ("buf_action", vp), ("buf_r_sum", vp), ("buf_logprob", vp),
@@ -100,6 +104,8 @@ SYMBOLS = [
     "pime_wt_rollout_schedule_f32", "pime_wt_rollout_schedule_f64", "pime_ph_rollout_schedule_f32", "pime_ph_rollout_schedule_f64",
     "pime_wt_rollout_schedule_ext_f32", "pime_wt_rollout_schedule_ext_f64", "pime_ph_rollout_schedule_ext_f32",
     "pime_ph_rollout_schedule_ext_f64",
+    "pime_wt_rollout_schedule_response_f32", "pime_wt_rollout_schedule_response_f64", "pime_ph_rollout_schedule_response_f32",
+    "pime_ph_rollout_schedule_response_f64",
     "pime_gae_scan", "pime_reduce_episode_stats_f32", "pime_reduce_episode_stats_f64",
     "pime_ppo_theta_count", "pime_ppo_theta_layout", "pime_ppo_work_floats", "pime_ppo_transpose", "pime_ppo_step", "pime_ppo_apply_grad",
     "pime_ppo_tc_work_bytes", "pime_ppo_tc_layout", "pime_ppo_grad_tc", "pime_ppo_close_step",

@@ -239,6 +239,7 @@ struct SegParams {
 
 template <typename Glue> struct Segmented : Glue {
     static constexpr bool kSegmented = true;
+    static constexpr bool kTracked = false;
     SegParams sg;
     struct Env : Glue::Env {
         double m_ret, m_iae, m_err, m_ovs;   // this segment's sum of rewards, sum of |e|, last |e|, overshoot
@@ -248,6 +249,26 @@ template <typename Glue> struct Segmented : Glue {
         Glue::store(v, i, n);
         Glue::store_reset_extra(i);
     }
+};
+
+// Step response of a scheduled launch (pime_step_response): per env and segment, settling time, rise time, control effort
+// and peak action.  Tracked<Glue> is a Segmented<Glue> whose Stepper also keeps those four in registers; a Segmented glue
+// has kTracked = false, for which none of it generates code.  Its kernels live in objects of their own (rollout_track_*).
+constexpr int kMaxTrackedSteps = 0xffff;   // settle and rise are packed as two 16-bit step counts
+struct TrackParams {
+    double *response;    // [4][K][n] (settle, rise, effort, peak_action)
+    double settle_band;  // the settling band relative to |r - y_b|, in (0, 1)
+};
+
+template <typename Glue> struct Tracked : Segmented<Glue> {
+    static constexpr bool kTracked = true;
+    TrackParams tr;
+    using T = typename Glue::Real;
+    struct Env : Segmented<Glue>::Env {
+        double t_eff;           // sum of |u_j - u_{j-1}| so far
+        T t_peak, t_prev, t_yb; // max |u_j| so far, u_{j-1}, the output at the segment begin
+        uint32_t t_idx;         // bits 0-15: 1 + the last j with |e_j| > band (0: none); bits 16-31: 1 + the first j at 90 %
+    };
 };
 
 template <typename T> __device__ __forceinline__ T prior_k(const RolloutParams &rp, int k);
@@ -390,7 +411,7 @@ template <typename Plant> struct Stepper {
             if (!plant.reset(env, rp.seed, rp.env_offset + (uint64_t)ii, rp.keep_params == 0)) fault = true;
             env.ret = (T)0;
         }
-        if constexpr (Plant::kSegmented) track(plant, rp, env, rew, s, ii, live);
+        if constexpr (Plant::kSegmented) track(plant, rp, env, rew, action, s, ii, live);
     }
 
     // Segment k begins for the env: reset + restore + set-point (the glue's restart), metrics cleared.  The kernels call
@@ -404,25 +425,56 @@ template <typename Plant> struct Stepper {
             env.ret = (T)0;
             env.m_ret = env.m_iae = env.m_err = env.m_ovs = 0.0;
             env.up = r >= plant.output(env);
+            if constexpr (Plant::kTracked) {
+                env.t_eff = 0.0;
+                env.t_peak = env.t_prev = (T)0;
+                env.t_yb = plant.output(env);
+                env.t_idx = 0u;
+            }
         }
     }
 
-    // after step s: the metrics of the step; at a segment end, their store (live envs only) and the next segment's begin
-    __device__ __forceinline__ void track(const Plant &plant, const RolloutParams &rp, typename Plant::Env &env, T rew, int s,
-                                          int64_t ii, bool live) {
+    // after step s: the metrics of the step; at a segment end, their store (live envs only) and the next segment's begin.
+    // u is the action the plant was fed.
+    __device__ __forceinline__ void track(const Plant &plant, const RolloutParams &rp, typename Plant::Env &env, T rew, T u,
+                                          int s, int64_t ii, bool live) {
         const double y = (double)plant.output(env), r = (double)env.e.r;
         env.m_ret += (double)rew;
         env.m_err = fabs(r - y);
         env.m_iae += env.m_err;
         env.m_ovs = fmax(env.m_ovs, env.up ? y - r : r - y);
         const int k = (s + 1) / plant.sg.L;
+        if constexpr (Plant::kTracked) respond(plant, env, u, y, r, k * plant.sg.L == s + 1 ? plant.sg.L : s + 1 - k * plant.sg.L);
         if (k * plant.sg.L != s + 1) return;
         if (live && plant.sg.metrics) {   // metrics[m][k - 1][ii]
             const int64_t stride = (int64_t)plant.sg.K * rp.n;
             double *m = plant.sg.metrics + (int64_t)(k - 1) * rp.n + ii;
             m[0] = env.m_ret; m[stride] = env.m_iae; m[2 * stride] = env.m_err; m[3 * stride] = env.m_ovs;
         }
+        if constexpr (Plant::kTracked) {
+            if (live) {   // response[m][k - 1][ii]
+                const int64_t stride = (int64_t)plant.sg.K * rp.n;
+                double *o = plant.tr.response + (int64_t)(k - 1) * rp.n + ii;
+                const uint32_t rise = env.t_idx >> 16;
+                o[0] = (double)(env.t_idx & 0xffffu);
+                o[stride] = fabs(r - (double)env.t_yb) == 0.0 ? 0.0 : rise ? (double)rise : -1.0;
+                o[2 * stride] = env.t_eff;
+                o[3 * stride] = (double)env.t_peak;
+            }
+        }
         if (s + 1 < rp.T) begin_segment(plant, rp, env, k, ii);
+    }
+
+    // The step-response accumulators after step j = j1 - 1 of a segment, all comparisons in fp64 (pime_step_response):
+    // |e_j| > band . |r - y_b| sets settle = j1; the first j with d (y_j - y_b) >= 0.9 |r - y_b| sets rise = j1 (d = +1 when
+    // r >= y_b, i.e. env.up); effort adds |u_j - u_{j-1}| from j = 1 on; peak = max |u_j|.
+    __device__ __forceinline__ void respond(const Plant &plant, typename Plant::Env &env, T u, double y, double r, int j1) {
+        const double yb = (double)env.t_yb, dlt = fabs(r - yb);
+        if (j1 > 1) env.t_eff += fabs((double)u - (double)env.t_prev);
+        env.t_prev = u;
+        if (N::abs(u) > env.t_peak) env.t_peak = N::abs(u);
+        if (env.m_err > plant.tr.settle_band * dlt) env.t_idx = (env.t_idx & 0xffff0000u) | (uint32_t)j1;
+        if ((env.t_idx >> 16) == 0u && (env.up ? y - yb : yb - y) >= 0.9 * dlt) env.t_idx |= (uint32_t)j1 << 16;
     }
 
     // warp-shuffle reduction of the episode / set-point statistics; lane 0 of each calling warp adds to red[][slot]
@@ -679,12 +731,17 @@ int launch_rollout_actor(const Plant &plant, const RolloutParams &rp, const tc::
     return launch_rollout_k<Plant, PIME_ACTOR_PLAIN>(plant, &L, a->actor_pack, rp, L.H, stream);
 }
 
-// the plain launch of glue g, or the scheduled one (Segmented<Glue>) when sg is given
-template <bool MODULAR, typename Glue>
+// the plain launch of glue g, or the scheduled one (Segmented<Glue>) when sg is given.  TRACK: the scheduled launch with
+// the step response (Tracked<Glue>, sg and tr given); it instantiates the Tracked kernels alone.
+template <bool MODULAR, bool TRACK = false, typename Glue>
 int launch_rollout_glue(const Glue &g, const SegParams *sg, const RolloutParams &rp, const tc::PackLayout &L,
-                        const pime_rollout_args *a, cudaStream_t stream) {
-    if (sg) return launch_rollout_actor<Segmented<Glue>, MODULAR>(Segmented<Glue>{g, *sg}, rp, L, a, stream);
-    return launch_rollout_actor<Glue, MODULAR>(g, rp, L, a, stream);
+                        const pime_rollout_args *a, cudaStream_t stream, const TrackParams *tr = nullptr) {
+    if constexpr (TRACK) {
+        return launch_rollout_actor<Tracked<Glue>, MODULAR>(Tracked<Glue>{Segmented<Glue>{g, *sg}, *tr}, rp, L, a, stream);
+    } else {
+        if (sg) return launch_rollout_actor<Segmented<Glue>, MODULAR>(Segmented<Glue>{g, *sg}, rp, L, a, stream);
+        return launch_rollout_actor<Glue, MODULAR>(g, rp, L, a, stream);
+    }
 }
 
 // Checks a schedule (and its extension, NULL for the entries without one) against the argument block and fills SegParams
@@ -716,6 +773,15 @@ inline int fill_seg_params(const pime_schedule *sc, const pime_schedule_ext *ext
         for (int k = 0; k < sg.K; ++k) sg.r[k] = sc->setpoints_host[k];
     sg.setpoints = dev;
     sg.metrics = sc->metrics;
+    return PIME_OK;
+}
+
+// Checks a step-response block against a filled schedule and fills TrackParams (host arithmetic only).
+inline int fill_track_params(const pime_step_response *resp, const SegParams &sg, TrackParams &tr) {
+    PIME_REQUIRE(resp && resp->response, "null step-response block / response");
+    PIME_REQUIRE(resp->settle_band > 0.0 && resp->settle_band < 1.0, "settle_band must be in (0, 1)");
+    PIME_REQUIRE(sg.L <= kMaxTrackedSteps, "segment_steps must be <= 65535 with a step response");
+    tr = TrackParams{resp->response, resp->settle_band};
     return PIME_OK;
 }
 

@@ -17,8 +17,11 @@ return the metrics alone ([K, n] per metric, no trajectory buffers), which is wh
 ensemble members needs.  ``staircase_metrics`` and ``robust_map`` run either policy in that one launch -- the clipped
 linear baseline (get_linear_action, computed in the plant dtype) as well as the agent -- and take either one staircase for
 every env or a [K, n] matrix of per-env set-points (e.g. random staircases in [r_lo, r_hi], or a map over set-point
-sequence x ensemble parameters).  ``staircase(policy='linear')`` keeps the per-step loop of the prior kernel + the step
-kernel, which returns the same trajectories in fp64 and is what the fused linear policy is tested against.
+sequence x ensemble parameters).  With ``response=True`` the same launch also returns each segment's step response --
+settling time, rise time, control effort (total variation of the action) and peak action -- without any trajectory, so a
+map can show where a policy commands more than the actuator takes.  ``staircase(policy='linear')`` keeps the per-step
+loop of the prior kernel + the step kernel, which returns the same trajectories in fp64 and is what the fused linear
+policy is tested against.
 """
 from __future__ import annotations
 
@@ -56,7 +59,8 @@ def _staircase_setup(vec, setpoints, steps):
         setattr(vec.cfg, limit_field, saved_limit)
 
 
-def _scheduled(vec, K, actor, setpoints, steps, resample_params, start, trajectories, policy="agent"):
+def _scheduled(vec, K, actor, setpoints, steps, resample_params, start, trajectories, policy="agent", response=False,
+               settle_band=0.02):
     """The deterministic agent (or linear) policy over the whole staircase in one scheduled launch; the first segment
     restores ``start`` after its reset (utils/test.py:102-104)."""
     if policy not in ("agent", "linear"):
@@ -71,7 +75,8 @@ def _scheduled(vec, K, actor, setpoints, steps, resample_params, start, trajecto
             vec.x.fill_(float(start[0]))
         return vec.rollout_schedule(setpoints, steps, -K[:vec.state_dim], actor=actor, deterministic=True,
                                     replay=trajectories, want_actions=trajectories, resample_params=resample_params,
-                                    policy="actor" if policy == "agent" else "linear")
+                                    policy="actor" if policy == "agent" else "linear", response=response,
+                                    settle_band=settle_band)
 
 
 def _begin_segment(vec, r, resample, first, start):
@@ -140,28 +145,39 @@ def staircase(vec, policy: str, K, actor: Optional[V.ActorPack] = None, setpoint
 
 
 METRICS = ("ret", "iae", "final_err", "overshoot")
+RESPONSE = ("settle", "rise", "effort", "peak_action")
 
 
 def staircase_metrics(vec, K, actor: Optional[V.ActorPack] = None, setpoints=None, steps: Optional[int] = None,
-                      resample_params: bool = False, start=(0.0, 0.0), policy: str = "agent"):
+                      resample_params: bool = False, start=(0.0, 0.0), policy: str = "agent", response: bool = False,
+                      settle_band: float = 0.02):
     """The staircase of ``staircase`` as one launch without trajectories: {"ret", "iae", "final_err", "overshoot"}, each
     [K, n] float64 (segment k, env i).  With y the controlled output (h2 / pH) and e = r - y: ret = sum of rewards, iae =
     sum of |e| over the segment's steps, final_err = |e| after its last step, overshoot = max(0, max of d (y - r)) with
     d = +1 when the segment starts below its set-point, -1 when above.
     policy: 'agent' or 'linear' as in ``staircase`` (K is the reference's K; 'linear' takes no actor).  setpoints: K
-    floats for every env, or a [K, n] array / tensor (column i: env i's staircase)."""
-    m = _scheduled(vec, K, actor, setpoints, steps, resample_params, start, False, policy)["metrics"]
-    return dict(zip(METRICS, m.unbind(0)))
+    floats for every env, or a [K, n] array / tensor (column i: env i's staircase).
+    response=True adds the step response of each segment, [K, n] float64 each, computed in the same launch (L steps per
+    segment, j = 0 .. L-1, u_j the action fed to the plant, y_b the output at the segment begin, D = |r - y_b|):
+    settle = 1 + the last j with |e_j| > settle_band D (0: always inside the band, L: not settled); rise = 1 + the first j
+    at which y has covered 90 % of D (-1: never, 0: D = 0); effort = sum of |u_j - u_{j-1}|; peak_action = max |u_j|."""
+    out = _scheduled(vec, K, actor, setpoints, steps, resample_params, start, False, policy, response, settle_band)
+    res = dict(zip(METRICS, out["metrics"].unbind(0)))
+    if response:
+        res.update(zip(RESPONSE, out["response"].unbind(0)))
+    return res
 
 
 def robust_map(K, params, actor: Optional[V.ActorPack] = None, plant: str = "wt", setpoints=None, steps=None,
-               dtype=torch.float32, device="cuda", obs_mode="integrator", integrator="integrator", policy="agent", **cfg):
+               dtype=torch.float32, device="cuda", obs_mode="integrator", integrator="integrator", policy="agent",
+               response: bool = False, settle_band: float = 0.02, **cfg):
     """Tracking metrics of the agent (or, policy='linear', the clipped linear baseline) policy over any number of off-nominal
     parameter sets, one env per set, in one launch.  setpoints: K floats, or [K, n] with column i for parameter row i.
     plant = 'wt': rows (a1, a2, Kp) as in robust_sweep (utils/robust_test.py), steps default 500; plant = 'ph': rows
     (qww_V, qc_V) with the discretised system refreshed (set_params(update_system=True)), steps default
     max_episode_steps.  The ensemble parameters are kept between segments (if_reset_all = False).  A grid over the axes
-    is one np.meshgrid (or parameter_grid) in the caller.  Returns (metrics dict as staircase_metrics, params array)."""
+    is one np.meshgrid (or parameter_grid) in the caller.  response / settle_band: the step response, as in
+    staircase_metrics.  Returns (metrics dict as staircase_metrics, params array)."""
     if plant == "wt":
         p = np.asarray(params, dtype=np.float64).reshape(-1, 3)
         steps = int(steps or 500)
@@ -175,7 +191,8 @@ def robust_map(K, params, actor: Optional[V.ActorPack] = None, plant: str = "wt"
         env.set_params(torch.as_tensor(p[:, 0]), torch.as_tensor(p[:, 1]), update_system=True)
     else:
         raise ValueError("plant must be 'wt' or 'ph'")
-    return staircase_metrics(env, K, actor=actor, setpoints=setpoints, steps=steps, resample_params=False, policy=policy), p
+    return staircase_metrics(env, K, actor=actor, setpoints=setpoints, steps=steps, resample_params=False, policy=policy,
+                             response=response, settle_band=settle_band), p
 
 
 ROBUST_TESTS = ((0.0024, 0.0019, 0.12), (0.0024, 0.0015, 0.12), (0.0024, 0.0015, 0.07))   # utils/robust_test.py:12-37

@@ -181,6 +181,17 @@ def _schedule(env, setpoints, segment_steps, resample_params, metrics, policy, k
     return sc, ext, metrics
 
 
+def _step_response(env, K, response, settle_band):
+    """pime_step_response and its [4, K, n] float64 output (settle, rise, effort, peak_action), or (None, None) when
+    response is False.  response: True (allocated) or a preallocated tensor of that shape."""
+    if response is False:
+        return None, None
+    if response is True:
+        response = torch.empty((4, K, env.n), dtype=torch.float64, device=env.device)
+    assert response.shape == (4, K, env.n) and response.dtype == torch.float64 and response.is_cuda and response.is_contiguous()
+    return L.StepResponse(response=L.ptr(response), settle_band=float(settle_band)), response
+
+
 class _VecBase:
     def _alloc(self, names, n, f64=()):
         for k in names:
@@ -293,20 +304,29 @@ class WaterTankVec(_VecBase):
 
     def rollout_schedule(self, setpoints, segment_steps: int, priorK, actor: Optional[ActorPack] = None, deterministic=False,
                          reward_scale=1.0, gamma=0.99, eps=None, pnoise=None, replay=None, want_actions=False, stats=None,
-                         a_std_log=None, resample_params=False, metrics=True, policy="actor"):
+                         a_std_log=None, resample_params=False, metrics=True, policy="actor", response=False,
+                         settle_band=0.02):
         """The set-point staircase in one launch (pime_wt_rollout_schedule_*): T = K * segment_steps fused steps, segment k
         tracking setpoints[k] and beginning with reset(resample_params) -> set_state(levels before it) -> set_r(setpoints[k]).
         setpoints: K floats for every env, or a [K, n] array / tensor whose column i is env i's staircase.
         policy = 'actor': the residual policy of ``actor`` (None: the prior term alone); 'linear': get_linear_action,
         clip(state . priorK, -1, 1) in the plant dtype (no actor, deterministic=True).
-        Returns rollout()'s dict plus metrics [4, K, n] float64 (ret, iae, final_err, overshoot per segment and env)."""
+        Returns rollout()'s dict plus metrics [4, K, n] float64 (ret, iae, final_err, overshoot per segment and env).
+        response=True (or a preallocated [4, K, n] float64 tensor) adds out["response"]: settle, rise, effort, peak_action per
+        segment and env (pime_wt_rollout_schedule_response_*; settle_band in (0, 1) relative to |r - y| at the segment
+        begin, see include/pime_b200.h); response=False calls exactly the entries above."""
         keep = []
         sc, ext, metrics = _schedule(self, setpoints, segment_steps, resample_params, metrics, policy, keep)
         T = sc.num_segments * sc.segment_steps
         a, out = _rollout_args(self, T, actor, priorK, deterministic, False, reward_scale, gamma, eps, pnoise, replay,
                                want_actions, stats, keep, a_std_log)
+        resp, response = _step_response(self, sc.num_segments, response, settle_band)
         args = (C.byref(self.cfg), C.c_int64(self.n), C.byref(self._st), C.byref(a), C.byref(sc))
-        if ext is None:
+        if resp is not None:
+            L.check(_fn("pime_wt_rollout_schedule_response", self.dtype)(*args, None if ext is None else C.byref(ext),
+                                                                         C.byref(resp), L.stream_ptr()))
+            out["response"] = response
+        elif ext is None:
             L.check(_fn("pime_wt_rollout_schedule", self.dtype)(*args, L.stream_ptr()))
         else:
             L.check(_fn("pime_wt_rollout_schedule_ext", self.dtype)(*args, C.byref(ext), L.stream_ptr()))
@@ -447,7 +467,7 @@ class PHVec(_VecBase):
 
     def rollout_schedule(self, setpoints, segment_steps: int, priorK, actor: Optional[ActorPack] = None, deterministic=False,
                          reward_scale=1.0, gamma=0.99, eps=None, replay=None, want_actions=False, stats=None, a_std_log=None,
-                         resample_params=False, metrics=True, policy="actor"):
+                         resample_params=False, metrics=True, policy="actor", response=False, settle_band=0.02):
         """The set-point staircase in one launch (pime_ph_rollout_schedule_*): segment k begins with reset(resample_params),
         the state x before it restored (y looked up under the new C) and r = setpoints[k].  policy = 'linear': state . priorK
         in the plant dtype, not clipped (ph.py:227-231).  See WaterTankVec.rollout_schedule."""
@@ -456,8 +476,13 @@ class PHVec(_VecBase):
         T = sc.num_segments * sc.segment_steps
         a, out = _rollout_args(self, T, actor, priorK, deterministic, False, reward_scale, gamma, eps, None, replay,
                                want_actions, stats, keep, a_std_log)
+        resp, response = _step_response(self, sc.num_segments, response, settle_band)
         args = (C.byref(self.cfg), L.ptr(self.table), C.c_int64(self.n), C.byref(self._st), C.byref(a), C.byref(sc))
-        if ext is None:
+        if resp is not None:
+            L.check(_fn("pime_ph_rollout_schedule_response", self.dtype)(*args, None if ext is None else C.byref(ext),
+                                                                         C.byref(resp), L.stream_ptr()))
+            out["response"] = response
+        elif ext is None:
             L.check(_fn("pime_ph_rollout_schedule", self.dtype)(*args, L.stream_ptr()))
         else:
             L.check(_fn("pime_ph_rollout_schedule_ext", self.dtype)(*args, C.byref(ext), L.stream_ptr()))
