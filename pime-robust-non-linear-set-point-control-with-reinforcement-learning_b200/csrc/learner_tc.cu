@@ -128,6 +128,7 @@ struct GemmProb {
     float *db, *db2; int db_split;                       // data gradient: bias gradients of the layer(s) that produced APREV: column sums of the
                                                          // result go to db[unit] (unit < db_split) or db2[unit - db_split]; NULL: none
     float db_scale;                                      // 1 / (gradient scale of this net), see StepCommon::dz_scale
+    const float *db_mul;                                 // critic: inv_cs, the factor its carried gradients leave out; NULL: 1
 };
 struct GemmBatch {
     GemmProb p[kMaxProb];
@@ -286,7 +287,8 @@ __global__ void __launch_bounds__(kGemmThreads, kGemmStages == 1 ? 3 : 1) gemm_k
     __syncthreads();
     if (P.mode == 1 && P.db && tid < P.n_cols) {
         const int unit = nt * 128 + tid;
-        atomicAdd(unit < P.db_split ? P.db + unit : P.db2 + (unit - P.db_split), s_db[tid] * P.db_scale);
+        const float scale = P.db_mul ? P.db_scale * *P.db_mul : P.db_scale;
+        atomicAdd(unit < P.db_split ? P.db + unit : P.db2 + (unit - P.db_split), s_db[tid] * scale);
     }
     if (warp == 1) tc_fence_after();
     if (warp == 1) tmem_dealloc(tmem, 128);
@@ -305,6 +307,7 @@ struct WgProb {
     int in_lo, in_hi, out_n;
     int bias_col, b_off;                                 // first layers: input unit bias_col (the ones column) -> grad[b_off + out]; -1: none
     float scale;                                         // 1 / (gradient scale of this net)
+    const float *scale_mul;                              // critic: inv_cs, the factor its carried gradients leave out; NULL: 1
 };
 struct WgBatch {
     WgProb p[kMaxProb];
@@ -313,6 +316,12 @@ struct WgBatch {
 };
 constexpr int kWgSmem = 12 * kBlk + 1024;   // two hi buffers (M_hi 2 blocks + N_hi 2 blocks) + one lo buffer
 constexpr int kWgThreads = 192;
+// Row tile i accumulates into TMEM accumulator i % kWgAcc (128 columns each; the shared memory above admits one CTA per SM,
+// so the 512 columns are free), and the epilogue adds the accumulators in fp32.  The tensor cores' fp32 accumulation loses
+// precision in proportion to the number of products summed into one accumulator: one accumulator over the 32 row tiles
+// of a CTA left 5.3e-5 of a gradient tensor's largest entry at B = 2^17, and 3.3e-4 at B = 2^20 (256 row tiles per CTA).
+constexpr int kWgAcc = 4;
+constexpr int kWgMaxTiles = 32;             // row tiles per CTA at most: the row split grows past 32 for B > 2^17
 
 // Shared memory: H[0], H[1] (the hi blocks of row tile i, i + 1: 64 KB each) and L (the lo blocks of row tile i: 64 KB).  A row
 // tile's products are  M_hi N_hi  (needs H only)  then  M_lo N_hi + M_hi N_lo  (needs L too): while those run, the hi blocks
@@ -332,7 +341,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_mn_kernel(const __grid_co
         mbar_init(l_full, 1); mbar_init(l_empty, 1); mbar_init(acc_ready, 1);
         fence_barrier_init();
     }
-    if (warp == 1) tmem_alloc(tmem_slot, 128);
+    if (warp == 1) tmem_alloc(tmem_slot, 128 * kWgAcc);
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -365,12 +374,13 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_mn_kernel(const __grid_co
             const uint32_t hb = smem_u32(smem) + buf * 4 * kBlk, lb = smem_u32(sL);
             // MN-major, no swizzle: K groups (8 rows) 128 B apart (LBO), MN groups (8 units) one unit group apart (SBO);
             // 16 batch rows per MMA = 256 B further into every unit group
+            const uint32_t acc = tmem + 128u * (uint32_t)(i % kWgAcc);
             mbar_wait(&h_full[buf], ((uint32_t)i >> 1) & 1u);
             tc_fence_after();
             if (elect_one()) {
 #pragma unroll
                 for (int kk = 0; kk < 8; ++kk)
-                    mma_f16(tmem, make_desc(hb + kk * 256, 128, kUg), make_desc(hb + 2 * kBlk + kk * 256, 128, kUg), id, (i == 0 && kk == 0) ? 0u : 1u);
+                    mma_f16(acc, make_desc(hb + kk * 256, 128, kUg), make_desc(hb + 2 * kBlk + kk * 256, 128, kUg), id, (i < kWgAcc && kk == 0) ? 0u : 1u);
             }
             __syncwarp();
             mbar_wait(l_full, (uint32_t)i & 1u);
@@ -378,8 +388,8 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_mn_kernel(const __grid_co
             if (elect_one()) {
 #pragma unroll
                 for (int kk = 0; kk < 8; ++kk) {
-                    mma_f16(tmem, make_desc(lb + kk * 256, 128, kUg), make_desc(hb + 2 * kBlk + kk * 256, 128, kUg), id, 1u);   // M_lo N_hi
-                    mma_f16(tmem, make_desc(hb + kk * 256, 128, kUg), make_desc(lb + 2 * kBlk + kk * 256, 128, kUg), id, 1u);   // M_hi N_lo
+                    mma_f16(acc, make_desc(lb + kk * 256, 128, kUg), make_desc(hb + 2 * kBlk + kk * 256, 128, kUg), id, 1u);   // M_lo N_hi
+                    mma_f16(acc, make_desc(hb + kk * 256, 128, kUg), make_desc(lb + 2 * kBlk + kk * 256, 128, kUg), id, 1u);   // M_hi N_lo
                 }
                 mma_commit(l_empty);
                 mma_commit(&h_empty[buf]);
@@ -392,23 +402,31 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_mn_kernel(const __grid_co
         tc_fence_after();
         const int m_unit = mt * 128 + 32 * (warp & 3) + lane;
         const uint32_t taddr = tmem + ((uint32_t)(32 * (warp & 3)) << 16);
+        const float scale = P.scale_mul ? P.scale * *P.scale_mul : P.scale;
+        const int n_acc = my_tiles < kWgAcc ? my_tiles : kWgAcc;
         for (int j = 0; j < P.n_cols / 32; ++j) {
             float v[32];
             tmem_ld32(taddr + j * 32, v);
+            for (int q = 1; q < n_acc; ++q) {
+                float u[32];
+                tmem_ld32(taddr + 128 * q + j * 32, u);
+#pragma unroll
+                for (int e = 0; e < 32; ++e) v[e] += u[e];
+            }
 #pragma unroll
             for (int e = 0; e < 32; ++e) {
                 const int n_unit = ntile * P.n_cols + j * 32 + e;
                 const int out = P.swap ? n_unit : m_unit, in = P.swap ? m_unit : n_unit;
                 if (out < P.out_n) {
-                    if (in >= P.in_lo && in < P.in_hi) atomicAdd(wb.grad + P.w_off + (size_t)out * P.ldw + (in - P.in_lo), v[e] * P.scale);
-                    else if (in == P.bias_col) atomicAdd(wb.grad + P.b_off + out, v[e] * P.scale);
+                    if (in >= P.in_lo && in < P.in_hi) atomicAdd(wb.grad + P.w_off + (size_t)out * P.ldw + (in - P.in_lo), v[e] * scale);
+                    else if (in == P.bias_col) atomicAdd(wb.grad + P.b_off + out, v[e] * scale);
                 }
             }
         }
         tc_fence_before();
     }
     __syncthreads();
-    if (warp == 1) tmem_dealloc(tmem, 128);
+    if (warp == 1) tmem_dealloc(tmem, 128 * kWgAcc);
 }
 
 // ------------------------------------------------------------------------------------------------ small kernels
@@ -459,10 +477,15 @@ struct StepCommon {
     float *rowv;        // [row_tiles * 128][4]: action, r_sum, old logprob, advantage
     float *inv_cs;      // 1 / (r_sum.std() + 1e-5) of the minibatch
     const float *theta;
-    // Gradient scaling.  d united / d out is O(1 / B) per row (and another 1 / std(r_sum) for the critic): at B = 2^17 the
-    // pre-activation gradients would sit in fp16's subnormal range and lose the lo part.  They are therefore carried
-    // multiplied by a power of two (exact), per net, through the whole data-gradient chain (which is linear in them), and
-    // every sum that leaves for the fp32 gradient is multiplied by the inverse.  Saturated at +-6e4 instead of overflowing.
+    // Gradient scaling.  d united / d out is O(1 / B) per row: at B = 2^17 the pre-activation gradients would sit in fp16's
+    // subnormal range and lose the lo part.  They are therefore carried multiplied by a power of two (exact), per net,
+    // through the whole data-gradient chain (which is linear in them), and every sum that leaves for the fp32 gradient is
+    // multiplied by the inverse.  The critic's carried gradients also leave out the factor inv_cs = 1 / (std(r_sum) + 1e-5)
+    // of its d out, so their size does not depend on the return scale: |d out| B / inv_cs = |clamp(v - r_sum, +-1)| <= 1,
+    // the carried output-layer gradient is at most 2 * 16 |w|, and inv_cs is applied in fp32 where critic sums leave for
+    // grad (the last hidden bias in out_obj_kernel, GemmProb::db_mul, WgProb::scale_mul).  The actor's |d out| B is
+    // |adv * ratio - lambda (...)| * |a - mean| / std^2: bounded by the replay's normalised advantages, the ratio and the
+    // sampling noise of the action over exp(a_std_log); saturated at +-6e4 instead of overflowing.
     float dz_scale[2];
 };
 
@@ -524,7 +547,7 @@ struct OutNet {
 };
 __global__ void __launch_bounds__(256) out_obj_kernel(const StepCommon c, const OutNet na, const OutNet nc) {
     __shared__ float part[32][129];
-    __shared__ float dout[128];
+    __shared__ float dout[128], dcarry[128];   // d out of the row; what the data-gradient chain carries (critic: without inv_cs)
     __shared__ float gw[257];
     __shared__ float gb_last[256];
     __shared__ float red4[8][4];
@@ -552,11 +575,13 @@ __global__ void __launch_bounds__(256) out_obj_kernel(const StepCommon c, const 
         float out = __ldg(c.theta + N.b_off);
         for (int ug = 0; ug < UG; ++ug) out += part[ug][row];
         const float4 rv = reinterpret_cast<const float4 *>(c.rowv)[b];   // action, r_sum, old logprob, advantage
-        const ppo::RowObj ob = ppo::row_objectives(net, out, rv.x, rv.y, rv.z, rv.w, __ldg(c.theta + c.n_theta - 1), *c.inv_cs,
+        // critic: d out = clamp(e) / B * inv_cs, evaluated in that order; the carried gradient stops before inv_cs
+        const ppo::RowObj ob = ppo::row_objectives(net, out, rv.x, rv.y, rv.z, rv.w, __ldg(c.theta + c.n_theta - 1), 1.0f,
                                                    c.ratio_clip, c.lambda_entropy, 1.0f / (float)c.B, live);
-        const float d = ob.d_out;
+        const float d = net == 1 ? ob.d_out * *c.inv_cs : ob.d_out;
         float o_act = ob.o_act, o_cri = ob.o_cri, o_ent = ob.o_ent, g_asl = ob.g_asl;
         dout[row] = d;
+        dcarry[row] = ob.d_out;
         float db = d;
 #pragma unroll
         for (int o2 = 16; o2 > 0; o2 >>= 1) {
@@ -580,7 +605,7 @@ __global__ void __launch_bounds__(256) out_obj_kernel(const StepCommon c, const 
         float a[8], x[8];
         join8(*reinterpret_cast<const uint4 *>(N.LAST + tblock(rt, N.chunks, ug >> 3, 0) + o),
               *reinterpret_cast<const uint4 *>(N.LAST + tblock(rt, N.chunks, ug >> 3, 1) + o), a);
-        const float d = dout[row], ds = d * c.dz_scale[net];
+        const float d = dout[row], ds = dcarry[row] * c.dz_scale[net];
 #pragma unroll
         for (int e = 0; e < 8; ++e) x[e] = fminf(fmaxf(ds * __ldg(w + ug * 8 + e) * act_grad(N.act, a[e]), -6e4f), 6e4f);
         uint4 hi, lo;
@@ -596,7 +621,7 @@ __global__ void __launch_bounds__(256) out_obj_kernel(const StepCommon c, const 
         if ((lane & 3) == 0) { atomicAdd(&gw[ug * 8 + col], sw); atomicAdd(&gb_last[ug * 8 + col], sb); }
     }
     __syncthreads();
-    const float unscale = 1.0f / c.dz_scale[net];
+    const float unscale = net == 1 ? *c.inv_cs / c.dz_scale[net] : 1.0f / c.dz_scale[net];
     for (int j = tid; j < H; j += 256) { atomicAdd(c.grad + N.w_off + j, gw[j]); atomicAdd(c.grad + N.db_last_off + j, gb_last[j] * unscale); }
     if (tid == 0) atomicAdd(c.grad + N.b_off, gw[H]);
 }
@@ -679,8 +704,8 @@ static GemmProb fwd(uint8_t *w, const Plan &pl, size_t A, int a_chunks, int a_c0
     p.OUT = w + OUT; p.out_chunks = pl.H / 64; p.out_c0 = out_c0;
     return p;
 }
-static GemmProb bwd(uint8_t *w, const Plan &pl, float unscale, size_t DZ, int dz_c0, int kc, size_t WT, int wt_chunks, int K, int act, size_t APREV,
-                    size_t OUT, float *db, float *db2 = nullptr, int db_split = 1 << 30) {
+static GemmProb bwd(uint8_t *w, const Plan &pl, float unscale, const float *mul, size_t DZ, int dz_c0, int kc, size_t WT, int wt_chunks, int K, int act,
+                    size_t APREV, size_t OUT, float *db, float *db2 = nullptr, int db_split = 1 << 30) {
     GemmProb p{};
     p.A = w + DZ; p.a_chunks = pl.H / 64; p.a_c0 = dz_c0; p.kc = kc;
     p.W = w + WT; p.w_chunks = wt_chunks;
@@ -688,14 +713,14 @@ static GemmProb bwd(uint8_t *w, const Plan &pl, float unscale, size_t DZ, int dz
     p.mode = 1; p.act = act;
     p.OUT = w + OUT; p.out_chunks = pl.H / 64; p.out_c0 = 0;
     p.APREV = w + APREV; p.ap_chunks = pl.H / 64; p.ap_c0 = 0;
-    p.db = db; p.db2 = db2; p.db_split = db_split; p.db_scale = unscale;
+    p.db = db; p.db2 = db2; p.db_split = db_split; p.db_scale = unscale; p.db_mul = mul;
     return p;
 }
 // dW[out][in] = sum_rows DZ[row][out] * A[row][in]
-static WgProb wg(uint8_t *w, const Plan &pl, float unscale, size_t DZ, int dz_c0, int out_n, size_t A, int a_chunks, int in_units, int w_off, int ldw,
+static WgProb wg(uint8_t *w, const Plan &pl, float unscale, const float *mul, size_t DZ, int dz_c0, int out_n, size_t A, int a_chunks, int in_units, int w_off, int ldw,
                  int in_lo, int in_hi, int bias_col, int b_off) {
     WgProb p{};
-    p.scale = unscale;
+    p.scale = unscale; p.scale_mul = mul;
     const bool swap = out_n < 128;   // 64 output units (H = 128: the H/2-wide layers): they become the MMA's N, the inputs its M
     const uint8_t *dz = w + DZ, *a = w + A;
     if (!swap) {
@@ -777,8 +802,9 @@ int pime_ppo_grad_tc(const pime_ppo_args *a, void *work_tc, float *grad, void *s
     float pow2B = 1.0f;
     while (pow2B < (float)a->batch) pow2B *= 2.0f;
     c.dz_scale[0] = pow2B;            // actor: |d out| B is O(advantage * ratio / std)
-    c.dz_scale[1] = pow2B * 16.0f;    // critic: |d out| B <= 1 / (std(r_sum) + 1e-5)
+    c.dz_scale[1] = pow2B * 16.0f;    // critic: |d out| B / inv_cs <= 1
     const float un_a = 1.0f / c.dz_scale[0], un_c = 1.0f / c.dz_scale[1];
+    const float *cs = c.inv_cs;       // the critic's sums leave for grad times inv_cs
 
     const Net &A = pl.act, &C = pl.cri;
     const int actA = ACT_TANH, actC = ACT_RELU;
@@ -842,21 +868,21 @@ int pime_ppo_grad_tc(const pime_ppo_args *a, void *work_tc, float *grad, void *s
         GemmBatch g{};
         float *ga = grad + A.theta_off, *gc = grad + C.theta_off;
         if (mod)   // dZ(cat) = (dZ(net.0) W_net.0) * tanh'(cat); its halves are the bias gradients of other_net.2 | integrator_net.2
-            g.p[g.n++] = bwd(w, pl, un_a, pl.Z[4], 0, HC, pl.WT[4], HC, H, actA, pl.A[2], pl.Z[2], ga + A.src[3], ga + A.src[7], Hh);
+            g.p[g.n++] = bwd(w, pl, un_a, nullptr, pl.Z[4], 0, HC, pl.WT[4], HC, H, actA, pl.A[2], pl.Z[2], ga + A.src[3], ga + A.src[7], Hh);
         else       // dZ(net.2) = (dZ(net.4) W_net.4) * tanh'
-            g.p[g.n++] = bwd(w, pl, un_a, pl.Z[4], 0, HC, pl.WT[4], HC, H, actA, pl.A[2], pl.Z[2], ga + A.src[3]);
-        g.p[g.n++] = bwd(w, pl, un_c, pl.Z[7], 0, HC, pl.WT[7], HC, H, actC, pl.A[6], pl.Z[6], gc + C.src[3]);
+            g.p[g.n++] = bwd(w, pl, un_a, nullptr, pl.Z[4], 0, HC, pl.WT[4], HC, H, actA, pl.A[2], pl.Z[2], ga + A.src[3]);
+        g.p[g.n++] = bwd(w, pl, un_c, cs, pl.Z[7], 0, HC, pl.WT[7], HC, H, actC, pl.A[6], pl.Z[6], gc + C.src[3]);
         if (int rc = run_gemm(g)) return rc;
     }
     {
         GemmBatch g{};
         if (mod) {
-            g.p[g.n++] = bwd(w, pl, un_a, pl.Z[2], 0, Hh / 64, pl.WT[2], Hh / 64, H, actA, pl.A[0], pl.Z[0], nullptr);          // -> dZ(other_net.0)
-            g.p[g.n++] = bwd(w, pl, un_a, pl.Z[2], Hh / 64, Hh / 64, pl.WT[3], Hh / 64, H, actA, pl.A[1], pl.Z[1], nullptr);    // -> dZ(integrator_net.0)
+            g.p[g.n++] = bwd(w, pl, un_a, nullptr, pl.Z[2], 0, Hh / 64, pl.WT[2], Hh / 64, H, actA, pl.A[0], pl.Z[0], nullptr);          // -> dZ(other_net.0)
+            g.p[g.n++] = bwd(w, pl, un_a, nullptr, pl.Z[2], Hh / 64, Hh / 64, pl.WT[3], Hh / 64, H, actA, pl.A[1], pl.Z[1], nullptr);    // -> dZ(integrator_net.0)
         } else {
-            g.p[g.n++] = bwd(w, pl, un_a, pl.Z[2], 0, HC, pl.WT[2], HC, H, actA, pl.A[0], pl.Z[0], nullptr);
+            g.p[g.n++] = bwd(w, pl, un_a, nullptr, pl.Z[2], 0, HC, pl.WT[2], HC, H, actA, pl.A[0], pl.Z[0], nullptr);
         }
-        g.p[g.n++] = bwd(w, pl, un_c, pl.Z[6], 0, HC, pl.WT[6], HC, H, actC, pl.A[5], pl.Z[5], nullptr);
+        g.p[g.n++] = bwd(w, pl, un_c, cs, pl.Z[6], 0, HC, pl.WT[6], HC, H, actC, pl.A[5], pl.Z[5], nullptr);
         if (int rc = run_gemm(g)) return rc;
     }
     // ---- weight gradients: all matrices in one launch
@@ -866,22 +892,23 @@ int pime_ppo_grad_tc(const pime_ppo_args *a, void *work_tc, float *grad, void *s
         auto W_ = [&](const Net &d, int j) { return d.theta_off + d.src[j]; };
         const int S = c.S;
         if (mod) {
-            g.p[g.n++] = wg(w, pl, un_a, pl.Z[0], 0, H, pl.X, 1, 64, W_(A, 0), A.So, 0, A.So, kBiasCol, W_(A, 1));                 // other_net.0
-            g.p[g.n++] = wg(w, pl, un_a, pl.Z[1], 0, H, pl.X, 1, 64, W_(A, 4), S - A.So, A.So, S, kBiasCol, W_(A, 5));            // integrator_net.0
-            g.p[g.n++] = wg(w, pl, un_a, pl.Z[2], 0, Hh, pl.A[0], HC, H, W_(A, 2), H, 0, H, -1, 0);                               // other_net.2
-            g.p[g.n++] = wg(w, pl, un_a, pl.Z[2], Hh / 64, Hh, pl.A[1], HC, H, W_(A, 6), H, 0, H, -1, 0);                         // integrator_net.2
-            g.p[g.n++] = wg(w, pl, un_a, pl.Z[4], 0, H, pl.A[2], HC, H, W_(A, 8), H, 0, H, -1, 0);                                // net.0
+            g.p[g.n++] = wg(w, pl, un_a, nullptr, pl.Z[0], 0, H, pl.X, 1, 64, W_(A, 0), A.So, 0, A.So, kBiasCol, W_(A, 1));                 // other_net.0
+            g.p[g.n++] = wg(w, pl, un_a, nullptr, pl.Z[1], 0, H, pl.X, 1, 64, W_(A, 4), S - A.So, A.So, S, kBiasCol, W_(A, 5));            // integrator_net.0
+            g.p[g.n++] = wg(w, pl, un_a, nullptr, pl.Z[2], 0, Hh, pl.A[0], HC, H, W_(A, 2), H, 0, H, -1, 0);                               // other_net.2
+            g.p[g.n++] = wg(w, pl, un_a, nullptr, pl.Z[2], Hh / 64, Hh, pl.A[1], HC, H, W_(A, 6), H, 0, H, -1, 0);                         // integrator_net.2
+            g.p[g.n++] = wg(w, pl, un_a, nullptr, pl.Z[4], 0, H, pl.A[2], HC, H, W_(A, 8), H, 0, H, -1, 0);                                // net.0
         } else {
-            g.p[g.n++] = wg(w, pl, un_a, pl.Z[0], 0, H, pl.X, 1, 64, W_(A, 0), S, 0, S, kBiasCol, W_(A, 1));
-            g.p[g.n++] = wg(w, pl, un_a, pl.Z[2], 0, H, pl.A[0], HC, H, W_(A, 2), H, 0, H, -1, 0);
-            g.p[g.n++] = wg(w, pl, un_a, pl.Z[4], 0, H, pl.A[2], HC, H, W_(A, 4), H, 0, H, -1, 0);
+            g.p[g.n++] = wg(w, pl, un_a, nullptr, pl.Z[0], 0, H, pl.X, 1, 64, W_(A, 0), S, 0, S, kBiasCol, W_(A, 1));
+            g.p[g.n++] = wg(w, pl, un_a, nullptr, pl.Z[2], 0, H, pl.A[0], HC, H, W_(A, 2), H, 0, H, -1, 0);
+            g.p[g.n++] = wg(w, pl, un_a, nullptr, pl.Z[4], 0, H, pl.A[2], HC, H, W_(A, 4), H, 0, H, -1, 0);
         }
-        g.p[g.n++] = wg(w, pl, un_c, pl.Z[5], 0, H, pl.X, 1, 64, W_(C, 0), S, 0, S, kBiasCol, W_(C, 1));
-        g.p[g.n++] = wg(w, pl, un_c, pl.Z[6], 0, H, pl.A[5], HC, H, W_(C, 2), H, 0, H, -1, 0);
-        g.p[g.n++] = wg(w, pl, un_c, pl.Z[7], 0, H, pl.A[6], HC, H, W_(C, 4), H, 0, H, -1, 0);
+        g.p[g.n++] = wg(w, pl, un_c, cs, pl.Z[5], 0, H, pl.X, 1, 64, W_(C, 0), S, 0, S, kBiasCol, W_(C, 1));
+        g.p[g.n++] = wg(w, pl, un_c, cs, pl.Z[6], 0, H, pl.A[5], HC, H, W_(C, 2), H, 0, H, -1, 0);
+        g.p[g.n++] = wg(w, pl, un_c, cs, pl.Z[7], 0, H, pl.A[6], HC, H, W_(C, 4), H, 0, H, -1, 0);
         int mx = 1;
         for (int i = 0; i < g.n; ++i) mx = g.p[i].m_tiles * g.p[i].n_tiles > mx ? g.p[i].m_tiles * g.p[i].n_tiles : mx;
         int split = RT < 32 ? RT : 32;
+        if (RT > split * kWgMaxTiles) split = (RT + kWgMaxTiles - 1) / kWgMaxTiles;
         if (int rc = launch_batch(wgrad_mn_kernel, g, dim3(mx, split, g.n), kWgThreads, kWgSmem, s)) return rc;
     }
     return PIME_OK;
