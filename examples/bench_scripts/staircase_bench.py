@@ -1,6 +1,6 @@
 """Scheduled staircase (robustness map) throughput against the plain fused rollout of the same number of steps.
 
-    python examples/bench_scripts/staircase_bench.py [--reps 5] [--arm all|response]
+    python examples/bench_scripts/staircase_bench.py [--reps 5] [--arm all|response|gains]
 
 Cases (env-steps/s = envs x K x L / time, CUDA events, after a warm-up launch of every shape):
   wt  2^20 envs, Modular-256 actor, staircase 3, 6, 9, 4, 2 x 500 steps
@@ -18,6 +18,10 @@ Then the step response (--arm response runs this arm alone): the metrics-only la
 (settle, rise, effort, peak action per env and segment, the Tracked kernels), alternated rep by rep, for the agent on the
 water tank (2^20 envs, Modular-256, 5 x 500 steps) and pH (2^23 envs, Modular-128, 5 x 50 steps) and for the linear
 baseline in f32 on the water tank (2^23 envs, 5 x 500 steps).
+Then per-env controller gains (--arm gains runs this arm alone): the step-response launch with one shared K against the
+gain launch whose [S, n] K matrix has that K in every column (the same work), alternated rep by rep, median of the reps,
+on the same three shapes; and one real gain x plant map, 64 x 64 (kp, ki) integrator gains x 2048 (a1, a2, Kp) rows =
+2^23 envs, linear f32, 5 x 500 steps, with the step response.
 Prints the GPU name and power limit of the run first.
 """
 import argparse
@@ -152,10 +156,62 @@ def response_arm(reps):
         torch.cuda.empty_cache()
 
 
+def gains_arm(reps):
+    """metrics-only launches with the step response: shared K against a K matrix of equal columns, alternated rep by rep"""
+    runs = (("wt agent  Modular-256 f32", "wt", 1 << 20, 256, 500, SC.WT_INTEGRATOR_SETPOINTS, [0.0, 0.4, -0.4, 0.0], "agent"),
+            ("ph agent  Modular-128 f32", "ph", 1 << 23, 128, 50, SC.PH_SETPOINTS, [-0.02, 0.02, 0.035], "agent"),
+            ("wt linear f32            ", "wt", 1 << 23, 0, 500, SC.WT_INTEGRATOR_SETPOINTS, [0.0, 0.4, -0.4, 0.0], "linear"))
+    for name, plant, n, H, steps, setpoints, K, policy in runs:
+        pack = modular_pack(4 if plant == "wt" else 3, H) if policy == "agent" else None
+        env = V.WaterTankVec(n) if plant == "wt" else V.PHVec(n)
+        env.reset()
+        Kmat = torch.tensor(K, dtype=torch.float64, device="cuda")[:, None].expand(len(K), n).contiguous()
+        kw = dict(actor=pack, setpoints=setpoints, steps=steps, policy=policy, response=True)
+        shared = lambda: SC.staircase_metrics(env, K, **kw)        # noqa: E731
+        per_env = lambda: SC.staircase_metrics(env, Kmat, **kw)    # noqa: E731
+        shared()
+        per_env()
+        torch.cuda.synchronize()
+        t0, t1 = [], []
+        for _ in range(reps):
+            t0.append(timed(shared))
+            t1.append(timed(per_env))
+        env.check_status()
+        a, b = np.median(t0), np.median(t1)
+        steps_total = n * len(setpoints) * steps
+        print(f"  {name} n=2^{n.bit_length() - 1} K={len(setpoints)} L={steps}: shared K {a * 1e3:9.2f} ms "
+              f"({steps_total / a:.3e} env-steps/s, min {min(t0) * 1e3:.2f}, max {max(t0) * 1e3:.2f}), per-env K "
+              f"{b * 1e3:9.2f} ms ({steps_total / b:.3e}, min {min(t1) * 1e3:.2f}, max {max(t1) * 1e3:.2f}); "
+              f"per-env / shared {b / a:.4f}", flush=True)
+        del env, Kmat
+        torch.cuda.empty_cache()
+    # the map: u = kp (r - h2) + ki I, i.e. K = [0, kp, -kp, -ki], gain g on plant rows g m .. g m + m - 1
+    rng = np.random.default_rng(2)
+    m, steps, setpoints = 2048, 500, SC.WT_INTEGRATOR_SETPOINTS
+    P = np.stack([rng.uniform(0.0015, 0.0024, m), rng.uniform(0.0015, 0.0024, m), rng.uniform(0.07, 0.17, m)], 1)
+    kp, ki = np.meshgrid(np.linspace(0.05, 1.0, 64), np.linspace(0.0, 0.05, 64), indexing="ij")
+    Kg = np.stack([0 * kp, kp, -kp, -ki]).reshape(4, -1)
+    Kmap = torch.as_tensor(np.repeat(Kg, m, axis=1), device="cuda")
+    params = np.tile(P, (Kg.shape[1], 1))
+    n = params.shape[0]
+    env = V.WaterTankVec(n, max_step=steps)
+    env.reset()
+    env.reset_changable_parameters(torch.as_tensor(params[:, 0]), torch.as_tensor(params[:, 1]), torch.as_tensor(params[:, 2]))
+    run = lambda: SC.staircase_metrics(env, Kmap, setpoints=setpoints, steps=steps, policy="linear", response=True)  # noqa: E731
+    res = run()
+    t = [timed(run) for _ in range(reps)]
+    env.check_status()
+    f = np.median(t)
+    settled = (res["settle"] < steps).double().mean().item()
+    print(f"  gain map 64 x 64 (kp, ki) x {m} plants = 2^{n.bit_length() - 1} envs, linear f32, K=5 L={steps}: "
+          f"{f * 1e3:9.2f} ms  {n * len(setpoints) * steps / f:.3e} env-steps/s (min {min(t) * 1e3:.2f}, "
+          f"max {max(t) * 1e3:.2f} ms); {settled:.1%} of the segments settle inside 2 %", flush=True)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=5)
-    ap.add_argument("--arm", choices=("all", "response"), default="all")
+    ap.add_argument("--arm", choices=("all", "response", "gains"), default="all")
     args = ap.parse_args()
     assert torch.cuda.is_available(), "needs a CUDA device"
     q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
@@ -164,6 +220,10 @@ def main():
     if args.arm == "response":
         print("step response: metrics-only launch without / with response=True", flush=True)
         response_arm(args.reps)
+        return
+    if args.arm == "gains":
+        print("per-env gains: step-response launch with a shared K / with a [S, n] K matrix of equal columns", flush=True)
+        gains_arm(args.reps)
         return
     rng = np.random.default_rng(1)
     n = 1 << 20
@@ -177,6 +237,8 @@ def main():
     linear_case(args.reps)
     print("step response: metrics-only launch without / with response=True", flush=True)
     response_arm(args.reps)
+    print("per-env gains: step-response launch with a shared K / with a [S, n] K matrix of equal columns", flush=True)
+    gains_arm(args.reps)
 
 
 if __name__ == "__main__":

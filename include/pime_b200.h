@@ -382,6 +382,35 @@ int pime_ph_rollout_schedule_response_f64(const pime_ph_config *cfg, const doubl
                                           const pime_rollout_args *args, const pime_schedule *sched,
                                           const pime_schedule_ext *ext, const pime_step_response *resp, void *stream);
 
+/* Scheduled rollout with the step response and per-env controller gains: the launch of the _response entries (ext may be
+ * NULL), with env i's priorK (= -K, S entries, S the observation dimension) taken from column i of a DEVICE matrix instead
+ * of args->priorK_host, for the agent's prior term and for the linear policy:
+ *
+ *   priorK of env i  =  priorK_dev[k * n + i],  k = 0 .. S-1   (i is the env's index in this call, not env_offset + i)
+ *
+ * Each env computes exactly what the _response entries compute from priorK_host equal to its column: a launch whose
+ * columns are all equal is bit-identical to that one.  A gain x plant robustness map is one launch with one column per
+ * (gain, plant) pair.  Besides everything the _response entries reject, these reject (PIME_EINVAL, also without a device
+ * and for n = 0) a NULL gains or priorK_dev, args->priorK_host != NULL (the gains are given exactly once), and the water
+ * tank's PIME_WT_OBS_STACKING (its K spans the frame history, which no gain map tunes).
+ */
+typedef struct pime_schedule_gains {
+    const double *priorK_dev;       /* DEVICE double[S][n]: env i's priorK (= -K) is priorK_dev[k * n + i]    */
+} pime_schedule_gains;
+
+int pime_wt_rollout_schedule_gains_f32(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st,
+                                       const pime_rollout_args *args, const pime_schedule *sched, const pime_schedule_ext *ext,
+                                       const pime_step_response *resp, const pime_schedule_gains *gains, void *stream);
+int pime_wt_rollout_schedule_gains_f64(const pime_wt_config *cfg, int64_t n, const pime_wt_state *st,
+                                       const pime_rollout_args *args, const pime_schedule *sched, const pime_schedule_ext *ext,
+                                       const pime_step_response *resp, const pime_schedule_gains *gains, void *stream);
+int pime_ph_rollout_schedule_gains_f32(const pime_ph_config *cfg, const float *table, int64_t n, const pime_ph_state *st,
+                                       const pime_rollout_args *args, const pime_schedule *sched, const pime_schedule_ext *ext,
+                                       const pime_step_response *resp, const pime_schedule_gains *gains, void *stream);
+int pime_ph_rollout_schedule_gains_f64(const pime_ph_config *cfg, const double *table, int64_t n, const pime_ph_state *st,
+                                       const pime_rollout_args *args, const pime_schedule *sched, const pime_schedule_ext *ext,
+                                       const pime_step_response *resp, const pime_schedule_gains *gains, void *stream);
+
 /* Per-env GAE / reward-to-go reverse scan over a time-major replay (AgentPPO.compute_reward_gae
  * agent.py:685-708 without the final normalisation): reward, mask, value are [T][n] with element stride
  * `stride` floats (4 for buf_other columns, 1 for dense); r_sum, adv are dense [T][n]. */

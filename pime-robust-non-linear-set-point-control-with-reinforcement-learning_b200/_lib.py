@@ -85,6 +85,10 @@ class StepResponse(C.Structure):
     _fields_ = [("response", vp), ("settle_band", C.c_double)]
 
 
+class ScheduleGains(C.Structure):
+    _fields_ = [("priorK_dev", vp)]
+
+
 class PpoArgs(C.Structure):
     _fields_ = [("actor", C.POINTER(ActorConfig)), ("theta", vp), ("theta_t", vp), ("adam_m", vp), ("adam_v", vp),
                 ("grad_out", vp), ("buf_state", vp), ("buf_action", vp), ("buf_r_sum", vp), ("buf_logprob", vp),
@@ -106,6 +110,8 @@ SYMBOLS = [
     "pime_ph_rollout_schedule_ext_f64",
     "pime_wt_rollout_schedule_response_f32", "pime_wt_rollout_schedule_response_f64", "pime_ph_rollout_schedule_response_f32",
     "pime_ph_rollout_schedule_response_f64",
+    "pime_wt_rollout_schedule_gains_f32", "pime_wt_rollout_schedule_gains_f64", "pime_ph_rollout_schedule_gains_f32",
+    "pime_ph_rollout_schedule_gains_f64",
     "pime_gae_scan", "pime_reduce_episode_stats_f32", "pime_reduce_episode_stats_f64",
     "pime_ppo_theta_count", "pime_ppo_theta_layout", "pime_ppo_work_floats", "pime_ppo_transpose", "pime_ppo_step", "pime_ppo_apply_grad",
     "pime_ppo_tc_work_bytes", "pime_ppo_tc_layout", "pime_ppo_grad_tc", "pime_ppo_close_step",

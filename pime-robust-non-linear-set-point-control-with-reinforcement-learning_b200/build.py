@@ -18,7 +18,8 @@ LIB = os.path.join(HERE, "libpime_b200.so")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 
 SOURCES = ["common.cu", "step.cu", "actor.cu", "learner.cu", "learner_tc.cu", "rollout_wt_f32.cu", "rollout_wt_f64.cu", "rollout_ph_f32.cu", "rollout_ph_f64.cu",
-           "rollout_track_wt_f32.cu", "rollout_track_wt_f64.cu", "rollout_track_ph_f32.cu", "rollout_track_ph_f64.cu"]
+           "rollout_track_wt_f32.cu", "rollout_track_wt_f64.cu", "rollout_track_ph_f32.cu", "rollout_track_ph_f64.cu",
+           "rollout_gain_wt_f32.cu", "rollout_gain_wt_f64.cu", "rollout_gain_ph_f32.cu", "rollout_gain_ph_f64.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
               "--expt-relaxed-constexpr", "-Xptxas", "-v", "-I", INCLUDE]
 

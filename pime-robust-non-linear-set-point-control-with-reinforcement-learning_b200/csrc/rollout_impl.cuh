@@ -42,6 +42,7 @@ template <typename T, bool STACK> struct WtGlue {
     using Real = T;
     static constexpr int kObsMax = STACK ? kMaxFrames : 4;   // widest observation of this plant (loop bounds)
     static constexpr bool kSegmented = false;
+    static constexpr bool kGained = false;
     WtConst<T> c;
     WtPtrs<T> p;
 
@@ -160,6 +161,7 @@ template <typename T> struct PhGlue {
     using Real = T;
     static constexpr int kObsMax = 3;
     static constexpr bool kSegmented = false;
+    static constexpr bool kGained = false;
     PhConst<T> c;
     const T *table;
     PhPtrs<T> p;
@@ -271,6 +273,25 @@ template <typename Glue> struct Tracked : Segmented<Glue> {
     };
 };
 
+// Per-env controller gains of a scheduled launch with the step response (pime_schedule_gains): env i's priorK (= -K) is
+// column i of a [S][n] device matrix instead of the launch's one RolloutParams::priorK.  Gained<Glue> is a Tracked<Glue>
+// whose Stepper reads the env's gain k from that matrix each time it needs it, in fp64, and rounds it exactly as it rounds
+// RolloutParams::priorK[k], so each env computes what a shared launch with priorK equal to its column computes.  The read
+// is coalesced (consecutive envs are consecutive threads) and L1 / L2-resident: the resident CTAs' columns are a few MB.
+// Keeping the gains in registers instead spills in tcgen05 kernels that are at the 128-register limit (DESIGN.md §4).
+// Every other glue has kGained = false, for which none of it generates code.  Its kernels live in objects of their own
+// (rollout_gain_*), without the stacking observation.
+struct GainParams {
+    const double *priorK;   // [S][n]: env i's priorK[k] is priorK[k * n + i]
+};
+
+template <typename Glue> struct Gained : Tracked<Glue> {
+    static constexpr bool kGained = true;
+    GainParams gn;
+    // env i's priorK[k] (k < S); a tail row shadows env n - 1 (i < n), so the read stays inside the matrix
+    __device__ __forceinline__ double gain(int k, int64_t i, int64_t n) const { return __ldg(gn.priorK + (int64_t)k * n + i); }
+};
+
 template <typename T> __device__ __forceinline__ T prior_k(const RolloutParams &rp, int k);
 template <> __device__ __forceinline__ float prior_k<float>(const RolloutParams &rp, int k) { return rp.priorKf[k]; }
 template <> __device__ __forceinline__ double prior_k<double>(const RolloutParams &rp, int k) { return rp.priorK[k]; }
@@ -283,6 +304,22 @@ template <typename Plant> struct Stepper {
     using N = Num<T>;
     double s_ret = 0.0, s_ret2 = 0.0, s_cnt = 0.0, s_err = 0.0, s_rew = 0.0, s_steps = 0.0;
     bool fault = false;
+
+    // Gain k of env ii's prior: the launch's priorK, or with Plant::kGained the env's own (Gained<Glue>), rounded alike.
+    // gain_f is the fp32 factor of the deterministic prior term (float(priorK)), gain the plant-dtype one of the stochastic
+    // term, neg_gain the K = -priorK of the linear policy.
+    static __device__ __forceinline__ float gain_f(const Plant &plant, const RolloutParams &rp, int64_t ii, int k) {
+        if constexpr (Plant::kGained) return (float)plant.gain(k, ii, rp.n);
+        else return rp.priorKf[k];
+    }
+    static __device__ __forceinline__ T gain(const Plant &plant, const RolloutParams &rp, int64_t ii, int k) {
+        if constexpr (Plant::kGained) return (T)plant.gain(k, ii, rp.n);
+        else return prior_k<T>(rp, k);
+    }
+    static __device__ __forceinline__ T neg_gain(const Plant &plant, const RolloutParams &rp, int64_t ii, int k) {
+        if constexpr (Plant::kGained) return (T)(-plant.gain(k, ii, rp.n));
+        else return (T)(-rp.priorK[k]);
+    }
 
     // The part of a step that does not depend on the network output: exploration / process noise (Philox + Box-Muller, or
     // the injected arrays) and the prior term obs32 . priorK.  The fused kernel runs it BEFORE it waits for net(obs), i.e.
@@ -312,13 +349,13 @@ template <typename Plant> struct Stepper {
             float prior = 0.0f;
 #pragma unroll
             for (int k = 0; k < Plant::kObsMax; ++k)
-                if (k < S) prior = fmaf(obs[k], rp.priorKf[k], prior);
+                if (k < S) prior = fmaf(obs[k], gain_f(plant, rp, ii, k), prior);
             p_prior_f = prior;
         } else {
             T prior = (T)0;
 #pragma unroll
             for (int k = 0; k < Plant::kObsMax; ++k)
-                if (k < S) prior = N::add(prior, N::mul((T)obs[k], prior_k<T>(rp, k)));
+                if (k < S) prior = N::add(prior, N::mul((T)obs[k], gain(plant, rp, ii, k)));
             p_prior = prior;
         }
     }
@@ -329,14 +366,15 @@ template <typename Plant> struct Stepper {
     // fused multiply-add per term (prior_kernel<float>'s acc + obs * K compiles to that FFMA chain; fmaf pins it here).
     // Negating priorK and the sum is exact, so the action is the one pime_prior_action computes from the same state.
     T p_linear = (T)0;
-    __device__ __forceinline__ void linear_action(const Plant &plant, const RolloutParams &rp, const typename Plant::Env &env) {
+    __device__ __forceinline__ void linear_action(const Plant &plant, const RolloutParams &rp, const typename Plant::Env &env,
+                                                  int64_t ii) {
         T st[Plant::kObsMax];
         plant.observe_state(env, st);
         T acc = (T)0;
 #pragma unroll
         for (int k = 0; k < Plant::kObsMax; ++k) {
             if (k >= rp.S) continue;
-            const T K = (T)(-rp.priorK[k]);
+            const T K = neg_gain(plant, rp, ii, k);
             if constexpr (sizeof(T) == 4) acc = fmaf(st[k], K, acc);
             else acc = N::add(acc, N::mul(st[k], K));
         }
@@ -349,7 +387,7 @@ template <typename Plant> struct Stepper {
     __device__ __forceinline__ void step(const Plant &plant, const RolloutParams &rp, typename Plant::Env &env,
                                          const float (&obs)[kMaxS], float a_avg, int s, int64_t ii, bool live) {
         prepare(plant, rp, obs, s, ii);
-        if constexpr (LINEAR) linear_action(plant, rp, env);
+        if constexpr (LINEAR) linear_action(plant, rp, env, ii);
         finish<LINEAR>(plant, rp, env, obs, a_avg, s, ii, live);
     }
 
@@ -732,11 +770,17 @@ int launch_rollout_actor(const Plant &plant, const RolloutParams &rp, const tc::
 }
 
 // the plain launch of glue g, or the scheduled one (Segmented<Glue>) when sg is given.  TRACK: the scheduled launch with
-// the step response (Tracked<Glue>, sg and tr given); it instantiates the Tracked kernels alone.
-template <bool MODULAR, bool TRACK = false, typename Glue>
+// the step response (Tracked<Glue>, sg and tr given); it instantiates the Tracked kernels alone.  GAIN (with TRACK): the
+// same with per-env gains (Gained<Glue>, gn given); it instantiates the Gained kernels alone.
+template <bool MODULAR, bool TRACK = false, bool GAIN = false, typename Glue>
 int launch_rollout_glue(const Glue &g, const SegParams *sg, const RolloutParams &rp, const tc::PackLayout &L,
-                        const pime_rollout_args *a, cudaStream_t stream, const TrackParams *tr = nullptr) {
-    if constexpr (TRACK) {
+                        const pime_rollout_args *a, cudaStream_t stream, const TrackParams *tr = nullptr,
+                        const GainParams *gn = nullptr) {
+    static_assert(TRACK || !GAIN, "per-env gains go with the step response");
+    if constexpr (GAIN) {
+        return launch_rollout_actor<Gained<Glue>, MODULAR>(Gained<Glue>{Tracked<Glue>{Segmented<Glue>{g, *sg}, *tr}, *gn}, rp,
+                                                           L, a, stream);
+    } else if constexpr (TRACK) {
         return launch_rollout_actor<Tracked<Glue>, MODULAR>(Tracked<Glue>{Segmented<Glue>{g, *sg}, *tr}, rp, L, a, stream);
     } else {
         if (sg) return launch_rollout_actor<Segmented<Glue>, MODULAR>(Segmented<Glue>{g, *sg}, rp, L, a, stream);
@@ -785,11 +829,21 @@ inline int fill_track_params(const pime_step_response *resp, const SegParams &sg
     return PIME_OK;
 }
 
-// Fills RolloutParams from the public argument block; returns the pack layout in L when an actor is given.
-inline int fill_rollout_params(const pime_rollout_args *a, int64_t n, int S, RolloutParams &rp, tc::PackLayout &L) {
+// Checks a per-env gain block and fills GainParams (host arithmetic only).
+inline int fill_gain_params(const pime_schedule_gains *gains, GainParams &gn) {
+    PIME_REQUIRE(gains && gains->priorK_dev, "null gain block / priorK_dev");
+    gn = GainParams{gains->priorK_dev};
+    return PIME_OK;
+}
+
+// Fills RolloutParams from the public argument block; returns the pack layout in L when an actor is given.  gains: the
+// launch takes per-env gains (GainParams), so priorK_host must be NULL and RolloutParams::priorK stays zero.
+inline int fill_rollout_params(const pime_rollout_args *a, int64_t n, int S, RolloutParams &rp, tc::PackLayout &L,
+                               bool gains = false) {
     PIME_REQUIRE(a, "null rollout args");
     PIME_REQUIRE(a->T >= 1, "T must be >= 1");
-    PIME_REQUIRE(a->priorK_host, "priorK_host is required (pass zeros for no prior)");
+    if (gains) PIME_REQUIRE(a->priorK_host == nullptr, "priorK_host must be NULL with per-env gains (priorK_dev)");
+    else PIME_REQUIRE(a->priorK_host, "priorK_host is required (pass zeros for no prior)");
     PIME_REQUIRE(S >= 1 && S <= kMaxS, "observation dim");
     PIME_REQUIRE((a->buf_state == nullptr) == (a->buf_other == nullptr), "buf_state/buf_other must both be given or both NULL");
     PIME_REQUIRE((a->pnoise1 == nullptr) == (a->pnoise2 == nullptr), "pnoise1/pnoise2 must both be given or both NULL");
@@ -802,7 +856,7 @@ inline int fill_rollout_params(const pime_rollout_args *a, int64_t n, int S, Rol
     rp.reward_scale = a->reward_scale; rp.gamma = a->gamma; rp.seed = a->seed; rp.env_offset = a->env_offset; rp.tick0 = a->tick0;
     rp.S = S;
     for (int k = 0; k < kMaxS; ++k) {
-        rp.priorK[k] = k < S ? a->priorK_host[k] : 0.0;
+        rp.priorK[k] = k < S && a->priorK_host ? a->priorK_host[k] : 0.0;
         rp.priorKf[k] = (float)rp.priorK[k];
     }
     rp.reward_scale_f = (float)a->reward_scale;

@@ -19,7 +19,9 @@ linear baseline (get_linear_action, computed in the plant dtype) as well as the 
 every env or a [K, n] matrix of per-env set-points (e.g. random staircases in [r_lo, r_hi], or a map over set-point
 sequence x ensemble parameters).  With ``response=True`` the same launch also returns each segment's step response --
 settling time, rise time, control effort (total variation of the action) and peak action -- without any trajectory, so a
-map can show where a policy commands more than the actuator takes.  ``staircase(policy='linear')`` keeps the per-step
+map can show where a policy commands more than the actuator takes.  Both also take the controller gains K per env ([S, n],
+column i for env i), which is what a gain x plant map -- the fairness of the linear baseline, or the sensitivity of the
+residual agent to the prior it runs over (fix_K) -- needs, in the same one launch.  ``staircase(policy='linear')`` keeps the per-step
 loop of the prior kernel + the step kernel, which returns the same trajectories in fp64 and is what the fused linear
 policy is tested against.
 """
@@ -67,13 +69,18 @@ def _scheduled(vec, K, actor, setpoints, steps, resample_params, start, trajecto
         raise ValueError("policy must be 'agent' or 'linear'")
     if policy == "linear" and actor is not None:
         raise ValueError("the linear policy takes no actor")
-    K = np.asarray(K, dtype=np.float64).reshape(-1)
+    if np.ndim(K) > 2:
+        raise ValueError("K must be [S] or [S, n]")
+    if np.ndim(K) == 2:   # per-env gains: column i is env i's K
+        priorK = -torch.as_tensor(K, dtype=torch.float64)
+    else:
+        priorK = -np.asarray(K, dtype=np.float64).reshape(-1)[:vec.state_dim]
     with _staircase_setup(vec, setpoints, steps) as (setpoints, steps):
         if _is_wt(vec):
             vec.set_state(*start)
         else:
             vec.x.fill_(float(start[0]))
-        return vec.rollout_schedule(setpoints, steps, -K[:vec.state_dim], actor=actor, deterministic=True,
+        return vec.rollout_schedule(setpoints, steps, priorK, actor=actor, deterministic=True,
                                     replay=trajectories, want_actions=trajectories, resample_params=resample_params,
                                     policy="actor" if policy == "agent" else "linear", response=response,
                                     settle_band=settle_band)
@@ -104,13 +111,18 @@ def staircase(vec, policy: str, K, actor: Optional[V.ActorPack] = None, setpoint
 
     policy = 'agent': deterministic ``tanh(net(obs)) + obs @ (-K)`` (``actor`` = the agent's ActorPack; None = prior only);
     policy = 'linear': ``clip(-obs @ K, -1, 1)`` for the water tank (get_P_action), ``-obs @ K`` for pH (ph.py:227-231).
+    K: [S], or [S, n] with column i for env i (policy='agent' only: the linear policy's per-step loop takes one K).
     Returns time-major arrays over all segments: obs [T, n, S] (the states the policy saw), xs [T, n, 2] (levels) or
     ys [T, n] (pH), refs [T, n], actions [T, n], rewards [T, n], totals [T, n] (running sum), integrators [T, n] or None.
     """
     wt = _is_wt(vec)
     # stacking observation: set_state / set_r do not touch the frame history (nonlinear_watertank.py:205-212 are inherited
     # unchanged), so the first num_stack observations of a segment still show the frames of the reset -- reproduced
-    K = np.asarray(K, dtype=np.float64).reshape(-1)
+    if np.ndim(K) == 2:
+        if policy == "linear":
+            raise ValueError("staircase(policy='linear') takes one K ([S]); per-env gains go through staircase_metrics")
+    else:
+        K = np.asarray(K, dtype=np.float64).reshape(-1)
     S = vec.state_dim
     if policy == "agent":
         out = _scheduled(vec, K, actor, setpoints, steps, resample_params, start, True)
@@ -155,8 +167,9 @@ def staircase_metrics(vec, K, actor: Optional[V.ActorPack] = None, setpoints=Non
     [K, n] float64 (segment k, env i).  With y the controlled output (h2 / pH) and e = r - y: ret = sum of rewards, iae =
     sum of |e| over the segment's steps, final_err = |e| after its last step, overshoot = max(0, max of d (y - r)) with
     d = +1 when the segment starts below its set-point, -1 when above.
-    policy: 'agent' or 'linear' as in ``staircase`` (K is the reference's K; 'linear' takes no actor).  setpoints: K
-    floats for every env, or a [K, n] array / tensor (column i: env i's staircase).
+    policy: 'agent' or 'linear' as in ``staircase`` (K is the reference's K; 'linear' takes no actor).  K: [S] for every
+    env, or a [S, n] array / tensor (column i: env i's K; not with the stacking observation).  setpoints: K floats for
+    every env, or a [K, n] array / tensor (column i: env i's staircase).
     response=True adds the step response of each segment, [K, n] float64 each, computed in the same launch (L steps per
     segment, j = 0 .. L-1, u_j the action fed to the plant, y_b the output at the segment begin, D = |r - y_b|):
     settle = 1 + the last j with |e_j| > settle_band D (0: always inside the band, L: not settled); rise = 1 + the first j
@@ -177,7 +190,19 @@ def robust_map(K, params, actor: Optional[V.ActorPack] = None, plant: str = "wt"
     (qww_V, qc_V) with the discretised system refreshed (set_params(update_system=True)), steps default
     max_episode_steps.  The ensemble parameters are kept between segments (if_reset_all = False).  A grid over the axes
     is one np.meshgrid (or parameter_grid) in the caller.  response / settle_band: the step response, as in
-    staircase_metrics.  Returns (metrics dict as staircase_metrics, params array)."""
+    staircase_metrics.  Returns (metrics dict as staircase_metrics, params array).
+
+    K: the reference's K (= -priorK), [S] for every row, or [S, n] with column i for parameter row i.  A gain x plant map
+    is one np.repeat / np.tile in the caller; e.g. the water-tank integrator loop u = kp (r - h2) + ki I, i.e.
+    K = [0, kp, -kp, -ki], over a (kp, ki) grid times a plant grid P ([m, 3]):
+
+        kp, ki = np.meshgrid(kps, kis, indexing="ij")                        # G = kp.size gains
+        Kg = np.stack([0 * kp, kp, -kp, -ki]).reshape(4, -1)                  # [4, G]
+        K = np.repeat(Kg, len(P), axis=1)                                     # gain g for rows g m .. g m + m - 1
+        metrics, p = robust_map(K, np.tile(P, (Kg.shape[1], 1)), policy="linear", response=True)
+
+    (metrics[...][k].reshape(G, m) is then the map of segment k).  The ensemble parameter Kp in ``params`` is the pump
+    constant of the plant (nonlinear_watertank.py), not a controller gain."""
     if plant == "wt":
         p = np.asarray(params, dtype=np.float64).reshape(-1, 3)
         steps = int(steps or 500)

@@ -109,10 +109,11 @@ def _rollout_args(env, T, actor, priorK, deterministic, auto_reset, reward_scale
         a.actor_pack = L.ptr(actor.pack)
         if a_std_log is None:
             a.a_std_log = float(actor.a_std_log)
-    pk = np.ascontiguousarray(np.asarray(priorK, dtype=np.float64).reshape(-1))
-    assert pk.shape[0] == S, f"priorK must have {S} entries"
-    keep.append(pk)
-    a.priorK_host = pk.ctypes.data_as(C.POINTER(C.c_double))
+    if priorK is not None:   # None: per-env gains (pime_schedule_gains) take its place
+        pk = np.ascontiguousarray(np.asarray(priorK, dtype=np.float64).reshape(-1))
+        assert pk.shape[0] == S, f"priorK must have {S} entries"
+        keep.append(pk)
+        a.priorK_host = pk.ctypes.data_as(C.POINTER(C.c_double))
     a.deterministic = int(deterministic)
     a.T = int(T)
     a.auto_reset = int(auto_reset)
@@ -190,6 +191,22 @@ def _step_response(env, K, response, settle_band):
         response = torch.empty((4, K, env.n), dtype=torch.float64, device=env.device)
     assert response.shape == (4, K, env.n) and response.dtype == torch.float64 and response.is_cuda and response.is_contiguous()
     return L.StepResponse(response=L.ptr(response), settle_band=float(settle_band)), response
+
+
+def _schedule_gains(env, priorK, keep):
+    """pime_schedule_gains for a [S, n] priorK (column i: env i's priorK = -K), or None for a 1-D one.  Numpy or torch
+    input becomes a float64 contiguous device tensor, kept alive in ``keep`` for the call."""
+    if np.ndim(priorK) > 2:
+        raise ValueError("priorK must be [S] or [S, n]")
+    if np.ndim(priorK) != 2:
+        return None
+    if getattr(env, "obs_mode", None) == "stacking":
+        raise ValueError("per-env gains do not take the stacking observation")
+    pk = torch.as_tensor(priorK).to(device=env.device, dtype=torch.float64).contiguous()
+    if tuple(pk.shape) != (env.state_dim, env.n):
+        raise ValueError(f"per-env priorK must be [{env.state_dim}, {env.n}], got {list(pk.shape)}")
+    keep.append(pk)
+    return L.ScheduleGains(priorK_dev=L.ptr(pk))
 
 
 class _VecBase:
@@ -309,6 +326,9 @@ class WaterTankVec(_VecBase):
         """The set-point staircase in one launch (pime_wt_rollout_schedule_*): T = K * segment_steps fused steps, segment k
         tracking setpoints[k] and beginning with reset(resample_params) -> set_state(levels before it) -> set_r(setpoints[k]).
         setpoints: K floats for every env, or a [K, n] array / tensor whose column i is env i's staircase.
+        priorK: [S] for every env, or a [S, n] array / tensor whose column i is env i's priorK (= -K), for the prior term
+        and the linear policy (pime_wt_rollout_schedule_gains_*: the step response is computed too, and returned only when
+        response is asked for; not with the stacking observation).
         policy = 'actor': the residual policy of ``actor`` (None: the prior term alone); 'linear': get_linear_action,
         clip(state . priorK, -1, 1) in the plant dtype (no actor, deterministic=True).
         Returns rollout()'s dict plus metrics [4, K, n] float64 (ret, iae, final_err, overshoot per segment and env).
@@ -316,13 +336,22 @@ class WaterTankVec(_VecBase):
         segment and env (pime_wt_rollout_schedule_response_*; settle_band in (0, 1) relative to |r - y| at the segment
         begin, see include/pime_b200.h); response=False calls exactly the entries above."""
         keep = []
+        gains = _schedule_gains(self, priorK, keep)
         sc, ext, metrics = _schedule(self, setpoints, segment_steps, resample_params, metrics, policy, keep)
         T = sc.num_segments * sc.segment_steps
-        a, out = _rollout_args(self, T, actor, priorK, deterministic, False, reward_scale, gamma, eps, pnoise, replay,
-                               want_actions, stats, keep, a_std_log)
+        a, out = _rollout_args(self, T, actor, None if gains is not None else priorK, deterministic, False, reward_scale, gamma, eps,
+                               pnoise, replay, want_actions, stats, keep, a_std_log)
+        want_response = response is not False
+        if gains is not None and not want_response:   # the gain entries always compute it: a scratch buffer, not returned
+            response = True
         resp, response = _step_response(self, sc.num_segments, response, settle_band)
         args = (C.byref(self.cfg), C.c_int64(self.n), C.byref(self._st), C.byref(a), C.byref(sc))
-        if resp is not None:
+        if gains is not None:
+            L.check(_fn("pime_wt_rollout_schedule_gains", self.dtype)(*args, None if ext is None else C.byref(ext),
+                                                                      C.byref(resp), C.byref(gains), L.stream_ptr()))
+            if want_response:
+                out["response"] = response
+        elif resp is not None:
             L.check(_fn("pime_wt_rollout_schedule_response", self.dtype)(*args, None if ext is None else C.byref(ext),
                                                                          C.byref(resp), L.stream_ptr()))
             out["response"] = response
@@ -470,15 +499,25 @@ class PHVec(_VecBase):
                          resample_params=False, metrics=True, policy="actor", response=False, settle_band=0.02):
         """The set-point staircase in one launch (pime_ph_rollout_schedule_*): segment k begins with reset(resample_params),
         the state x before it restored (y looked up under the new C) and r = setpoints[k].  policy = 'linear': state . priorK
-        in the plant dtype, not clipped (ph.py:227-231).  See WaterTankVec.rollout_schedule."""
+        in the plant dtype, not clipped (ph.py:227-231).  priorK: [S], or [S, n] per env (pime_ph_rollout_schedule_gains_*).
+        See WaterTankVec.rollout_schedule."""
         keep = []
+        gains = _schedule_gains(self, priorK, keep)
         sc, ext, metrics = _schedule(self, setpoints, segment_steps, resample_params, metrics, policy, keep)
         T = sc.num_segments * sc.segment_steps
-        a, out = _rollout_args(self, T, actor, priorK, deterministic, False, reward_scale, gamma, eps, None, replay,
-                               want_actions, stats, keep, a_std_log)
+        a, out = _rollout_args(self, T, actor, None if gains is not None else priorK, deterministic, False, reward_scale, gamma, eps,
+                               None, replay, want_actions, stats, keep, a_std_log)
+        want_response = response is not False
+        if gains is not None and not want_response:   # the gain entries always compute it: a scratch buffer, not returned
+            response = True
         resp, response = _step_response(self, sc.num_segments, response, settle_band)
         args = (C.byref(self.cfg), L.ptr(self.table), C.c_int64(self.n), C.byref(self._st), C.byref(a), C.byref(sc))
-        if resp is not None:
+        if gains is not None:
+            L.check(_fn("pime_ph_rollout_schedule_gains", self.dtype)(*args, None if ext is None else C.byref(ext),
+                                                                      C.byref(resp), C.byref(gains), L.stream_ptr()))
+            if want_response:
+                out["response"] = response
+        elif resp is not None:
             L.check(_fn("pime_ph_rollout_schedule_response", self.dtype)(*args, None if ext is None else C.byref(ext),
                                                                          C.byref(resp), L.stream_ptr()))
             out["response"] = response
