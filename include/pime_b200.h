@@ -129,7 +129,7 @@ typedef struct pime_ph_config {
     int32_t reserved0;
     double act_low, act_high;   /* 0.0, 1.5 (ph.py:146-147)                                              */
     double sample_t;            /* 20 (ph.py:40)                                                         */
-    double mhcl_step;           /* 1e-5                                                                  */
+    double mhcl_step;           /* 1e-5, the only step accepted (the table index is rint(C*x*1e5))      */
     double distance_threshold, integral_max, integral_punish, action_punishment;
     double kw, kchem, ka, MNaOH, MHA, MNH3; /* chemistry (ph.py:31-36); shared by every env              */
     double qww_lo, qww_hi, qc_lo, qc_hi;    /* ensemble ranges (ph.py:357-358)                           */
@@ -157,9 +157,9 @@ typedef struct pime_ph_state {
 void pime_ph_default_config(pime_ph_config *cfg); /* registered PH1D...Integrator-SqaureDistance-v35 values */
 
 /* PH1D.__init__ titration table (ph.py:72-84).  table_f64[table_len] (required) and table_f32 (may be NULL)
- * are written on the device.  Each grid point's quartic in [H+] is solved for its unique positive root
- * (bisection bracket, then the reference's abs-Newton iteration run to its fixed point); the reference's
- * warm-started 5-step chain converges to the same root, agreement <= 1e-12 relative in pH. */
+ * are written on the device.  The table is the reference's chain itself (5 abs-Newton steps per grid point,
+ * warm-started from the previous one), computed on the host and copied; the call returns when the copies are
+ * done.  PIME_EINVAL unless mhcl_step == 1e-5 (every pH entry point checks it: the table index is rint(C*x*1e5)). */
 int pime_ph_table_build(const pime_ph_config *cfg, double *table_f64, float *table_f32, void *stream);
 
 /* update_system (ph.py:114-121): A = exp(-qww_V*T), B = (1-A)/qww_V, C = qc_V for every env. */

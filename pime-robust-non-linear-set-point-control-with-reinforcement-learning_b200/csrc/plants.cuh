@@ -291,10 +291,18 @@ template <typename T> struct PhPtrs {
 
 inline int ph_obs_dim(const pime_ph_config &c) { return c.integrator_mode == PIME_PH_NO_INTEGRATOR ? 2 : 3; }
 
+// ph_lookup's index rint(C x 1e5) is the reference's first MHCl entry >= around(C x, 5) only on the grid i * 1e-5; any
+// other step would read a wrong entry, so it is rejected rather than looked up differently.
+inline int validate_mhcl_step(const pime_ph_config *cfg) {
+    PIME_REQUIRE(cfg->mhcl_step == 1e-5, "mhcl_step must be 1e-5 (the table index is rint(C x 1e5))");
+    return PIME_OK;
+}
+
 // The argument checks of every pH entry point (step, reset, update_system, rollout, host-buffer rollout), run before
 // require_device().  table_len > 1 also keeps ph_lookup's clamp to the last entry inside the table.
 inline int validate_ph(const pime_ph_config *cfg, int64_t n, const pime_ph_state *st) {
     PIME_REQUIRE(cfg && st, "null config/state");
+    if (int rc = validate_mhcl_step(cfg)) return rc;
     PIME_REQUIRE(n >= 0, "negative n");
     PIME_REQUIRE(st->x && st->y && st->r && st->A && st->B && st->C && st->qww_V && st->qc_V && st->t && st->episode,
                  "null state array");
@@ -305,8 +313,9 @@ inline int validate_ph(const pime_ph_config *cfg, int64_t n, const pime_ph_state
     return PIME_OK;
 }
 
-// observe_state (ph.py:187-189): first i with MHCl[i] >= around(C*x,5)  ==  rint(C*x*1e5)  (MHCl[i] = i*1e-5;
-// equivalence checked on the reference in tests/golden/ph.npz).  The index is computed in fp64 for both table types.
+// observe_state (ph.py:187-189): first i with MHCl[i] >= around(C*x,5)  ==  rint(C*x*1e5)  (MHCl[i] = i*1e-5, which
+// validate_mhcl_step enforces; equivalence checked on the reference in tests/golden/ph.npz and against the oracle's
+// index).  The index is computed in fp64 for both table types.
 // Returns false when past the table (IndexError).
 template <typename T>
 __device__ __forceinline__ bool ph_lookup(const T *__restrict__ table, int table_len, double C, double x, T &y) {

@@ -2,6 +2,8 @@
 // GAE scan, episode statistics.  One thread per env, SoA state, grid-stride over a grid sized in multiples of
 // the SM count.  HBM-bound in fp32 (57 B / env-step water tank, 53 B pH; DESIGN.md section 4).
 #include <initializer_list>
+#include <new>
+#include <vector>
 
 #include "plants.cuh"
 
@@ -319,40 +321,28 @@ __global__ void __launch_bounds__(kBlock) ph_update_system_kernel(double sample_
     }
 }
 
-// Titration table (ph.py:72-84).  One thread per grid point: the quartic f(H) = H^4 + a H^3 + b H^2 + c H + d has
-// d < 0 and exactly one positive root; bracket it by bisection on [1e-30, 4] (f(lo) < 0 < f(hi)), then run the
-// reference's own iteration H <- |H - f/f'| until it stops moving (its fixed point is what the reference's
-// warm-started 5-step chain converges to).
-__global__ void __launch_bounds__(kBlock) ph_table_kernel(int table_len, double step, double kw, double kchem, double ka,
-                                                          double MNaOH, double MHA, double MNH3, double *__restrict__ t64,
-                                                          float *__restrict__ t32) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= table_len) return;
-    double m = (double)i * step;
-    double ak = MNH3 - m + MNaOH + kchem + ka;
-    double bk = (kchem + ka) * MNaOH - (kchem + ka) * m - kw + MNH3 * ka + kchem * ka - ka * MHA;
-    double ck = MNaOH * kchem * ka - kw * (ka + kchem) - m * kchem * ka - ka * kchem * MHA;
-    double dk = -kchem * ka * kw;
-    auto f = [&](double H) { return (((H + ak) * H + bk) * H + ck) * H + dk; };
-    double lo = 1e-30, hi = 4.0;
-    for (int it = 0; it < 200; ++it) {  // geometric bisection: the root spans 1e-12 .. 1
-        double mid = sqrt(lo * hi);
-        if (f(mid) > 0.0) hi = mid; else lo = mid;
-        if (hi <= lo * (1.0 + 1e-9)) break;
+// Titration table (ph.py:72-84), the reference's own chain: 5 abs-Newton steps H <- |H - f/f'| per grid point on the
+// quartic f(H) = H^4 + a H^3 + b H^2 + c H + d, warm-started from the previous grid point, H**k as pow().  The chain is
+// sequential and is not always converged (e.g. MNH3 = 0.05, MHA = 0.02: its first entries are far from the quartic's
+// root), so it runs as written, on the host, once per chemistry; the table is then copied to the device.
+static void ph_table_host(const pime_ph_config &c, double *t64, float *t32) {
+    double H = 1e-14 / c.MNaOH;
+    const double kw = c.kw, kchem = c.kchem, ka = c.ka, MNaOH = c.MNaOH, MHA = c.MHA, MNH3 = c.MNH3;
+    for (int i = 0; i < c.table_len; ++i) {
+        double m = (double)i * c.mhcl_step;
+        double ak = MNH3 - m + MNaOH + kchem + ka;
+        double bk = (kchem + ka) * MNaOH - (kchem + ka) * m - kw + MNH3 * ka + kchem * ka - ka * MHA;
+        double ck = MNaOH * kchem * ka - kw * (ka + kchem) - m * kchem * ka - ka * kchem * MHA;
+        double dk = -kchem * ka * kw;
+        for (int j = 0; j < 5; ++j) {
+            double H2 = pow(H, 2.0), H3 = pow(H, 3.0), H4 = pow(H, 4.0);
+            double num = H4 + ak * H3 + bk * H2 + ck * H + dk;
+            double den = 4 * H3 + 3 * ak * H2 + 2 * bk * H + ck;
+            H = fabs(H - num / den);
+        }
+        t64[i] = -1 * log10(H);
+        t32[i] = (float)t64[i];
     }
-    double H = sqrt(lo * hi);
-    for (int it = 0; it < 50; ++it) {
-        double H2 = H * H, H3 = H2 * H, H4 = H3 * H;
-        double num = H4 + ak * H3 + bk * H2 + ck * H + dk;
-        double den = 4 * H3 + 3 * ak * H2 + 2 * bk * H + ck;
-        double Hn = fabs(H - num / den);
-        bool stop = fabs(Hn - H) <= 4e-16 * Hn;
-        H = Hn;
-        if (stop) break;
-    }
-    double v = -log10(H);
-    t64[i] = v;
-    if (t32) t32[i] = (float)v;
 }
 
 template <typename T>
@@ -533,11 +523,22 @@ int pime_wt_step_f64(const pime_wt_config *cfg, int64_t n, const pime_wt_state *
 int pime_ph_table_build(const pime_ph_config *cfg, double *table_f64, float *table_f32, void *stream) {
     PIME_REQUIRE(cfg && table_f64, "null config/table");
     PIME_REQUIRE(cfg->table_len > 1, "table_len");
+    if (int rc = validate_mhcl_step(cfg)) return rc;
     if (int rc = require_device()) return rc;
-    int grid = (cfg->table_len + kBlock - 1) / kBlock;
-    ph_table_kernel<<<grid, kBlock, 0, (cudaStream_t)stream>>>(cfg->table_len, cfg->mhcl_step, cfg->kw, cfg->kchem, cfg->ka,
-                                                              cfg->MNaOH, cfg->MHA, cfg->MNH3, table_f64, table_f32);
-    PIME_LAUNCH_CHECK();
+    std::vector<double> t64;
+    std::vector<float> t32;
+    try {   // no exception may cross the C ABI
+        t64.resize(cfg->table_len);
+        t32.resize(cfg->table_len);
+    } catch (const std::bad_alloc &) {
+        set_error("pime_ph_table_build: no host memory for the table");
+        return PIME_EINVAL;
+    }
+    ph_table_host(*cfg, t64.data(), t32.data());
+    cudaStream_t s = (cudaStream_t)stream;
+    PIME_CUDA(cudaMemcpyAsync(table_f64, t64.data(), t64.size() * sizeof(double), cudaMemcpyHostToDevice, s));
+    if (table_f32) PIME_CUDA(cudaMemcpyAsync(table_f32, t32.data(), t32.size() * sizeof(float), cudaMemcpyHostToDevice, s));
+    PIME_CUDA(cudaStreamSynchronize(s));   // the host buffers are freed on return
     return PIME_OK;
 }
 

@@ -319,6 +319,8 @@ class PH1DChangingParamUniformGoalIntegrator(_DeviceEnv):
         step = float(MHCl[1] - MHCl[0])
         if not np.array_equal(MHCl, np.arange(MHCl.shape[0]) * MHCl[1]):
             raise NotImplementedError("MHCl must be a uniform grid starting at 0 (np.arange(0, stop, step))")
+        if step != 1e-5:   # the kernels' table index is rint(C x 1e5), the reference's argwhere only on this grid
+            raise NotImplementedError("MHCl must have the step 1e-5 of every registered config")
         self.MHCl = MHCl
         self.qww_Vrange, self.qc_Vrange = list(qww_V), list(qc_V)
         self.sample_t, self.n_discrete, self.delta_t = sample_t, n_discrete, sample_t / n_discrete

@@ -404,7 +404,8 @@ _TABLES: dict = {}
 
 
 def ph_table(cfg: L.PhConfig, device) -> tuple:
-    """The titration table (ph.py:72-84) built once per device/config by the table kernel: (f64, f32) tensors."""
+    """The titration table (ph.py:72-84), the reference's chain computed on the host by pime_ph_table_build and copied to
+    the device once per device/config: (f64, f32) tensors."""
     key = (str(device), cfg.table_len, cfg.mhcl_step, cfg.kw, cfg.kchem, cfg.ka, cfg.MNaOH, cfg.MHA, cfg.MNH3)
     if key not in _TABLES:
         t64 = torch.empty(cfg.table_len, dtype=torch.float64, device=device)

@@ -150,22 +150,23 @@ def _grid(kps, kis, builder):
     return np.stack([builder(a, b) for a, b in zip(kp.ravel(), ki.ravel())], 1)   # [S, G]
 
 
-def _oracle_staircase(oracle, plant, K, params, setpoints, steps):
+def _oracle_staircase(oracle, plant, K, params, setpoints, steps, cfg=None, table=None, sample_t=20.0):
     """fp64 linear staircase stepped by the CPU oracle with each env's own K ([S, n], reference sign): metrics and response
-    [8, len(setpoints), n] in the order METRICS + RESPONSE."""
+    [8, len(setpoints), n] in the order METRICS + RESPONSE.  cfg (oracle.wt_cfg / ph_cfg, its step limit is lifted here),
+    table and sample_t (pH): the plant's configuration, by default the registered one."""
     n = params.shape[0]
     out = np.zeros((8, len(setpoints), n))
     j1 = np.arange(1, steps + 1)[:, None]
     if plant == "wt":
-        cfg = oracle.wt_cfg(reward_type="square_distance")
+        cfg = cfg or oracle.wt_cfg(reward_type="square_distance")
         cfg.max_step = 2 ** 30
         h1, h2 = np.zeros(n), np.zeros(n)
         a1, a2, Kp = (np.ascontiguousarray(params[:, j]) for j in range(3))
     else:
-        cfg = oracle.ph_cfg()
+        cfg = cfg or oracle.ph_cfg()
         cfg.max_episode_steps = 2 ** 30
-        table = oracle.ph_table()
-        A, B, Cc = oracle.ph_update_system(params[:, 0], params[:, 1])
+        table = oracle.ph_table() if table is None else table
+        A, B, Cc = oracle.ph_update_system(params[:, 0], params[:, 1], sample_t)
         x = np.zeros(n)
     for k, r_ in enumerate(setpoints):
         r, I, t = np.full(n, float(r_)), np.zeros(n), np.zeros(n, np.int32)
